@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]            product arm (CUDA path through the C ABI)
   python bench.py --impl reference [...]                          CPU arm: the oracle port on all host cores
   torchrun --nproc-per-node N ... bench.py --gpus N ...           one rank per GPU, files sharded by rank (weak scaling)
+  python bench.py ... --dump-outputs DIR                          also save what the timed legs returned (write_dump)
 
 Corpus (per GPU, synthetic): `--files` tone+noise 44.1 kHz stereo WAVs of `--frames` frames (SURVEY.md 8d), generated
 on the device; the decode corpus is those WAVs encoded to 320 kbps by the product's own encoder (bit-exact with the
@@ -318,6 +319,68 @@ def pcm_checksum(torch, pcm16, first_sample):
     return int(x.sum().item()), int((x * (1 + i % 65521)).sum().item())
 
 
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed legs returned in their last step, as .npy files (float32 / float64), so that two builds run
+# with the same arguments can be compared output for output.  The whole outputs are tens of GB; the per-file arrays go out
+# whole, the buffers as a sample whose positions come from a fixed seed and the arguments only.  NaN marks a sampled
+# position the call did not fill (a frame past the file's n_frames, a byte past its reveal_len / out_len).
+# ------------------------------------------------------------------------------------------------
+DUMP_FRAMES = 2048       # decoded frames sampled: their PCM (2,304 samples each), table ids and reveal-bit bytes (12 each)
+DUMP_WINDOWS = 2048      # MP3 byte windows sampled from the encoder's output
+DUMP_WINDOW = 418        # bytes per window: one 128 kbps frame at 44.1 kHz
+DUMP_LIMIT = 64 << 20
+
+
+def _gather(torch, buf, idx, valid):
+    """buf[idx] as float32 (buf on the device), NaN where not `valid`."""
+    valid = np.broadcast_to(valid, idx.shape)
+    idx = np.clip(np.where(valid, idx, 0), 0, buf.numel() - 1)
+    out = buf[torch.from_numpy(idx.reshape(-1)).to(buf.device)].float().cpu().numpy().reshape(idx.shape)
+    out[~valid] = np.nan
+    return out
+
+
+def dump_decode(torch, r, files, frames):
+    """m3s_decode's result of the device-resident leg: per-file arrays, and PCM / table ids / reveal bits of sampled frames."""
+    rng = np.random.default_rng(20261020)
+    n = min(DUMP_FRAMES, files * frames)
+    fi, fj = rng.integers(0, files, n), rng.integers(0, frames, n)          # frame fj of file fi
+    nfr = r["n_frames"]
+    base = np.concatenate([[0], np.cumsum(nfr)])
+    k = np.arange(12)
+    ok = (fj < nfr[fi])[:, None]
+    pcm = _gather(torch, r["pcm"], r["pcm_off"][fi][:, None] + 2304 * fj[:, None] + np.arange(2304), ok)
+    ids = _gather(torch, r["table_ids"], 12 * (base[fi] + fj)[:, None] + k, ok)
+    bits = _gather(torch, r["reveal_bits"], 12 * (base[fi] + fj)[:, None] + k, 12 * fj[:, None] + k < r["reveal_len"][fi][:, None])
+    out = {"decode_sample_frames": np.stack([fi, fj], 1), "decode_pcm": pcm, "decode_table_ids": ids, "decode_reveal_bits": bits}
+    for key in ("n_frames", "pcm_off", "reveal_len", "sample_rate", "channels", "bitrate", "status"):
+        out["decode_" + key] = r[key]
+    return out
+
+
+def dump_encode(torch, r, files):
+    """m3s_encode's result of the device-resident leg: per-clip out_len / hide_str_offset, and sampled windows of the MP3 bytes."""
+    rng = np.random.default_rng(20261021)
+    ci, u = rng.integers(0, files, DUMP_WINDOWS), rng.random(DUMP_WINDOWS)
+    ln = r["out_len"][ci]
+    start = (u * np.maximum(ln - DUMP_WINDOW, 0)).astype(np.int64)          # byte offset inside clip ci's MP3
+    k = np.arange(DUMP_WINDOW)
+    mp3 = _gather(torch, r["mp3"], (r["mp3_off"][ci] + start)[:, None] + k, start[:, None] + k < ln[:, None])
+    return {"encode_sample_windows": np.stack([ci, start], 1), "encode_mp3": mp3, "encode_out_len": r["out_len"],
+            "encode_hide_str_offset": r["hide_str_offset"]}
+
+
+def write_dump(out_dir, arrays):
+    arrays = {k: (v if v.dtype == np.float32 else v.astype(np.float64)) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total / 2**20:.1f} MiB (limit {DUMP_LIMIT >> 20} MiB)")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    log(f"dump: {len(arrays)} arrays, {total / 2**20:.1f} MiB -> {out_dir}")
+
+
 def run_product_arm(args):
     import torch
     import __graft_entry__ as ge
@@ -469,8 +532,11 @@ def run_product_arm(args):
     log(f"[rank {rank}] host ceiling ({world} ranks at once): D2H {roof['d2h_gbs']:.1f} GB/s, H2D {roof['h2d_gbs']:.1f} GB/s, "
         f"D2H under the decode mix {roof['mix_gbs']:.1f} GB/s")
 
+    last = {}      # the result of each device-resident leg's latest call (for --dump-outputs)
+
     def dec_device():
         r = h.decode(mp3_all, off_all, pcm=pcm_out_dev, table_ids=ids_dev, reveal_bits=bits_dev, frames_bound=total_frames)
+        last["decode"] = r
         check["reveal_bits"] = int(r["reveal_len"].sum())
         return int(r["n_frames"].sum())
 
@@ -489,6 +555,7 @@ def run_product_arm(args):
     # encode+hide: ONE call over all clips (the per-clip offset scan of the rate loop wants every clip's chain in flight together)
     def enc_device():
         r = h.encode(pcm_all, ns_all, 44100, 128, payload_packed=(pay_all, pay_off_all), mp3_out=enc_out_dev)
+        last["encode"] = r
         check["hide_off"] = int(r["hide_str_offset"].sum())
         check["enc_bytes"] = int(r["out_len"].sum())
         return total_frames
@@ -544,6 +611,9 @@ def run_product_arm(args):
         return
     D = measure(dec_device, dec_host, DEC_K, DEC_BYTES_PER_FRAME)
     log(f"[rank {rank}] decode+reveal: {D['value']:.4g} frames/s device-resident, {D['e2e_value']:.4g} e2e")
+    dump = {}
+    if args.dump_outputs and rank == 0:
+        dump.update(dump_decode(torch, last["decode"], args.files, args.frames))
 
     # ---- what the timed decode legs computed, against the oracle (untimed, rank 0): 3 corpus files out of the device-resident
     #      leg's output buffer -- reveal bits equal, int16 PCM within 1 LSB
@@ -573,6 +643,8 @@ def run_product_arm(args):
         log(f"[rank {rank}] encode e2e leg: {args.files} clips x {fe} frames from pinned host memory ({args.files * fe * 4608 / 1e9:.1f} GB)")
         E = measure(enc_device, enc_host, ENC_K, ENC_BYTES_PER_FRAME)
         log(f"[rank {rank}] encode+hide:   {E['value']:.4g} frames/s device-resident, {E['e2e_value']:.4g} e2e")
+        if args.dump_outputs and rank == 0:
+            dump.update(dump_encode(torch, last["encode"], args.files))
         if rank == 0:
             from oracle import oracle as O
             rng = np.random.default_rng(777)
@@ -588,6 +660,8 @@ def run_product_arm(args):
                 got = bytes(enc_out_dev[mo: mo + nbytes].cpu().numpy())
                 ok = ok and got == ref["mp3"][:nbytes]
             parity["encode"] = dict(clips=pick, frames_compared_per_clip=nf_chk, bytes_equal=bool(ok), ok=bool(ok))
+    if dump:
+        write_dump(args.dump_outputs, dump)
 
     # ---- composites (SURVEY 8f row 1): hide_message / clear_file for a batch, decode (float64) -> int16 in HBM -> encode
     comp = None
@@ -600,7 +674,7 @@ def run_product_arm(args):
         cut = int(h.decode_frame_pos()[f_c]) if f_c < args.frames else b1
         blobs = [bytes(mp3_host_all[int(off_all[i]): int(off_all[i]) + cut].numpy()) for i in range(n_c)]
         msgs = ["".join(chr(32 + (7 * i + 3 * k) % 95) for k in range(40)) for i in range(n_c)]
-        cs = max(1, min(args.steps, 3))
+        cs = max(1, args.steps)
         batch.hide_batch(h, blobs, msgs)      # warm-up
         barrier()
         t0 = time.perf_counter()
@@ -715,7 +789,7 @@ def run_cfg5(args, torch, dist, h, stream, dev, rank, world, barrier, timed, pcm
     del chunks
     frames_mine = len(mine) * NF
     mp3_host = mp3.cpu().pin_memory()
-    steps = max(1, min(args.steps, 3))
+    steps = max(1, args.steps)
     cap_files = max(1, (pcm_out_dev.numel() - 64) // (n_samp * 2))
     cap_host = max(1, (arena.numel() - 64) // (n_samp * 2))
 
@@ -865,6 +939,8 @@ def main():
     ap.add_argument("--only-cfg5", action="store_true", help="diagnostic: run configs[4] alone")
     ap.add_argument("--cfg5-files", type=int, default=10000, help="tracks of the strong-scaled configs[4] corpus (whole job)")
     ap.add_argument("--cfg5-long", type=int, default=60000, help="frames of the long file split by frame range")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the device-resident decode and encode legs returned in "
+                    "their last timed step to DIR/<name>.npy (rank 0; a seeded sample of the large buffers, <= 64 MiB)")
     args = ap.parse_args()
     quiet_stdout()
     if args.impl == "reference":
