@@ -219,6 +219,7 @@ struct m3s_ctx {
     bool scanned = false;
     double dec_bpf_guess = 0.0;        // bytes per frame seen by earlier scans of device-resident input (sizes the next scan's workspaces)
     int64_t dec_wave_bytes = 0;        // M3S_DEC_WAVE_BYTES override of the pipelined call's wave size (0 = default)
+    bool dec_hybrid_direct = false;    // M3S_HYBRID_DIRECT: synthesis by the direct-form kernels (k_hybrid), the A/B and cross-check form
     M3sBuf b_stage_in[2], b_pcm_stage[2];
     M3sBuf b_sf, b_S, b_spec, b_work, b_spec_export;
     void *work_pin[2] = {nullptr, nullptr};   // pinned staging of the hybrid kernel's work lists

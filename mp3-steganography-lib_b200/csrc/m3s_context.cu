@@ -262,6 +262,7 @@ extern "C" int m3s_create(int device, m3s_handle_t *out)
     h->stream = h->own_stream;
     if (const char *cb = getenv("M3S_ENC_CHUNK_FRAMES")) h->enc_chunk_budget = atoll(cb);
     if (const char *cb = getenv("M3S_DEC_WAVE_BYTES")) h->dec_wave_bytes = atoll(cb);
+    h->dec_hybrid_direct = getenv("M3S_HYBRID_DIRECT") != nullptr;
     M3sDevTables *T = new M3sDevTables();
     memset(T, 0, sizeof *T);
     build_tables(T);

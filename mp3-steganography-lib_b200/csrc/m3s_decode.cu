@@ -1412,10 +1412,9 @@ k_hybrid(const uint32_t *__restrict__ spec, const M3sUnitRec *__restrict__ units
                                 const int64_t e = wk.pcm_elem + (row0 + 32 * (par + 2 * (q0 + q))) * nch + ch;
                                 if (FLOAT_OUT) ((float *)pcm_out)[e] = (float)out[q];
                                 else {
-                                    // (pcm * 32767).astype(int16): truncate toward zero, keep the low 16 bits (A.D8)
-                                    int a;
-                                    if constexpr (sizeof(R) == 4) a = __float2int_rz(out[q] * 32767.f);
-                                    else a = __double2int_rz(out[q] * 32767.0);
+                                    // (pcm * 32767).astype(int16): truncate toward zero to int32 (0x80000000 outside it), keep the
+                                    // low 16 bits (A.D8)
+                                    const int a = hf_to_int(out[q] * (R)32767);
                                     ((int16_t *)pcm_out)[e] = (int16_t)(a & 0xFFFF);
                                 }
                             }
@@ -1874,8 +1873,7 @@ static int run_enqueue(m3s_ctx *h, M3sScanSet &ss, void *d_pcm, int16_t *d_spect
         if (n_stereo > 0) M3S_LAUNCH_HYBRID_FAST1(OUT, FL, 2, R, TAB, tabptr, 0, n_stereo);                                   \
         if (work.size() > n_stereo) M3S_LAUNCH_HYBRID_FAST1(OUT, FL, 1, R, TAB, tabptr, n_stereo, work.size() - n_stereo);    \
     } while (0)
-    static const bool direct = getenv("M3S_HYBRID_DIRECT") != nullptr;   // A/B and cross-check: the direct-form kernels of round 1
-    if (direct) {
+    if (h->dec_hybrid_direct) {   // A/B and cross-check: the direct-form kernels of round 1 (M3S_HYBRID_DIRECT, read per handle)
         if (exact) {
             if (fl) M3S_LAUNCH_HYBRID(double, M3sDevTablesD, true, h->d_tab_f64);
             else M3S_LAUNCH_HYBRID(double, M3sDevTablesD, false, h->d_tab_f64);

@@ -58,8 +58,10 @@ __device__ __forceinline__ float hf_pow43_big(float, int ax) { return (float)ax 
 __device__ __forceinline__ double hf_pow43_big(double, int ax) { return pow((double)ax, 4.0 / 3.0); }
 __device__ __forceinline__ float hf_signed(float m, int x) { return __int_as_float(__float_as_int(m) | (x & 0x80000000)); }   // m >= 0: OR in the sign of x
 __device__ __forceinline__ double hf_signed(double m, int x) { return x < 0 ? -m : m; }
-__device__ __forceinline__ int hf_to_int(float o) { return __float2int_rz(o); }
-__device__ __forceinline__ int hf_to_int(double o) { return __double2int_rz(o); }
+// v -> int32 as numpy's astype does it on x86 (cvttss2si / cvttsd2si): truncation toward zero, and 0x80000000 for v >= 2^31,
+// v < -2^31 or NaN, where __float2int_rz / __double2int_rz would saturate (A.D8).  2^31 is exact in both types.
+__device__ __forceinline__ int hf_to_int(float o) { return o >= -2147483648.0f && o < 2147483648.0f ? __float2int_rz(o) : (int)0x80000000; }
+__device__ __forceinline__ int hf_to_int(double o) { return o >= -2147483648.0 && o < 2147483648.0 ? __double2int_rz(o) : (int)0x80000000; }
 
 // Packed FP32 (Blackwell FFMA2, PTX fma.rn.f32x2): two independent round-to-nearest FMAs per instruction -- the same results as two
 // fmaf, half the issue slots.  The windowing's two accumulator chains per output sample (even / odd history rows) run as one.
@@ -451,7 +453,8 @@ k_hybrid_fast(const uint32_t *__restrict__ spec, const M3sUnitRec *__restrict__ 
                         o = acc0 + acc1;
                     }
                     OUT *so = &sm.stage[ch][gr * 576 + 32 * par + lane];
-                    // (pcm * 32767).astype(int16): truncate, keep the low 16 bits (A.D8); FP32 carries the factor in its window coefficients
+                    // (pcm * 32767).astype(int16): truncate to int32 (0x80000000 outside it), keep the low 16 bits (A.D8); FP32 carries
+                    // the factor in its window coefficients
                     if (FLOAT_OUT) so[64 * q] = (OUT)o;
                     else if constexpr (sizeof(R) == 8) so[64 * q] = (OUT)(int16_t)hf_to_int(o * (R)32767);
                     else so[64 * q] = (OUT)(int16_t)hf_to_int(o);

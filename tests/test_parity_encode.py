@@ -205,6 +205,34 @@ def test_analysis_kernel_forms(built, oracle, monkeypatch, form):
         assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
 
 
+@pytest.mark.parametrize("env", [{"M3S_PROBE_CTAS": "1"}, {"M3S_PROBE_CTAS": "7"}, {"M3S_PROBE_CFG": "1"}, {"M3S_PROBE_CFG": "2"},
+                                 {"M3S_ENC_OVERLAP": "1", "M3S_ENC_CHUNK_FRAMES": "64"},
+                                 {"M3S_ENC_SERIAL": "1", "M3S_ENC_CHAIN": "1", "M3S_ENC_CHUNK_FRAMES": "64"}],
+                         ids=["probe_ctas1", "probe_ctas7", "probe_cfg1", "probe_cfg2", "overlap", "serial_chain"])
+def test_encoder_switches(built, oracle, monkeypatch, env):
+    """The encoder's diagnostic switches (read per call) give the oracle's MDCT lines, bytes and offsets: a probe grid smaller than
+    the tile count (M3S_PROBE_CTAS, k_enc_probe's strided tile walk), the other probe CTA shapes (M3S_PROBE_CFG 1, 2), the analysis
+    of chunk k + 1 overlapped with the rate loop of chunk k (M3S_ENC_OVERLAP) and the serial sequential rate loop, both over
+    64-frame chunks (bytes and offsets; the taps need a single-chunk batch)."""
+    from mp3stego_b200 import _lib
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)
+    quiet = synth_wav(31, 40).copy()
+    quiet[1152 * 5:1152 * 9] = 0
+    quiet[1152 * 9:1152 * 12] = (quiet[1152 * 9:1152 * 12] >> 13).astype(np.int16)
+    clips = [synth_wav(30, 150), quiet, _clicks(11, 33 * 1152, 5), np.zeros((7 * 1152, 2), np.int16)]
+    bits = ["0110" * 900, "1" * 300, "10" * 200, ""]
+    taps = "M3S_ENC_CHUNK_FRAMES" not in env     # the taps of a batch need it in one chunk
+    h = _lib.Handle(0)
+    got = _encode(h, clips, 128, payloads=bits, taps=taps)
+    h.close()
+    for c, p, g in zip(clips, bits, got):
+        ref = oracle.encode(c, 44100, 128, p, taps=taps)
+        if taps:
+            _check_taps(g, ref)
+        assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
+
+
 def test_chunked_regular_batch_host_and_device(built, oracle):
     """Equal-length clips take the strided (2-D) PCIe staging path of the host pipeline; host and device buffers and the
     oracle must agree byte for byte across chunk boundaries."""

@@ -33,7 +33,7 @@ def main():
     configs = [("default", {}), ("overlap", {"M3S_ENC_OVERLAP": "1"}), ("probe_ctas=296", {"M3S_PROBE_CTAS": "296"}), ("probe_ctas=444", {"M3S_PROBE_CTAS": "444"}),
                ("serial", {"M3S_ENC_SERIAL": "1"}), ("chain (old rate loop)", {"M3S_ENC_CHAIN": "1"}),
                ("chain serial", {"M3S_ENC_CHAIN": "1", "M3S_ENC_SERIAL": "1"})]
-    configs += [(f"cfg{k} serial", {"M3S_PROBE_CFG": str(k), "M3S_ENC_SERIAL": "1"}) for k in range(6)]
+    configs += [(f"cfg{k} serial", {"M3S_PROBE_CFG": str(k), "M3S_ENC_SERIAL": "1"}) for k in range(3)]   # configurations 0..2 exist
     if len(sys.argv) > 3:   # only the named configurations; "env:A=1,B=2" adds an ad-hoc one
         adhoc = [(a[4:], dict(kv.split("=") for kv in a[4:].split(","))) for a in sys.argv[3:] if a.startswith("env:")]
         configs = [c for c in configs if any(c[0].startswith(a) for a in sys.argv[3:])] + adhoc
