@@ -151,7 +151,7 @@ struct M3sBuf {
     size_t cap = 0;
 };
 
-// One CTA's run of frames in k_hybrid.
+// One CTA's run of frames in k_hybrid_fast.
 struct M3sWork {
     int64_t g_first;   // first frame whose PCM this CTA emits
     int32_t count;     // frames to emit
@@ -219,7 +219,6 @@ struct m3s_ctx {
     bool scanned = false;
     double dec_bpf_guess = 0.0;        // bytes per frame seen by earlier scans of device-resident input (sizes the next scan's workspaces)
     int64_t dec_wave_bytes = 0;        // M3S_DEC_WAVE_BYTES override of the pipelined call's wave size (0 = default)
-    bool dec_hybrid_direct = false;    // M3S_HYBRID_DIRECT: synthesis by the direct-form kernels (k_hybrid), the A/B and cross-check form
     M3sBuf b_stage_in[2], b_pcm_stage[2];
     M3sBuf b_sf, b_S, b_spec, b_work, b_spec_export;
     void *work_pin[2] = {nullptr, nullptr};   // pinned staging of the hybrid kernel's work lists
@@ -252,7 +251,7 @@ struct M3sRow { char *dst; const char *src; size_t bytes; };
 int m3s_copy_paced(m3s_ctx *h, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind);
 cudaError_t m3s_copy_bulk(void *dst, const void *src, size_t bytes, cudaMemcpyKind kind, cudaStream_t s);   // in bounded pieces
 cudaError_t m3s_copy_rows(const std::vector<M3sRow> &rows, cudaMemcpyKind kind, cudaStream_t s);
-int m3s_upload_cos36(const float *f, const double *d);  // m3s_decode.cu: constant-memory IMDCT rows of the current device
+int m3s_upload_fast_const();  // m3s_decode.cu: the fast transforms' twiddles in constant memory of the current device
 
 // launches on `s` are timed on `s` (m3s_time_begin records on launch_stream); restored when the scope ends, error returns included
 struct M3sLaunchOn {

@@ -262,7 +262,6 @@ extern "C" int m3s_create(int device, m3s_handle_t *out)
     h->stream = h->own_stream;
     if (const char *cb = getenv("M3S_ENC_CHUNK_FRAMES")) h->enc_chunk_budget = atoll(cb);
     if (const char *cb = getenv("M3S_DEC_WAVE_BYTES")) h->dec_wave_bytes = atoll(cb);
-    h->dec_hybrid_direct = getenv("M3S_HYBRID_DIRECT") != nullptr;
     M3sDevTables *T = new M3sDevTables();
     memset(T, 0, sizeof *T);
     build_tables(T);
@@ -282,19 +281,7 @@ extern "C" int m3s_create(int device, m3s_handle_t *out)
         if (e == cudaSuccess) e = cudaMemcpy(h->d_tab_f64, TD, sizeof(M3sDevTablesD), cudaMemcpyHostToDevice);
         delete TD;
     }
-    if (e == cudaSuccess) {
-        // the 18 distinct IMDCT-36 rows (outputs 0..8 and 18..26) as immediate constant-bank operands
-        const double PI = 3.141592653589793;
-        static float cf[18][18];
-        static double cd[18][18];
-        for (int r = 0; r < 18; r++)
-            for (int k = 0; k < 18; k++) {
-                const int i = r < 9 ? r : 18 + (r - 9);
-                cd[r][k] = cos(PI / 72.0 * (2 * i + 1 + 18) * (2 * k + 1));
-                cf[r][k] = (float)cd[r][k];
-            }
-        if (m3s_upload_cos36(&cf[0][0], &cd[0][0]) != 0) e = cudaErrorUnknown;
-    }
+    if (e == cudaSuccess && m3s_upload_fast_const() != 0) e = cudaErrorUnknown;
     if (e != cudaSuccess) {
         if (h->d_tab) cudaFree(h->d_tab);
         if (h->d_tab_f64) cudaFree(h->d_tab_f64);

@@ -1032,68 +1032,16 @@ __global__ void k_spec_export(const uint32_t *__restrict__ spec, int64_t total_f
 
 // ================================================================================================
 // D2 + D3: requantize, MS stereo, reorder / alias, IMDCT + window + overlap, frequency inversion,
-// polyphase synthesis, int16 pack.  One CTA walks a run of consecutive frames of one file, keeping the
-// overlap buffer and the 15-slot V history in shared memory; a run that does not start its file first
-// re-decodes one warm-up frame (SURVEY.md 8e) whose PCM is discarded.
+// polyphase synthesis, int16 pack: k_hybrid_fast (m3s_hybrid_fast.cuh).  One CTA walks a run of consecutive
+// frames of one file; a run that does not start its file first re-decodes one warm-up frame (SURVEY.md 8e)
+// whose PCM is discarded.
 // (Frame.py:157-218 re_quantize, :561-572, :574-602, :604-622, :106-154 imdct, :624-631, :65-103 synth,
 //  :633-640 interleave, MP3_Parser.py:91 int16 conversion)
 // ================================================================================================
-
-#define HYB_THREADS 256
-
-template <typename R>
-struct HybSmem {
-    uint4 specw[2][288];       // integer spectra of the current / next frame: [pair] = (x, y) int16 of the four granule-channels
-    R xr[2][576];
-    R prev[2][2][576];
-    R tt[2][18][32];
-    R v[2][51][32];            // the 32 DISTINCT matrixing outputs per slot (see "matrixing"): 15 slots of history + 2 granules x 18 new
-    R uw[HYB_THREADS / 32][32];  // per-warp butterfly scratch: u[0..15] | w[0..15]
-    R cos12[12][8];
-    R sine[4][36];
-    R pow43[256];
-    R scale[4][64];             // per slot: 2^(e4/4) of long sfb 0..21 | short (sfb * 3 + window) at 22..60, rebuilt every frame
-    R cs[8], ca[8];
-    R quarter[4];
-    uint16_t reorder[576];
-    uint8_t long_sfb[576];
-    uint8_t short_sfw[576];
-    uint8_t pretab[24];
-    M3sUnitRec rec[4];
-    uint8_t sf[4][M3S_SF_STRIDE];
-    int sr_loaded;
-};
-
-__device__ __forceinline__ float pow2i(int e)  // 2^e for e in the normal float range
-{
-    e = e < -126 ? -126 : (e > 127 ? 127 : e);
-    return __int_as_float((e + 127) << 23);
-}
-
-// requantize (Frame.py:210-215): |x|^(4/3) * 2^(e4/4).  The exponent e4 depends only on the scalefactor band (and window), so the factor
-// 2^(e4/4) = quarter[e4 & 3] * 2^(e4 >> 2) is tabulated once per frame and slot (HybSmem::scale); a sample costs one lookup and one multiply.
-// FP32: |x|^(4/3) from a table / cbrt, exact powers of two; FP64 (the `exact` instantiation): double-precision pow for the large values.
-__device__ __forceinline__ float requant_scale(const HybSmem<float> &sm, int e4) { return sm.quarter[e4 & 3] * pow2i(e4 >> 2); }
-__device__ __forceinline__ double requant_scale(const HybSmem<double> &sm, int e4) { return sm.quarter[e4 & 3] * scalbn(1.0, e4 >> 2); }
-__device__ __forceinline__ float requant_pow43(const HybSmem<float> &sm, int ax) { return ax < 256 ? sm.pow43[ax] : (float)ax * cbrtf((float)ax); }
-__device__ __forceinline__ double requant_pow43(const HybSmem<double> &sm, int ax) { return ax < 256 ? sm.pow43[ax] : pow((double)ax, 4.0 / 3.0); }
-__device__ __forceinline__ float fma_t(float a, float b, float c) { return fmaf(a, b, c); }
-__device__ __forceinline__ double fma_t(double a, double b, double c) { return fma(a, b, c); }
-
-// The 18 distinct rows of the 36-point IMDCT matrix (rows 0..8: outputs 0..8; rows 9..17: outputs 18..26) in constant memory:
-// with the row and column known at compile time every coefficient is an immediate constant-bank operand of its FMA.
-__constant__ float c_cos36_f[18][18];
-__constant__ double c_cos36_d[18][18];
-template <typename R> __device__ __forceinline__ R cos36c(int row, int k);
-template <> __device__ __forceinline__ float cos36c<float>(int row, int k) { return c_cos36_f[row][k]; }
-template <> __device__ __forceinline__ double cos36c<double>(int row, int k) { return c_cos36_d[row][k]; }
-
 #include "m3s_hybrid_fast.cuh"
 
-int m3s_upload_cos36(const float *f, const double *d)
+int m3s_upload_fast_const()
 {
-    if (cudaMemcpyToSymbol(c_cos36_f, f, sizeof(float) * 18 * 18) != cudaSuccess) return -1;
-    if (cudaMemcpyToSymbol(c_cos36_d, d, sizeof(double) * 18 * 18) != cudaSuccess) return -1;
     M3sFastConst fc;   // twiddles of the fast transforms, in both precisions
     m3s_fast_const_build(fc);
     if (cudaMemcpyToSymbol(c_fast, &fc, sizeof fc) != cudaSuccess) return -1;
@@ -1101,338 +1049,6 @@ int m3s_upload_cos36(const float *f, const double *d)
     m3s_fast_const_build(fcd);
     if (cudaMemcpyToSymbol(c_fast_d, &fcd, sizeof fcd) != cudaSuccess) return -1;
     return 0;
-}
-
-// Long-block IMDCT of one subband for warp role Q (Frame.py:119-133, 150-153): x_i = sum_k X_k cos(pi/72 (2 i + 19)(2 k + 1)) has
-// x_{17-i} = -x_i and x_{53-i} = x_i, so 18 sums give all 36 outputs; roles 0/1 take sums 0..4 / 5..8 of the first half (windowed,
-// overlap-added, frequency-inverted into tt), roles 2/3 the same of the second half (windowed into the next overlap buffer).
-template <typename R, int Q>
-__device__ __forceinline__ void imdct_long(const R (&x)[18], const R *sine_bt, const R *pv, R *pn, R *tt_col, int sb)
-{
-    constexpr int D0 = (Q & 1) ? 5 : 0, N = (Q & 1) ? 4 : 5;
-    constexpr bool SECOND = Q >= 2;
-#pragma unroll
-    for (int ii = 0; ii < N; ii++) {
-        const int d = D0 + ii;
-        R acc = (R)0;
-#pragma unroll
-        for (int k = 0; k < 18; k++) acc = fma_t(x[k], cos36c<R>((SECOND ? 9 : 0) + d, k), acc);
-        if (!SECOND) {
-            const int j = 17 - d;
-            R o1 = acc * sine_bt[d] + pv[18 * sb + d];
-            R o2 = -acc * sine_bt[j] + pv[18 * sb + j];
-            if ((sb & 1) && (d & 1)) o1 = -o1;
-            if ((sb & 1) && (j & 1)) o2 = -o2;
-            tt_col[32 * d] = o1;      // tt[ch][d][sb]
-            tt_col[32 * j] = o2;
-        } else {
-            pn[18 * sb + d] = acc * sine_bt[18 + d];
-            pn[18 * sb + 17 - d] = acc * sine_bt[35 - d];
-        }
-    }
-}
-
-// Windowing of NQ same-parity slots t = par + 2 (q0 + q) for one (channel, lane): pcm[32 t + i] = sum_m V_{t-2m}[i] D[64 m + i] +
-// V_{t-2m-1}[32 + i] D[64 m + 32 + i] (Frame.py:89-101).  Slots of one parity share their V rows (row offset 2 (q - m)), so NQ + 7
-// loads per operand feed NQ x 8 FMAs instead of one load per FMA.  va0 / vb0 point at the rows of q = q0, m = 7.
-template <typename R, int NQ>
-__device__ __forceinline__ void window_tile(const R *__restrict__ va0, const R *__restrict__ vb0, const R (&dA)[8], const R (&dB)[8], R (&out)[5])
-{
-    R a[NQ + 7], b[NQ + 7];
-#pragma unroll
-    for (int d = 0; d < NQ + 7; d++) { a[d] = va0[64 * d]; b[d] = vb0[64 * d]; }
-#pragma unroll
-    for (int q = 0; q < NQ; q++) {
-        R acc0 = (R)0, acc1 = (R)0;
-#pragma unroll
-        for (int m = 0; m < 8; m++) {
-            acc0 = fma_t(a[q - m + 7], dA[m], acc0);
-            acc1 = fma_t(b[q - m + 7], dB[m], acc1);
-        }
-        out[q] = acc0 + acc1;
-    }
-}
-
-template <typename R, typename TAB, bool FLOAT_OUT>
-__global__ void __launch_bounds__(HYB_THREADS, sizeof(R) == 4 ? 3 : 1)
-k_hybrid(const uint32_t *__restrict__ spec, const M3sUnitRec *__restrict__ units, const uint8_t *__restrict__ sfin,
-         const uint32_t *__restrict__ fr_meta, const M3sWork *__restrict__ work, const M3sDevTables *__restrict__ T,
-         const TAB *__restrict__ TF, void *__restrict__ pcm_out)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    HybSmem<R> &sm = *reinterpret_cast<HybSmem<R> *>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const M3sWork wk = work[blockIdx.x];
-    const int nch = wk.channels;
-
-    // ---- one-time table staging
-    for (int i = tid; i < 12 * 8; i += HYB_THREADS) (&sm.cos12[0][0])[i] = (&TF->imdct_cos12[0][0])[i];
-    for (int i = tid; i < 4 * 36; i += HYB_THREADS) (&sm.sine[0][0])[i] = (&TF->sine_block[0][0])[i];
-    for (int i = tid; i < 256; i += HYB_THREADS) sm.pow43[i] = TF->pow43[i];
-    if (tid < 8) { sm.cs[tid] = TF->alias_cs[tid]; sm.ca[tid] = TF->alias_ca[tid]; }
-    if (tid < 4) sm.quarter[tid] = TF->quarter[tid];
-    if (tid < 22) sm.pretab[tid] = T->pretab[tid];
-    if (tid == 0) sm.sr_loaded = -1;
-    for (int i = tid; i < 2 * 2 * 576; i += HYB_THREADS) (&sm.prev[0][0][0])[i] = (R)0;
-    for (int i = tid; i < 2 * 51 * 32; i += HYB_THREADS) (&sm.v[0][0][0])[i] = (R)0;
-    // ---- matrixing (Frame.py:81-87): V[i] = sum_j N[i][j] S[j], N[i][j] = cos((16 + i)(2 j + 1) pi / 64).
-    // Two exact symmetries shrink the 64 x 32 product to 32 x 16:
-    //   (a) N[i][31 - j] = (-1)^i N[i][j]            -> V[i] = sum_{j<16} N[i][j] (S[j] +- S[31 - j])      (u for even i, w for odd i)
-    //   (b) V[32 - i] = -V[i] (so V[16] = 0) and V[96 - i] = V[i]  -> only i = 0..15 and 48..63 are distinct.
-    // Lane l owns the distinct output i(l) = l (l < 16) or 32 + l (l >= 16) and keeps its 16 coefficients in registers.
-    R ncoef[16];
-    {
-        const int i = lane < 16 ? lane : 32 + lane;
-#pragma unroll
-        for (int j = 0; j < 16; j++) ncoef[j] = TF->synth_n[i][j];
-    }
-    // ---- windowing (Frame.py:89-101): pcm[32 t + i] = sum_m V_{t-2m}[i] D[64 m + i] + V_{t-2m-1}[32 + i] D[64 m + 32 + i].
-    // Lane i reads V through symmetry (b): V[i] = +W[i] | 0 | -W[32 - i], V[32 + i] = -W[0] | +W[32 - i] | +W[i]; the signs are
-    // folded into its 16 window coefficients, which stay in registers.
-    R dA[8], dB[8];
-    int idxA, idxB;
-    {
-        const int i = lane;
-        const R sA = i < 16 ? (R)1 : (i == 16 ? (R)0 : (R)-1);
-        const R sB = i == 0 ? (R)-1 : (R)1;
-        idxA = i < 16 ? i : (i == 16 ? 0 : 32 - i);
-        idxB = i == 0 ? 0 : (i < 16 ? 32 - i : i);
-#pragma unroll
-        for (int m = 0; m < 8; m++) { dA[m] = sA * TF->synth_d[64 * m + i]; dB[m] = sB * TF->synth_d[64 * m + 32 + i]; }
-    }
-    __syncthreads();
-
-    int pp = 0;  // ping-pong index of the overlap buffer: prev[pp] is read, prev[pp ^ 1] written
-    const int64_t g_begin = wk.g_first - (wk.warm ? 1 : 0);
-    const int64_t g_end = wk.g_first + wk.count;
-    // the frame's integer spectra (one 16-byte word per pair: the four granule-channels) are fetched one frame ahead with cp.async
-    // into shared memory, so that the requantize phase does not wait for DRAM in front of its barrier (and no registers are held)
-    const uint4 *spec4 = (const uint4 *)spec;
-    auto fetch_spec = [&](int64_t gf, int buf) {
-        for (int p = tid; p < 288; p += HYB_THREADS) {
-            const unsigned dst = (unsigned)__cvta_generic_to_shared(&sm.specw[buf][p]);
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(spec4 + gf * 288 + p) : "memory");
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-    fetch_spec(g_begin, 0);
-    for (int64_t g = g_begin; g < g_end; g++) {
-        const bool emit = g >= wk.g_first;
-        const uint32_t meta = fr_meta[g];
-        const int sbuf = (int)((g - g_begin) & 1);
-        asm volatile("cp.async.wait_group 0;" ::: "memory");   // my part of this frame's spectra has landed; the barrier below publishes everyone's
-        const int sr = (meta >> M3S_META_SR_SHIFT) & 3;
-        // ---- per-frame records
-        if (tid < 4) sm.rec[tid] = units[4 * g + tid];
-        if (tid >= 32 && tid < 32 + 16) ((uint4 *)&sm.sf[0][0])[tid - 32] = ((const uint4 *)(sfin + 4 * g * M3S_SF_STRIDE))[tid - 32];
-        if (sm.sr_loaded != sr) {  // uniform branch: sr_loaded is only written behind the barrier below
-            for (int i = tid; i < 576; i += HYB_THREADS) {
-                sm.reorder[i] = T->reorder_dst[sr][i];
-                sm.long_sfb[i] = T->long_sfb_of[sr][i];
-                sm.short_sfw[i] = T->short_sfw_of[sr][i];
-            }
-        }
-        __syncthreads();
-        if (tid == 0) sm.sr_loaded = sr;
-        if (g + 1 < g_end) fetch_spec(g + 1, sbuf ^ 1);   // the other buffer was last read two barriers or more ago (previous frame's requantize)
-        const bool ms = (meta & M3S_META_MS) != 0;
-        {   // scale table: thread = (slot, band index)
-            const int slot = tid >> 6, idx = tid & 63;
-            const M3sUnitRec &r = sm.rec[slot];
-            const uint8_t *sf = sm.sf[slot];
-            const int gg = M3S_UA_GG(r.a), mult4 = M3S_UB_SFSCALE(r.b) ? 4 : 2;
-            int e4 = 0;
-            if (idx < 22) e4 = gg - 210 - mult4 * ((int)sf[idx] + (int)M3S_UB_PREFLAG(r.b) * (int)sm.pretab[idx]);
-            else if (idx < 61) {
-                const int q = idx - 22, sfb = q / 3, wnd = q - 3 * sfb;
-                e4 = gg - 210 - 8 * (int)M3S_UC_SBG(r.c, wnd) - mult4 * (int)sf[M3S_SF_SHORT + 13 * wnd + sfb];
-            }
-            sm.scale[slot][idx] = requant_scale(sm, e4);
-        }
-        __syncthreads();
-
-        for (int gr = 0; gr < 2; gr++) {
-            // ------------------------------------------------ requantize + MS + reorder (fused)
-            for (int p = tid; p < 288; p += HYB_THREADS) {
-                const uint4 w4 = sm.specw[sbuf][p];
-                R val[2][2];
-#pragma unroll
-                for (int ch = 0; ch < 2; ch++) {
-                    if (ch >= nch) { val[ch][0] = val[ch][1] = (R)0; continue; }
-                    const int slot = 2 * gr + ch;
-                    const uint32_t wv = slot == 0 ? w4.x : (slot == 1 ? w4.y : (slot == 2 ? w4.z : w4.w));
-                    const bool shortp = M3S_UA_BT(sm.rec[slot].a) == 2;
-                    const R *sc = sm.scale[slot];
-#pragma unroll
-                    for (int h = 0; h < 2; h++) {
-                        const int i = 2 * p + h;
-                        const int x = (int)(int16_t)(h ? (wv >> 16) : (wv & 0xFFFFu));
-                        const int idx = shortp ? 22 + (int)sm.short_sfw[i] : (int)sm.long_sfb[i];
-                        const int ax = x < 0 ? -x : x;
-                        const R m = requant_pow43(sm, ax) * sc[idx];
-                        val[ch][h] = x < 0 ? -m : m;
-                    }
-                }
-                if (ms && nch == 2) {
-#pragma unroll
-                    for (int h = 0; h < 2; h++) {
-                        const R mm = val[0][h], ss = val[1][h];
-                        val[0][h] = (mm + ss) * (R)0.70710678118654752;   // (M + S) / SQRT2, Frame.py:568-572
-                        val[1][h] = (mm - ss) * (R)0.70710678118654752;
-                    }
-                }
-#pragma unroll
-                for (int ch = 0; ch < 2; ch++) {
-                    if (ch >= nch) continue;
-                    const M3sUnitRec &r = sm.rec[2 * gr + ch];
-                    const bool reord = M3S_UA_BT(r.a) == 2 || M3S_UB_MIXED(r.b);
-                    if (reord) {
-                        const uint32_t d0 = sm.reorder[2 * p], d1 = sm.reorder[2 * p + 1];
-                        sm.xr[ch][d0 & 0x3FFu] = (d0 & 0x8000u) ? (R)0 : val[ch][0];
-                        sm.xr[ch][d1 & 0x3FFu] = (d1 & 0x8000u) ? (R)0 : val[ch][1];
-                    } else {
-                        sm.xr[ch][2 * p] = val[ch][0];
-                        sm.xr[ch][2 * p + 1] = val[ch][1];
-                    }
-                }
-            }
-            __syncthreads();
-            // ------------------------------------------------ alias reduction (long blocks only)
-            for (int aidx = tid; aidx < nch * 248; aidx += HYB_THREADS) {
-                const int ch = aidx >= 248, r_ = aidx - 248 * ch;
-                const M3sUnitRec &r = sm.rec[2 * gr + ch];
-                if (M3S_UA_BT(r.a) == 2 || M3S_UB_MIXED(r.b)) continue;
-                const int sb = 1 + (r_ >> 3), i = r_ & 7;
-                const int o1 = 18 * sb - i - 1, o2 = 18 * sb + i;
-                const R s1 = sm.xr[ch][o1], s2 = sm.xr[ch][o2];
-                sm.xr[ch][o1] = s1 * sm.cs[i] - s2 * sm.ca[i];
-                sm.xr[ch][o2] = s2 * sm.cs[i] + s1 * sm.ca[i];
-            }
-            __syncthreads();
-            // ------------------------------------------------ IMDCT + window + overlap + frequency inversion
-            {
-                const int ch = warp & 1, q = warp >> 1, sb = lane;
-                if (ch < nch) {
-                    const M3sUnitRec &r = sm.rec[2 * gr + ch];
-                    const int bt = M3S_UA_BT(r.a);
-                    const R *pv = sm.prev[pp][ch];
-                    R *pn = sm.prev[pp ^ 1][ch];
-                    if (bt != 2) {
-                        R x[18];
-#pragma unroll
-                        for (int k = 0; k < 18; k++) x[k] = sm.xr[ch][18 * sb + k];
-                        R *ttc = &sm.tt[ch][0][sb];
-                        switch (q) {   // warp-uniform
-                        case 0: imdct_long<R, 0>(x, sm.sine[bt], pv, pn, ttc, sb); break;
-                        case 1: imdct_long<R, 1>(x, sm.sine[bt], pv, pn, ttc, sb); break;
-                        case 2: imdct_long<R, 2>(x, sm.sine[bt], pv, pn, ttc, sb); break;
-                        default: imdct_long<R, 3>(x, sm.sine[bt], pv, pn, ttc, sb); break;
-                        }
-                    } else {
-#pragma unroll
-                        for (int ii = 0; ii < 9; ii++) {
-                            const int i = 9 * q + ii;
-                            R acc = (R)0;
-                            if (i >= 6 && i < 30) {
-                                // three 12-point windows placed at 6/12/18 with overlap (Frame.py:135-148)
-                                const int w_hi = (i - 6) / 6;            // window whose first half covers i
-                                const int i_hi = i - 6 - 6 * w_hi;       // 0..5
-                                if (w_hi < 3) {
-                                    R a2 = (R)0;
-#pragma unroll
-                                    for (int k = 0; k < 6; k++) a2 = fma_t(sm.xr[ch][18 * sb + 6 * w_hi + k], sm.cos12[i_hi][k], a2);
-                                    acc += a2 * sm.sine[2][i_hi];
-                                }
-                                const int w_lo = w_hi - 1;               // window whose second half covers i
-                                if (w_lo >= 0) {
-                                    R a2 = (R)0;
-#pragma unroll
-                                    for (int k = 0; k < 6; k++) a2 = fma_t(sm.xr[ch][18 * sb + 6 * w_lo + k], sm.cos12[i_hi + 6][k], a2);
-                                    acc += a2 * sm.sine[2][i_hi + 6];
-                                }
-                            }
-                            if (i < 18) {
-                                R o = acc + pv[18 * sb + i];
-                                if ((sb & 1) && (i & 1)) o = -o;
-                                sm.tt[ch][i][sb] = o;
-                            } else pn[18 * sb + (i - 18)] = acc;
-                        }
-                    }
-                }
-            }
-            __syncthreads();
-            // ------------------------------------------------ matrixing: the 32 distinct V values of every (channel, slot)
-            for (int cidx = warp; cidx < nch * 18; cidx += HYB_THREADS / 32) {
-                const int ch = cidx / 18, t = cidx - 18 * ch;
-                const R sv = sm.tt[ch][t][lane];
-                const R pr = __shfl_sync(0xFFFFFFFFu, sv, 31 - lane);
-                // lanes 0..15: u[l] = S[l] + S[31 - l]; lanes 16..31: w[31 - l] = S[31 - l] - S[l]
-                sm.uw[warp][lane < 16 ? lane : 47 - lane] = lane < 16 ? sv + pr : pr - sv;
-                __syncwarp();
-                const R *in = sm.uw[warp] + ((lane & 1) ? 16 : 0);   // i(l) has the parity of l
-                R acc = (R)0;
-                if constexpr (sizeof(R) == 4) {
-                    const float4 *s4 = (const float4 *)in;
-#pragma unroll
-                    for (int j4 = 0; j4 < 4; j4++) {
-                        const float4 v4 = s4[j4];
-                        acc = fma_t((R)v4.x, ncoef[4 * j4 + 0], acc);
-                        acc = fma_t((R)v4.y, ncoef[4 * j4 + 1], acc);
-                        acc = fma_t((R)v4.z, ncoef[4 * j4 + 2], acc);
-                        acc = fma_t((R)v4.w, ncoef[4 * j4 + 3], acc);
-                    }
-                } else {
-                    const double2 *s2 = (const double2 *)in;
-#pragma unroll
-                    for (int j2 = 0; j2 < 8; j2++) {
-                        const double2 v2 = s2[j2];
-                        acc = fma_t((R)v2.x, ncoef[2 * j2 + 0], acc);
-                        acc = fma_t((R)v2.y, ncoef[2 * j2 + 1], acc);
-                    }
-                }
-                sm.v[ch][15 + 18 * gr + t][lane] = acc;
-                __syncwarp();
-            }
-            __syncthreads();
-            // ------------------------------------------------ windowing + output: warp = (channel, slot parity, half of the parity's 9 slots)
-            {
-                const int ch = warp >> 2, par = (warp >> 1) & 1, q0 = (warp & 1) ? 5 : 0, nq = (warp & 1) ? 4 : 5;
-                if (ch < nch) {
-                    R out[5];
-                    const R *va0 = &sm.v[ch][15 + 18 * gr + par + 2 * (q0 - 7)][idxA], *vb0 = &sm.v[ch][14 + 18 * gr + par + 2 * (q0 - 7)][idxB];
-                    if (warp & 1) window_tile<R, 4>(va0, vb0, dA, dB, out);
-                    else window_tile<R, 5>(va0, vb0, dA, dB, out);
-                    if (emit) {
-                        const int reps = (meta & M3S_META_DUP) ? 2 : 1;
-                        for (int rep = 0; rep < reps; rep++) {
-                            const int64_t row0 = (g - wk.g_first + rep) * 1152 + gr * 576 + lane;
-#pragma unroll
-                            for (int q = 0; q < 5; q++) {
-                                if (q >= nq) break;
-                                const int64_t e = wk.pcm_elem + (row0 + 32 * (par + 2 * (q0 + q))) * nch + ch;
-                                if (FLOAT_OUT) ((float *)pcm_out)[e] = (float)out[q];
-                                else {
-                                    // (pcm * 32767).astype(int16): truncate toward zero to int32 (0x80000000 outside it), keep the
-                                    // low 16 bits (A.D8)
-                                    const int a = hf_to_int(out[q] * (R)32767);
-                                    ((int16_t *)pcm_out)[e] = (int16_t)(a & 0xFFFF);
-                                }
-                            }
-                        }
-                    }
-                }
-            }
-            // ------------------------------------------------ slide the V history once per frame: slots 36..50 -> 0..14
-            if (gr == 1) {   // granule 0 needs no barrier here: granule 1 writes rows 33..50, nobody reads those yet
-                __syncthreads();
-                for (int idx = tid; idx < nch * 15 * 32; idx += HYB_THREADS) {
-                    const int ch = idx >= 15 * 32, r_ = idx - ch * 15 * 32;
-                    (&sm.v[ch][0][0])[r_] = (&sm.v[ch][36][0])[r_];
-                }
-            }
-            pp ^= 1;   // no barrier needed here: the next readers / writers of these rows sit behind the barriers of the next granule's phases
-        }
-    }
 }
 
 // ================================================================================================
@@ -1755,7 +1371,7 @@ extern "C" int m3s_decode_frame_pos(m3s_handle_t h, int64_t *frame_pos)
     return M3S_OK;
 }
 
-// frames per CTA run of k_hybrid.  Every run pays the CTA's table staging and one warm-up frame (together ~9 % of a 32-frame
+// frames per CTA run of k_hybrid_fast.  Every run pays the CTA's table staging and one warm-up frame (together ~9 % of a 32-frame
 // run), so large batches use long runs; small batches keep runs short enough to fill the SMs (3 CTAs per SM, >= 8 waves of them).
 static int hybrid_run_length(int64_t total_frames, int sm_count)
 {
@@ -1848,15 +1464,6 @@ static int run_enqueue(m3s_ctx *h, M3sScanSet &ss, void *d_pcm, int16_t *d_spect
         M3S_LAUNCH_CHECK(h);
     }
     const bool exact = (flags & M3S_DEC_EXACT) != 0;
-#define M3S_LAUNCH_HYBRID(R, TAB, FL, tabptr)                                                                              \
-    do {                                                                                                                   \
-        const size_t smem = sizeof(HybSmem<R>);                                                                            \
-        M3S_CUDA(h, cudaFuncSetAttribute(k_hybrid<R, TAB, FL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-        M3S_KBEGIN(h, M3S_K_HYBRID);                                                                                       \
-        k_hybrid<R, TAB, FL><<<(unsigned)work.size(), HYB_THREADS, smem, s>>>(                                             \
-            (const uint32_t *)h->b_spec.p, (const M3sUnitRec *)ss.units.p, (const uint8_t *)h->b_sf.p,                     \
-            (const uint32_t *)ss.fr_meta.p, (const M3sWork *)h->b_work.p, h->d_tab, (tabptr), d_pcm);                      \
-    } while (0)
 #define M3S_LAUNCH_HYBRID_FAST1(OUT, FL, NCH, R, TAB, tabptr, first, count)                                                 \
     do {                                                                                                                      \
         const size_t smem = sizeof(HybFastSmem<OUT, R>);                                                                      \
@@ -1873,16 +1480,7 @@ static int run_enqueue(m3s_ctx *h, M3sScanSet &ss, void *d_pcm, int16_t *d_spect
         if (n_stereo > 0) M3S_LAUNCH_HYBRID_FAST1(OUT, FL, 2, R, TAB, tabptr, 0, n_stereo);                                   \
         if (work.size() > n_stereo) M3S_LAUNCH_HYBRID_FAST1(OUT, FL, 1, R, TAB, tabptr, n_stereo, work.size() - n_stereo);    \
     } while (0)
-    if (h->dec_hybrid_direct) {   // A/B and cross-check: the direct-form kernels of round 1 (M3S_HYBRID_DIRECT, read per handle)
-        if (exact) {
-            if (fl) M3S_LAUNCH_HYBRID(double, M3sDevTablesD, true, h->d_tab_f64);
-            else M3S_LAUNCH_HYBRID(double, M3sDevTablesD, false, h->d_tab_f64);
-        } else {
-            if (fl) M3S_LAUNCH_HYBRID(float, M3sDevTables, true, h->d_tab);
-            else M3S_LAUNCH_HYBRID(float, M3sDevTables, false, h->d_tab);
-        }
-        M3S_LAUNCH_CHECK(h);
-    } else if (exact) {
+    if (exact) {
         if (fl) M3S_LAUNCH_HYBRID_FAST(float, true, double, M3sDevTablesD, h->d_tab_f64);
         else M3S_LAUNCH_HYBRID_FAST(int16_t, false, double, M3sDevTablesD, h->d_tab_f64);
     } else {

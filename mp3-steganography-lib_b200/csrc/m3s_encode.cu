@@ -2,8 +2,7 @@
 //
 //   E1 k_enc_analysis_fold  polyphase analysis + MDCT + alias butterflies, exact 32-bit fixed point; also the per-granule
 //                      spectral statistics the rate loop and scfsi need (xrmax, en_tot, en[21]).           (:322-370, :652-758, :817-861)
-//                      The shipped form computes equal truncated products once (generated straight-line code, m3s_enc_fold_gen.cuh);
-//                      k_enc_analysis is the direct form, every product on its own, kept as a cross-check: M3S_ENC_ANALYSIS_DIRECT=1.
+//                      Equal truncated products are computed once (generated straight-line code, m3s_enc_fold_gen.cuh).
 //   E2 the per-granule quantisation / rate loop with table selection and the stego table swap (:760-1264), in three kernels:
 //      k_enc_probe    one warp per granule-channel and NO chain between granules: the reference's step search is walked for every
 //                     payload variant the granule can meet (the <= 3 payload bits at its hide_str_offset: 15 cases), the
@@ -11,7 +10,6 @@
 //      k_enc_resolve  one warp per clip turns offsets into variants in the reference's order (frame, ch, gr) on registers,
 //                     and redoes the few granules that read the slot's stale address1/2/3 (SURVEY A.E5/A.E6);
 //      k_enc_emit     one warp per granule-channel quantises at the chosen step.
-//      (k_enc_rate_chain is the sequential form, one CTA per clip, kept as a cross-check: M3S_ENC_CHAIN=1.)
 //   E3 k_enc_pack      header, side info and Huffman bit packing, one warp per frame (frames are self-contained:
 //                      main_data_begin = 0 and every frame is filled to its nominal size by stuffing).            (:1266-1552)
 //
@@ -62,7 +60,6 @@ struct M3sEncWork {        // E1 work item: a run of granules of one clip
 };
 
 #define ENC_INFO_FIELDS 16
-#define ENC_RUN 36         // granules per E1 CTA (one warm-up granule of filterbank per run: 2.8 %)
 
 struct EncTables {         // small read-only tables of E2/E3, built on the host once per handle
     uint32_t hl4[256];     // code lengths of books 13 | 15 << 8 | 16 << 16 | 24 << 24 at [x * 16 + y]
@@ -80,204 +77,9 @@ __device__ __forceinline__ int32_t mulsr32(int32_t a, int32_t b)  // util.mulsr 
 }
 
 // ================================================================================================
-// E1, direct form (cross-check; the folded form below ships): analysis filterbank + MDCT.  Every product is the reference's
-// mul(a, b) = (a * b) >> 32 truncated on its own (util.py:121-127), so no algebraic folding of the SUMS is exact and the work
-// is 66,816 IMAD.HI per granule-channel; IMAD.HI issues
-// at a quarter of the FP32 rate (tools/ubench_pipes.cu: 29 lanes/clk/SM), which is this kernel's roof.  The design keeps
-// everything else off that pipe's critical path by register tiling: both channels advance together (half the barriers),
-//   windowing   thread (ch, slot parity, i): 16 samples in registers feed 9 slots x 8 taps               (0.22 LDS / mul)
-//   matrixing   thread (ch, slot half, band, row half): 32 matrix coefficients live in registers for the
-//               whole kernel, the windowed vector arrives as broadcast 128-bit loads                      (0.25 LDS / mul)
-//   MDCT        thread (ch, band, k range): cos_l is an immediate constant-bank operand of the IMAD.HI   (0.22 LDS / mul)
-// ================================================================================================
-#define ANA_THREADS 128
-
-__constant__ int32_t c_enc_cos[18][36];   // MP3Encoder.__cos_l (:557-566), window folded in
-
-struct AnaSmem {
-    int32_t x[2][1056];         // [buffer]: 480 samples of history + 576 new of this channel, as int16 << 16 (double buffered: no shift barrier)
-    __align__(16) int32_t y[18][72];   // [slot][i + 4 (i >= 32)] windowed vectors; the gap puts the two halves a matrixing warp reads together on different banks
-    int32_t sb[2][18][32];      // [ping-pong][slot][band] subband samples
-    int32_t mf[576];            // [band * 18 + k] MDCT lines
-    uint32_t bins[24];          // 0..20 band energies, 21 total, 22 xrmax
-    uint32_t en_thresh[32];     // EncTables::en_thresh
-    uint8_t sfb[576];
-    int32_t ca[8], cs[8];
-};
-
-// MDCT of band `lane` for outputs K0 .. K0 + NK - 1: X[k] = sum_j mul(in[j], cos_l[k][j]), in = 18 previous + 18 current
-// subband samples (:683-701)
-template <int K0, int NK>
-__device__ __forceinline__ void mdct_band(const int32_t *__restrict__ prev, const int32_t *__restrict__ cur, int lane,
-                                          int32_t *__restrict__ mf)
-{
-    uint32_t acc[NK];
-#pragma unroll
-    for (int q = 0; q < NK; q++) acc[q] = 0u;
-#pragma unroll
-    for (int j = 0; j < 18; j++) {
-        const int32_t v = prev[j * 32 + lane];
-#pragma unroll
-        for (int q = 0; q < NK; q++) acc[q] += (uint32_t)__mulhi(v, c_enc_cos[K0 + q][j]);
-    }
-#pragma unroll
-    for (int j = 0; j < 18; j++) {
-        const int32_t v = cur[j * 32 + lane];
-#pragma unroll
-        for (int q = 0; q < NK; q++) acc[q] += (uint32_t)__mulhi(v, c_enc_cos[K0 + q][18 + j]);
-    }
-#pragma unroll
-    for (int q = 0; q < NK; q++) mf[lane * 18 + K0 + q] = (int32_t)acc[q];
-}
-
-// One CTA of four warps walks a run of granules of ONE channel of one clip (work item = clip, first granule, count, channel).
-// The small CTA (128 threads, ~21 KB of shared memory) is what lets it share an SM with the rate loop's CTAs of the
-// previous chunk, whose latency-bound chains leave the IMAD.HI pipe idle (see m3s_encode: the two kernels overlap).
-__global__ void __launch_bounds__(ANA_THREADS, 4)
-k_enc_analysis(const int16_t *__restrict__ pcm, const M3sEncClip *__restrict__ clips, const M3sEncWork *__restrict__ work,
-               const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET, int sr_idx, int64_t chunk_frame0,
-               int32_t *__restrict__ mdct, M3sEncStats *__restrict__ stats)
-{
-    __shared__ AnaSmem S;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const M3sEncWork wk = work[blockIdx.x];
-    const M3sEncClip cl = clips[wk.clip];
-    const int ch = wk.ch;
-    for (int i = tid; i < 576; i += ANA_THREADS) S.sfb[i] = T->long_sfb_of[sr_idx][i];
-    if (tid < 8) { S.ca[tid] = T->enc_ca[tid]; S.cs[tid] = T->enc_cs[tid]; }
-    if (tid < 32) S.en_thresh[tid] = ET->en_thresh[tid];
-    for (int i = tid; i < 2 * 18 * 32; i += ANA_THREADS) (&S.sb[0][0][0])[i] = 0;
-    // ---- per-thread roles and their register-resident coefficients
-    const int wpar = tid >> 6, wi = tid & 63;                                  // windowing: slot parity, output i
-    int32_t wcoef[8];
-#pragma unroll
-    for (int k = 0; k < 8; k++) wcoef[k] = T->enwindow[wi + 64 * k];
-    const int mhalf = tid >> 6, mb = (tid & 63) >> 1, mh = tid & 1;            // matrixing: slots 9*mhalf.., band, row half
-    int32_t fl[32];
-#pragma unroll
-    for (int j = 0; j < 32; j++) fl[j] = T->enc_fl[mb][32 * mh + j];
-    __syncthreads();
-
-    const uint32_t *pcm32 = (const uint32_t *)(pcm + cl.pcm_base);  // one stereo sample per word (pcm_base is even)
-    const int sh = ch ? 0 : 16;                                     // channel 0 = low half of the word
-    const int g_begin = wk.g_first > 0 ? wk.g_first - 1 : 0;
-    const int g_end = wk.g_first + wk.count;
-    int pp = 0, xb = 0;
-    uint32_t nx[5] = {0u, 0u, 0u, 0u, 0u};
-    for (int G = g_begin; G < g_end; G++, pp ^= 1, xb ^= 1) {
-        // ---- PCM window: samples [576 G - 480, 576 G + 576); the history comes from the other buffer
-        const int64_t t0 = (int64_t)G * 576 - 480;
-        if (G == g_begin) {
-            for (int i = tid; i < 1056; i += ANA_THREADS) {
-                const int64_t t = t0 + i;
-                const uint32_t w = t >= 0 ? __ldg(pcm32 + t) : 0u;
-                S.x[xb][i] = (int32_t)((w << sh) & 0xFFFF0000u);
-            }
-        } else {
-            for (int i = tid; i < 480; i += ANA_THREADS) S.x[xb][i] = S.x[xb ^ 1][576 + i];
-#pragma unroll
-            for (int q = 0; q < 5; q++) {   // the 576 new samples were fetched during the previous granule
-                const int i = tid + ANA_THREADS * q;
-                if (i < 576) S.x[xb][480 + i] = (int32_t)((nx[q] << sh) & 0xFFFF0000u);
-            }
-        }
-        __syncthreads();
-        if (G + 1 < g_end) {   // prefetch the next granule's samples: their DRAM latency hides under this granule's arithmetic
-#pragma unroll
-            for (int q = 0; q < 5; q++) {
-                const int i = tid + ANA_THREADS * q;
-                if (i < 576) nx[q] = __ldg(pcm32 + (int64_t)(G + 1) * 576 + i);
-            }
-        }
-        // ---- windowing: y_s[i] = sum_k mul(x[32 s + 31 - i - 64 k], enwindow[i + 64 k])   (:337-356).  Slots s = p + 2 q of one
-        //      parity share their samples: x index = base + 64 (q - k), 16 distinct values for 9 slots x 8 taps
-        {
-            const int32_t *xp = &S.x[xb][480 + 32 * wpar + 31 - wi];
-            int32_t xv[16];
-#pragma unroll
-            for (int d = 0; d < 16; d++) xv[d] = xp[64 * (d - 7)];
-#pragma unroll
-            for (int q = 0; q < 9; q++) {
-                uint32_t acc = 0;
-#pragma unroll
-                for (int k = 0; k < 8; k += 2)
-                    acc += (uint32_t)__mulhi(xv[q - k + 7], wcoef[k]) + (uint32_t)__mulhi(xv[q - k + 6], wcoef[k + 1]);
-                S.y[wpar + 2 * q][wi + ((wi >> 5) << 2)] = (int32_t)acc;
-            }
-        }
-        __syncthreads();
-        // ---- matrixing: s_b = sum_j mul(fl[b][j], y_j); odd bands of odd slots negated   (:358-368, :678-679)
-#pragma unroll 1
-        for (int q = 0; q < 9; q++) {
-            const int s = 9 * mhalf + q;
-            const int4 *y4 = (const int4 *)&S.y[s][36 * mh];
-            uint32_t acc = 0;
-#pragma unroll
-            for (int m = 0; m < 8; m++) {
-                const int4 yv = y4[m];
-                acc += (uint32_t)__mulhi(fl[4 * m + 0], yv.x) + (uint32_t)__mulhi(fl[4 * m + 1], yv.y);
-                acc += (uint32_t)__mulhi(fl[4 * m + 2], yv.z) + (uint32_t)__mulhi(fl[4 * m + 3], yv.w);
-            }
-            acc += __shfl_xor_sync(0xFFFFFFFFu, acc, 1);
-            if (mh == 0) {
-                if ((s & 1) && (mb & 1)) acc = 0u - acc;
-                S.sb[pp][s][mb] = (int32_t)acc;
-            }
-        }
-        __syncthreads();
-        if (G < wk.g_first) continue;   // warm-up granule: only its subband samples are needed (block-uniform)
-        // ---- MDCT   (:683-701): warp = k range, lane = band
-        {
-            const int32_t *prev = &S.sb[pp ^ 1][0][0], *cur = &S.sb[pp][0][0];
-            switch (warp) {   // warp-uniform
-            case 0: mdct_band<0, 5>(prev, cur, lane, S.mf); break;
-            case 1: mdct_band<5, 5>(prev, cur, lane, S.mf); break;
-            case 2: mdct_band<10, 4>(prev, cur, lane, S.mf); break;
-            default: mdct_band<14, 4>(prev, cur, lane, S.mf); break;
-            }
-            if (tid < 24) S.bins[tid] = 0u;
-        }
-        __syncthreads();
-        // ---- alias butterflies between neighbouring bands, cmuls with >> 31   (:704-744, util.py:145-155)
-        for (int r = tid; r < 248; r += ANA_THREADS) {
-            const int band = 1 + (r >> 3), k = r & 7;
-            const int64_t are = S.mf[band * 18 + k], aim = S.mf[(band - 1) * 18 + 17 - k];
-            const int64_t bre = S.cs[k], bim = S.ca[k];
-            S.mf[band * 18 + k] = (int32_t)((are * bre - aim * bim) >> 31);
-            S.mf[(band - 1) * 18 + 17 - k] = (int32_t)((are * bim + aim * bre) >> 31);
-        }
-        __syncthreads();
-        // ---- store + statistics: xrmax, en_tot, en[sfb]   (:772-776, :836-857)
-        const int frame = G >> 1, gr = G & 1;
-        const int64_t gslot = (((int64_t)(cl.frame_base + frame) - chunk_frame0) * 2 + ch) * 2 + gr;
-        for (int i = tid; i < 576; i += ANA_THREADS) {   // 576 = 18 * 32: whole warps
-            const int32_t v = S.mf[i];
-            mdct[gslot * 576 + i] = v;
-            const uint32_t e = (uint32_t)(mulsr32(v, v) >> 10);
-            const int sfb = S.sfb[i];
-            if (sfb < 21 && e) atomicAdd(&S.bins[sfb], e);
-            const uint32_t a = v < 0 ? (uint32_t)(-(int64_t)v) : (uint32_t)v;
-            const uint32_t tot = __reduce_add_sync(0xFFFFFFFFu, e), mx = __reduce_max_sync(0xFFFFFFFFu, a);
-            if (lane == 0) { atomicAdd(&S.bins[21], tot); atomicMax(&S.bins[22], mx); }
-        }
-        __syncthreads();
-        if (tid < 22) {
-            const uint32_t temp = S.bins[tid];
-            int en = 0;
-            if (temp) {
-                en = -21;
-                for (int j = 0; j < 31; j++) en += S.en_thresh[j] <= temp;
-            }
-            M3sEncStats *st = stats + gslot;
-            if (tid == 21) { st->en_tot = (int8_t)en; st->xrmax = (int32_t)S.bins[22]; }
-            else st->en[tid] = (int8_t)en;
-        }
-        // no barrier: the next writers of bins (MDCT phase of the next granule) sit behind three barriers
-    }
-}
-
-// ================================================================================================
-// E1, folded form (the one that ships; M3S_ENC_ANALYSIS_DIRECT=1 selects the kernel above as a cross-check).
+// E1: analysis filterbank + MDCT, folded.  Every product is the reference's mul(a, b) = (a * b) >> 32 truncated on its own
+// (util.py:121-127), so no algebraic folding of the SUMS is exact: done directly, that is 66,816 IMAD.HI per granule-channel on a pipe
+// that issues 29 lanes/clk/SM (tools/ubench_pipes.cu).
 //
 // The matrixing's 32 x 64 matrix holds cosines of a 128-point grid: a column carries at most 16 distinct magnitudes (920 distinct
 // (|v|, j) pairs for 2,025 non-zero entries), and  mul(-v, y) = -mul(v, y) - [(v y) mod 2^32 != 0].  So ONE truncated product per
@@ -297,6 +99,8 @@ k_enc_analysis(const int16_t *__restrict__ pcm, const M3sEncClip *__restrict__ c
 // 2 CTAs: **46.4** (0.14); 16 warps x 1 CTA: 52.6 (nothing left to cover the barriers).  Barriers inside the straight-line code
 // to keep the warps aligned did not help (47.6 - 51.2).
 // ================================================================================================
+__constant__ int32_t c_enc_cos[18][36];   // MP3Encoder.__cos_l (:557-566), window folded in, for the MDCT's correction pass
+
 #define M3S_FOLD_FN __device__ __forceinline__
 #define M3S_FOLD_MULHI(a, b) __mulhi((a), (b))
 #include "m3s_enc_fold_gen.cuh"
@@ -304,17 +108,17 @@ k_enc_analysis(const int16_t *__restrict__ pcm, const M3sEncClip *__restrict__ c
 __constant__ int32_t c_enc_fl[32][64];    // MP3Encoder filter matrix (:544-555) and analysis window (tables.py:34-78) for the
 __constant__ int32_t c_enc_win[512];      // correction pass of a slot whose fast path reported `bad`
 
-template <int WARPS>   // warps per CTA = 32-slot groups per block
+#define ANA3_WARPS 8   // warps per CTA = 32-slot groups per block (8 warps x 2 CTAs per SM, see above)
 struct Ana3Smem {
-    static constexpr int SLOTS = 32 * WARPS;   // slots per block: one per thread
+    static constexpr int SLOTS = 32 * ANA3_WARPS;   // slots per block: one per thread
     static constexpr int XP = 15 + SLOTS;      // columns of the sample tile: 15 slots of history + the block's slots; odd: conflict-free fills
     static constexpr int RING = (SLOTS + 35 + 17) / 18 * 18;   // subband-sample ring: a granule reaches back 36 slots from its end, a block adds
                                                                // SLOTS more; a multiple of 18, so that the rows of a granule never wrap
     static constexpr int RUN = SLOTS * 9 / 18 - 1;   // granules per CTA: with the warm-up granule 9 blocks exactly
     int32_t xT[32][XP];                // sample 32 u + r of this channel at [r][u - u0], as int16 << 16
     int32_t sb[RING + 18][33];         // [ring row][band] subband samples; rows RING.. stay zero (the granule in front of a clip)
-    int32_t mf[WARPS][576];            // per warp: [band * 18 + k] MDCT lines of the granule it works on
-    uint32_t bins[WARPS][24];          // per warp: 0..20 band energies, 21 total, 22 xrmax
+    int32_t mf[ANA3_WARPS][576];       // per warp: [band * 18 + k] MDCT lines of the granule it works on
+    uint32_t bins[ANA3_WARPS][24];     // per warp: 0..20 band energies, 21 total, 22 xrmax
     uint32_t en_thresh[32];
     uint8_t sfb[576];
     int32_t ca[8], cs[8];
@@ -333,16 +137,16 @@ struct Ana3LoadSb {  // input j of the MDCT: slot j of the previous granule (j <
     __device__ __forceinline__ int32_t operator()(int j) const { return j < 18 ? prev[j * 33] : cur[(j - 18) * 33]; }
 };
 
-// GUARD: how shared products are protected from ptxas's multiply-add folding (m3s_enc_fold_gen.cuh); WARPS: warps per CTA
-template <int GUARD, int WARPS>
-__global__ void __launch_bounds__(32 * WARPS, 16 / WARPS)
+// `zero` (always 0) is added to every shared product (guard 0 of m3s_enc_fold_gen.cuh): ptxas cannot see through it, so it keeps
+// each product once instead of recomputing it per use, and the add folds into the multiply's addend
+__global__ void __launch_bounds__(32 * ANA3_WARPS, 2)
 k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restrict__ clips, const M3sEncWork *__restrict__ work,
                     const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET, int sr_idx, int64_t chunk_frame0,
                     int32_t *__restrict__ mdct, M3sEncStats *__restrict__ stats, const uint32_t zero)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef Ana3Smem<WARPS> Smem;
-    constexpr int ANA3_WARPS = WARPS, ANA3_THREADS = 32 * WARPS, ANA3_SLOTS = Smem::SLOTS, ANA3_XP = Smem::XP, ANA3_RING = Smem::RING;
+    typedef Ana3Smem Smem;
+    constexpr int ANA3_THREADS = 32 * ANA3_WARPS, ANA3_SLOTS = Smem::SLOTS, ANA3_XP = Smem::XP, ANA3_RING = Smem::RING;
     Smem &S = *reinterpret_cast<Smem *>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const M3sEncWork wk = work[blockIdx.x];
@@ -391,7 +195,7 @@ k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restric
         if (t0 + 32 * warp < t_stop) {   // warp-uniform
             uint32_t acc[32], bad, any;
             const Ana3LoadX<ANA3_XP> ld{&S.xT[0][15 + tid]};
-            m3s_matrix_fold<GUARD>(ld, zero, acc, bad, any);
+            m3s_matrix_fold<0>(ld, zero, acc, bad, any);
             if (bad) {   // some y has 26 zero low bits: its negative uses were charged a correction they may not owe
                 if (any == 0u) {
 #pragma unroll
@@ -428,7 +232,7 @@ k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restric
             {
                 uint32_t acc[18], bad, any;
                 const Ana3LoadSb ld{&S.sb[G == 0 ? ANA3_RING : (18 * (G - 1) - t_begin) % ANA3_RING][lane], &S.sb[(18 * G - t_begin) % ANA3_RING][lane]};
-                m3s_mdct_fold<GUARD>(ld, zero, acc, bad, any);
+                m3s_mdct_fold<0>(ld, zero, acc, bad, any);
                 if (bad) {
                     if (any == 0u) {
 #pragma unroll
@@ -495,17 +299,11 @@ k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restric
 }
 
 // ================================================================================================
-// E2: the probe machinery shared by every form of the rate loop, and its sequential form k_enc_rate_chain (one CTA per clip)
+// E2, shared pieces: the reference's step search on shared-memory tables (the slow path of k_enc_resolve, the quantiser of k_enc_emit)
 // ================================================================================================
-#define RATE_WARPS 2       // warps per clip of the sequential form: warp w owns granule index gr = w of every frame (see k_enc_rate_chain)
-
 struct RateSmem {
     uint16_t i2i[10000];
     uint2 hlc[256];        // .x = hl4 (code lengths of books 13 | 15 << 8 | 16 << 16 | 24 << 24), .y = signs | escapes << 16 of the pair
-    int32_t slot[4][4];    // per (gr, ch) slot: address1..3 (stale when big_values == 0, A.E6), quantizerStepSize
-    int32_t cnt[2][2];     // [round parity][gr] payload bits the granule consumed
-    int32_t p23[2][4];     // [frame parity][slot] part2_3_length before resv_frame_end
-    int32_t prec[16][24];  // probes of warp 1's speculative run: step, then the Pooled words (replayed when the speculation fails)
     int32_t steptabi[128];
     double steptab[128];
     uint16_t sfb[24];
@@ -573,13 +371,11 @@ __device__ __forceinline__ int choose_table(const RateSmem &S, int mx, uint32_t 
 
 // Everything a probe derives from the quantised values WITHOUT looking at the payload bits: run lengths, count1 bits, region
 // bounds and, per region, the maximum and the pooled code-length / sign / escape sums.  The table choice (with the stego swap)
-// and the bit count follow from it in a few scalar steps (probe_tables), which is what lets a mispredicted granule be replayed
-// from its recorded probes instead of re-running them (k_enc_rate_chain).
+// and the bit count follow from it in a few scalar steps (probe_tables).
 struct Pooled {
     int c1bits, c1sel, bv, count1, r0, r1, a1, a2, a3;
     uint32_t m0, m1, m2, lo0, hi0, cn0, lo1, hi1, cn1, lo2, hi2, cn2;
 };
-#define POOLED_WORDS 21
 
 // calc_run_len + count1_bit_count + subdivide + the pooled sums of big_v_tab_select / big_v_bit_count for the quantised values
 // held pair-interleaved in the warp (lane L holds pairs 32 j + L).  a1..a3 come in as the slot's current addresses.
@@ -700,29 +496,7 @@ __device__ __forceinline__ void quantize_all(const RateSmem &S, const uint32_t (
     }
 }
 
-// quantize() when the largest coefficient stays below the table limit (ln < 10000 for every value): no fallback, no clamp
-__device__ __forceinline__ void quantize_small(const RateSmem &S, const uint32_t (&ax)[9], const uint32_t (&ay)[9], int step,
-                                               uint32_t (&qx)[9], uint32_t (&qy)[9])
-{
-    const int32_t scalei = S.steptabi[step + 127];
-#pragma unroll
-    for (int j = 0; j < 9; j++) {
-        qx[j] = S.i2i[mulr32((int32_t)ax[j], scalei)];
-        qy[j] = S.i2i[mulr32((int32_t)ay[j], scalei)];
-    }
-}
-
-// payload bits a granule starting at payload offset `off` can consume: bits[off .. off + 2]   (:1154-1168)
-__device__ __forceinline__ void payload_bits_at(const uint8_t *__restrict__ payload, const M3sEncClip &cl, int64_t off, int lane,
-                                                int &hn, uint32_t &hb)
-{
-    const int64_t left = cl.payload_len - off;
-    hn = left > 3 ? 3 : (left < 0 ? 0 : (int)left);
-    const bool one = lane < hn && __ldg(payload + cl.payload_base + off + lane) == '1';
-    hb = __ballot_sync(0xFFFFFFFFu, one);
-}
-
-// the shared-memory tables of the rate loop (all kernels of E2 stage the same set)
+// the shared-memory tables of k_enc_resolve and k_enc_emit
 __device__ __forceinline__ void rate_tables_load(RateSmem &S, const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET,
                                                  int sr_idx, int tid, int nthr)
 {
@@ -743,238 +517,8 @@ __device__ __forceinline__ void rate_tables_load(RateSmem &S, const M3sDevTables
     if (tid < 16) { S.hlc1[0][tid] = ET->hlc1[0][tid]; S.hlc1[1][tid] = ET->hlc1[1][tid]; }
 }
 
-// One CTA of two warps per clip.  The reference visits a frame's granules as (ch0,gr0) (ch0,gr1) (ch1,gr0) (ch1,gr1) and
-// chains them through hide_str_offset (which payload bits a granule may consume) and through the per-slot stale
-// address1..3 / step.  Warp w owns granule index gr = w, so the slot state never leaves its warp; within a channel the
-// two granules run CONCURRENTLY: warp 0 with the exact offset, warp 1 speculating that granule 0 consumes three bits (one
-// per non-empty region; none if granule 0 is silent).  A granule depends on its offset only through the <= 3 bits it
-// reads, so after warp 0 publishes its count warp 1 keeps its result when the bits at the true offset equal the ones it
-// used and re-runs otherwise (the tone+noise corpus mispredicts 1-2 % of the granules, low tones up to 27 %).
-__global__ void __launch_bounds__(32 * RATE_WARPS, 11)
-k_enc_rate_chain(const M3sEncClip *__restrict__ clips, M3sEncState *__restrict__ states, const M3sDevTables *__restrict__ T,
-           const EncTables *__restrict__ ET, const uint32_t *__restrict__ byteoff, const uint8_t *__restrict__ payload,
-           int sr_idx, int whole_slots, int32_t chunk_first, int32_t chunk_frames, int64_t chunk_frame0,
-           const int32_t *__restrict__ mdct, const M3sEncStats *__restrict__ stats, uint32_t *__restrict__ ixout,
-           int32_t *__restrict__ info, uint8_t *__restrict__ scfsi_out, uint32_t *__restrict__ last_ix)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    RateSmem &S = *reinterpret_cast<RateSmem *>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, gr = tid >> 5;
-    const uint32_t FULL = 0xFFFFFFFFu;
-    const int c = blockIdx.x;
-    const M3sEncClip cl = clips[c];
-    rate_tables_load(S, T, ET, sr_idx, tid, 32 * RATE_WARPS);
-    if (tid < 4) {
-        const M3sEncState *sp = states + c;
-        S.slot[tid][0] = sp->a1[tid]; S.slot[tid][1] = sp->a2[tid]; S.slot[tid][2] = sp->a3[tid]; S.slot[tid][3] = sp->step[tid];
-    }
-    int64_t off = states[c].hide_off;   // MP3Encoder.hide_str_offset, tracked identically by both warps
-    __syncthreads();
-
-    const bool hiding = cl.payload_len > 0;
-    const int f_end = min(cl.n_frames, chunk_first + chunk_frames);
-    int round = 0;
-    for (int f = chunk_first; f < f_end; f++) {
-        const int padding = (int)(byteoff[f + 1] - byteoff[f]) - whole_slots;
-        const int bits_per_frame = 8 * (whole_slots + padding);
-        const int mean_bits = (bits_per_frame - 288) / 2;          // :634-636 (side info 8 * (4 + 32) bits)
-        const int max_bits = min(mean_bits / 2, 4095);             // :894-912 with the reservoir never enabled (A.E7)
-        const int64_t fl_ = cl.frame_base + f - chunk_frame0;      // frame slot in the chunk buffers
-#pragma unroll 1
-        for (int ch = 0; ch < 2; ch++, round ^= 1) {
-            const int slot = 2 * gr + ch;
-            const int64_t gslot = (fl_ * 2 + ch) * 2 + gr;
-            const int2 *xr = (const int2 *)(mdct + gslot * 576);
-            uint32_t ax[9], ay[9], sg = 0;
-#pragma unroll
-            for (int j = 0; j < 9; j++) {
-                const int2 v = __ldg(xr + 32 * j + lane);
-                ax[j] = v.x < 0 ? (uint32_t)(-(int64_t)v.x) : (uint32_t)v.x;
-                ay[j] = v.y < 0 ? (uint32_t)(-(int64_t)v.y) : (uint32_t)v.y;
-                sg |= (uint32_t)(v.x < 0) << (2 * j) | (uint32_t)(v.y < 0) << (2 * j + 1);
-            }
-            const int32_t xrmax = stats[gslot].xrmax;
-            // granule 1 starts where granule 0 of the same channel ends: predicted as three bits past `off` (none when it is silent)
-            int64_t use_off = off;
-            if (gr == 1 && stats[gslot - 1].xrmax) use_off += 3;
-            GranInfo gi;
-            int a1 = 0, a2 = 0, a3 = 0, step = 0, part23 = 0, cnt = 0, hn = 0, nrec = 0, qstep = 1000;
-            uint32_t hb = 0, qx[9], qy[9];
-            bool need = true;
-#pragma unroll 1
-            for (int attempt = 0; attempt < 2; attempt++) {
-                if (need) {
-                    gi.bv = 0; gi.count1 = 0; gi.c1sel = 0; gi.r0 = 0; gi.r1 = 0; gi.ts0 = 0; gi.ts1 = 0; gi.ts2 = 0;
-                    a1 = S.slot[slot][0]; a2 = S.slot[slot][1]; a3 = S.slot[slot][2]; step = S.slot[slot][3];
-                    part23 = 0; cnt = 0;
-                    if (xrmax) {
-                        if (hiding) payload_bits_at(payload, cl, use_off, lane, hn, hb);
-                        // warp 1 records the payload-independent part of every probe of its speculative run; if the speculation
-                        // fails, the second run replays them (a few scalar steps per probe) for as long as it follows the same path
-                        const bool record = gr == 1 && attempt == 0 && hiding;
-                        bool replay = attempt == 1;
-                        int ridx = 0;
-                        if (record) nrec = 0;
-                        // ---- bin_search_step_size (:958-996) then inner_loop (:1064-1095), as one loop with a single probe site
-                        int next = -120, count = 120, half = 0, bits = 0, s = 0;
-                        bool in_bin = true;
-                        for (;;) {
-                            bool ovf = false;
-                            if (in_bin) {
-                                half = count / 2;
-                                s = next + half;
-                                ovf = quant_max(S, xrmax, s) > 8192;
-                            } else {
-                                while (quant_max(S, xrmax, step + 1) > 8192) step++;
-                                step++;
-                                s = step;
-                            }
-                            bits = 100000;
-                            if (!ovf) {
-                                Pooled P;
-                                if (replay && ridx < min(nrec, 16) && S.prec[ridx][0] == s) {
-                                    const int32_t *w = S.prec[ridx] + 1;
-                                    P.c1bits = w[0]; P.c1sel = w[1]; P.bv = w[2]; P.count1 = w[3]; P.r0 = w[4]; P.r1 = w[5];
-                                    P.a1 = w[6]; P.a2 = w[7]; P.a3 = w[8];
-                                    P.m0 = w[9]; P.m1 = w[10]; P.m2 = w[11]; P.lo0 = w[12]; P.hi0 = w[13]; P.cn0 = w[14];
-                                    P.lo1 = w[15]; P.hi1 = w[16]; P.cn1 = w[17]; P.lo2 = w[18]; P.hi2 = w[19]; P.cn2 = w[20];
-                                    ridx++;
-                                } else {
-                                    replay = false;
-                                    quantize_all(S, ax, ay, s, qx, qy);
-                                    qstep = s;
-                                    probe_pool(S, qx, qy, lane, a1, a2, a3, P);
-                                    if (record) {
-                                        if (nrec < 16 && lane == 0) {
-                                            int32_t *w = S.prec[nrec];
-                                            w[0] = s;
-                                            w[1] = P.c1bits; w[2] = P.c1sel; w[3] = P.bv; w[4] = P.count1; w[5] = P.r0; w[6] = P.r1;
-                                            w[7] = P.a1; w[8] = P.a2; w[9] = P.a3;
-                                            w[10] = (int32_t)P.m0; w[11] = (int32_t)P.m1; w[12] = (int32_t)P.m2;
-                                            w[13] = (int32_t)P.lo0; w[14] = (int32_t)P.hi0; w[15] = (int32_t)P.cn0;
-                                            w[16] = (int32_t)P.lo1; w[17] = (int32_t)P.hi1; w[18] = (int32_t)P.cn1;
-                                            w[19] = (int32_t)P.lo2; w[20] = (int32_t)P.hi2; w[21] = (int32_t)P.cn2;
-                                        }
-                                        nrec++;
-                                    }
-                                }
-                                a1 = P.a1; a2 = P.a2; a3 = P.a3;
-                                bits = probe_tables(S, P, hiding, hn, hb, gi);
-                            }
-                            if (in_bin) {
-                                if (bits < max_bits) count = half;
-                                else { next += half; count -= half; }
-                                if (count <= 1) { in_bin = false; step = next; }
-                            } else if (bits <= max_bits) break;
-                        }
-                        if (qstep != s) {   // the run ended on a replayed probe: the registers hold another step's values
-                            quantize_all(S, ax, ay, s, qx, qy);
-                            qstep = s;
-                        }
-                        part23 = bits;
-                        cnt = (gi.ts0 > 0) + (gi.ts1 > 0) + (gi.ts2 > 0);   // :808-809
-                    }
-                }
-                if (attempt == 0) {
-                    if (gr == 0 && lane == 0) S.cnt[round][0] = cnt;
-                    __syncthreads();
-                    need = false;
-                    if (gr == 1 && hiding && xrmax) {
-                        const int64_t actual = off + S.cnt[round][0];
-                        if (actual != use_off) {
-                            int hn2;
-                            uint32_t hb2;
-                            payload_bits_at(payload, cl, actual, lane, hn2, hb2);
-                            need = hn2 != hn || hb2 != hb;
-                            use_off = actual;
-                        }
-                    }
-                }
-            }
-            // ---- results of this granule
-            uint32_t *ixd = ixout + gslot * 288;
-            if (xrmax) {
-                // signed ix as format_bitstream leaves it (:1272-1276)
-#pragma unroll
-                for (int j = 0; j < 9; j++) {
-                    const int vx = ((sg >> (2 * j)) & 1u) ? -(int)qx[j] : (int)qx[j];
-                    const int vy = ((sg >> (2 * j + 1)) & 1u) ? -(int)qy[j] : (int)qy[j];
-                    ixd[32 * j + lane] = ((uint32_t)vx & 0xFFFFu) | ((uint32_t)vy << 16);
-                }
-            } else {
-                // silent granule: l3_enc keeps the previous frame's values of this slot (never coded: big_values = count1 = 0)
-                const uint32_t *src = f > chunk_first ? ixout + (gslot - 4) * 288
-                                                      : (f > 0 ? last_ix + ((int64_t)c * 4 + (2 * ch + gr)) * 288 : nullptr);
-#pragma unroll
-                for (int j = 0; j < 9; j++) ixd[32 * j + lane] = src ? src[32 * j + lane] : 0u;
-            }
-            if (lane == 0) {
-                S.slot[slot][0] = a1; S.slot[slot][1] = a2; S.slot[slot][2] = a3; S.slot[slot][3] = step;
-                S.p23[f & 1][slot] = part23;
-                if (gr == 1) S.cnt[round][1] = cnt;
-                int32_t *r = info + (fl_ * 4 + slot) * ENC_INFO_FIELDS;   // info layout [frame][gr][ch] == slot order
-                r[1] = gi.bv; r[2] = gi.count1; r[3] = step + 210; r[4] = gi.ts0; r[5] = gi.ts1; r[6] = gi.ts2;
-                r[7] = gi.r0; r[8] = gi.r1; r[9] = gi.c1sel; r[10] = a1; r[11] = a2; r[12] = a3; r[13] = step; r[14] = padding;
-            }
-            __syncthreads();
-            off += S.cnt[round][0] + S.cnt[round][1];
-        }
-        // ---- calc_scfsi (:862-892), warp w takes channel w: needs the statistics of both granules
-        {
-            const M3sEncStats *s0 = stats + (fl_ * 2 + gr) * 2, *s1 = s0 + 1;
-            const int d = lane < 21 ? abs((int)s0->en[lane] - (int)s1->en[lane]) : 0;
-            const int tp = __reduce_add_sync(FULL, d);
-            int condition = 2 + (s0->xrmax != 0) + (s1->xrmax != 0);
-            if (abs((int)s0->en_tot - (int)s1->en_tot) < 10) condition++;
-            if (tp < 100) condition++;
-            const int b0 = __reduce_add_sync(FULL, lane < 6 ? d : 0), b1 = __reduce_add_sync(FULL, lane >= 6 && lane < 11 ? d : 0);
-            const int b2 = __reduce_add_sync(FULL, lane >= 11 && lane < 16 ? d : 0), b3 = __reduce_add_sync(FULL, lane >= 16 ? d : 0);
-            if (lane < 4) {
-                const int sum0 = lane == 0 ? b0 : (lane == 1 ? b1 : (lane == 2 ? b2 : b3));
-                scfsi_out[(fl_ * 2 + gr) * 4 + lane] = (condition == 6 && sum0 < 10) ? 1 : 0;   // xm[] is all zero: sum1 = 0
-            }
-        }
-        // ---- resv_frame_end (:1097-1145): every unused bit of the frame becomes stuffing
-        if (tid == 0) {
-            int p23[4];
-            int stuffing = 0;
-            for (int q = 0; q < 4; q++) { p23[q] = S.p23[f & 1][q]; stuffing += mean_bits / 2 - p23[q]; }   // :812 (mean_bits is even)
-            if (stuffing > 0) {
-                if (p23[0] + stuffing < 4095) p23[0] += stuffing;
-                else {
-                    for (int q = 0; q < 4 && stuffing > 0; q++) {   // gr0ch0, gr0ch1, gr1ch0, gr1ch1 == slot order
-                        const int t = min(4095 - p23[q], stuffing);
-                        p23[q] += t;
-                        stuffing -= t;
-                    }
-                }
-            }
-            for (int q = 0; q < 4; q++) {
-                int32_t *r = info + (fl_ * 4 + q) * ENC_INFO_FIELDS;
-                r[0] = p23[q];
-                r[15] = (int32_t)off;
-            }
-        }
-    }
-    // ---- hand the state to the next chunk
-    if (f_end > chunk_first && f_end < cl.n_frames) {
-        const int64_t fl_ = cl.frame_base + (f_end - 1) - chunk_frame0;
-        for (int ch = 0; ch < 2; ch++) {
-            const uint32_t *src = ixout + ((fl_ * 2 + ch) * 2 + gr) * 288;
-            uint32_t *dst = last_ix + ((int64_t)c * 4 + (2 * ch + gr)) * 288;
-            for (int j = 0; j < 9; j++) dst[32 * j + lane] = src[32 * j + lane];
-        }
-    }
-    __syncthreads();
-    if (tid < 4) {
-        M3sEncState *sp = states + c;
-        sp->a1[tid] = S.slot[tid][0]; sp->a2[tid] = S.slot[tid][1]; sp->a3[tid] = S.slot[tid][2]; sp->step[tid] = S.slot[tid][3];
-        if (tid == 0) sp->hide_off = off;
-    }
-}
-
 // ================================================================================================
-// E2 (parallel form): k_enc_probe -> k_enc_resolve -> k_enc_emit
+// E2: k_enc_probe -> k_enc_resolve -> k_enc_emit
 //
 // A granule depends on its predecessors only through (a) the <= 3 payload bits at its hide_str_offset -- i.e. through one of
 // 15 "variants": three bits (8), two (4) or one (2) left before the payload ends, or none -- and (b) the slot's stale
@@ -988,6 +532,7 @@ k_enc_rate_chain(const M3sEncClip *__restrict__ clips, M3sEncState *__restrict__
 //                  stale addresses (flagged by the probe kernel) are redone here with the true state;
 //   k_enc_emit     one warp per granule quantises at the chosen step and writes the values the packer reads.
 // ================================================================================================
+#define PROBE_WARPS 8        // warps per CTA of k_enc_probe, two CTAs per SM (128 registers a thread)
 #define PROBE_G 8            // granules per warp of k_enc_probe (amortises the CTA's table staging)
 #define PROBE_CACHE 24       // distinct steps cached per granule; more than that (never seen) sends the granule to the resolve kernel
 #define VAR_SILENT 0x80000000u
@@ -1062,10 +607,9 @@ struct ProbeTab {
     uint32_t subdiv[289];    // subdivide() by big_values: region0_count | region1_count << 4 | address1 << 8 | address2 << 18
     uint32_t c1cost[256];    // count1 quads two at a time: sum over the byte's two 4-bit patterns of (table A bits | table B bits << 16)
 };
-template <int NW>
 struct ProbeSmem {
     ProbeTab T;
-    ProbeWarpSmem W[NW];
+    ProbeWarpSmem W[PROBE_WARPS];
 };
 
 __device__ __forceinline__ uint32_t i2x_entry(uint32_t q)
@@ -1256,15 +800,14 @@ __device__ __forceinline__ bool probe_row(const ProbeTab &T, const uint32_t (&ax
     return true;
 }
 
-template <int PROBE_WARPS, int MIN_CTAS>
-__global__ void __launch_bounds__(32 * PROBE_WARPS, MIN_CTAS)
+__global__ void __launch_bounds__(32 * PROBE_WARPS, 2)
 k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ frame_clip, const M3sDevTables *__restrict__ DT,
             const EncTables *__restrict__ ET, const uint32_t *__restrict__ byteoff, int sr_idx, int whole_slots, int64_t n_gran,
             const int32_t *__restrict__ mdct, const M3sEncStats *__restrict__ stats, uint4 *__restrict__ var,
             uint32_t *__restrict__ sum, uint8_t *__restrict__ scfsi_out)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    ProbeSmem<PROBE_WARPS> &PS = *reinterpret_cast<ProbeSmem<PROBE_WARPS> *>(smem_raw);
+    ProbeSmem &PS = *reinterpret_cast<ProbeSmem *>(smem_raw);
     ProbeTab &T = PS.T;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t FULL = 0xFFFFFFFFu;
@@ -1307,13 +850,11 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
     int vhn;
     uint32_t vhb;
     variant_bits(lane, vhn, vhb);
-    // tiles of PROBE_WARPS * PROBE_G granules; a grid smaller than the tile count walks them with a stride (M3S_PROBE_CTAS)
-    const int64_t n_iter = ((n_gran + PROBE_WARPS * PROBE_G - 1) / (PROBE_WARPS * PROBE_G) - blockIdx.x + gridDim.x - 1) / gridDim.x * PROBE_G;
+    // one tile of PROBE_WARPS * PROBE_G granules per CTA: warp w takes granules w, w + PROBE_WARPS, ... of tile blockIdx.x
 #pragma unroll 1
-    for (int64_t it = 0; it < n_iter; it++) {
-        const int64_t tile = blockIdx.x + (it / PROBE_G) * gridDim.x;
-        const int64_t gs = tile * (PROBE_WARPS * PROBE_G) + warp + (it % PROBE_G) * PROBE_WARPS;
-        if (gs >= n_gran) continue;
+    for (int it = 0; it < PROBE_G; it++) {
+        const int64_t gs = (int64_t)blockIdx.x * (PROBE_WARPS * PROBE_G) + warp + it * PROBE_WARPS;
+        if (gs >= n_gran) break;
         const int64_t fl_ = gs >> 2;
         const int q = (int)(gs & 3);                         // position in the reference's order: (ch0,gr0) (ch0,gr1) (ch1,gr0) (ch1,gr1)
         const int c = frame_clip[fl_];
@@ -2127,8 +1668,6 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     M3S_CUDA(h, cudaMemsetAsync(h->e_state.p, 0, sizeof(M3sEncState) * n_clips, h->stream));
     const size_t lastix_bytes = (size_t)n_clips * 4 * 288 * 4;
     if ((rc = m3s_buf_reserve(h, h->e_lastix, 2 * lastix_bytes))) return rc;   // two sets: chunk k reads set k & 1 and writes the other
-    // M3S_ENC_CHAIN=1 selects the sequential form of the rate loop (one CTA per clip walking its granules in order)
-    const bool chain = getenv("M3S_ENC_CHAIN") != nullptr;
 
     // ---- chunking: all clips advance together through windows of `cf` frames so that the intermediates
     //      (MDCT spectra 9.2 KB/frame, quantised values 4.6 KB/frame) stay bounded while every clip keeps its warp busy
@@ -2150,43 +1689,17 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         if ((rc = m3s_buf_reserve(h, *b_ix[q], (size_t)chunk_cap * 4 * 288 * 4))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_info[q], (size_t)chunk_cap * 4 * ENC_INFO_FIELDS * 4))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_scfsi[q], (size_t)chunk_cap * 8))) return rc;
-        if (!chain) {
-            if ((rc = m3s_buf_reserve(h, *b_var[q], (size_t)chunk_cap * 4 * 16 * sizeof(uint4)))) return rc;
-            if ((rc = m3s_buf_reserve(h, *b_sum[q], (size_t)chunk_cap * 4 * sizeof(uint32_t)))) return rc;
-        }
+        if ((rc = m3s_buf_reserve(h, *b_var[q], (size_t)chunk_cap * 4 * 16 * sizeof(uint4)))) return rc;
+        if ((rc = m3s_buf_reserve(h, *b_sum[q], (size_t)chunk_cap * 4 * sizeof(uint32_t)))) return rc;
     }
 
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_rate_chain, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_rate_chain, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));   // 7 CTAs x 24 KB per SM
-    // shape of the probe kernel's CTAs (warps per CTA, CTAs per SM the register budget allows); M3S_PROBE_CFG picks another for experiments
-    typedef void (*probe_fn_t)(const M3sEncClip *, const int32_t *, const M3sDevTables *, const EncTables *, const uint32_t *, int, int, int64_t,
-                               const int32_t *, const M3sEncStats *, uint4 *, uint32_t *, uint8_t *);
-    static const struct { probe_fn_t fn; int warps; size_t smem; } kProbeCfg[] = {
-        {k_enc_probe<8, 2>, 8, sizeof(ProbeSmem<8>)}, {k_enc_probe<8, 3>, 8, sizeof(ProbeSmem<8>)}, {k_enc_probe<4, 4>, 4, sizeof(ProbeSmem<4>)}};
-    int probe_cfg = getenv("M3S_PROBE_CFG") ? atoi(getenv("M3S_PROBE_CFG")) : 0;
-    if (probe_cfg < 0 || probe_cfg >= (int)(sizeof kProbeCfg / sizeof kProbeCfg[0])) probe_cfg = 0;
-    const probe_fn_t probe_fn = kProbeCfg[probe_cfg].fn;
-    const int probe_warps = kProbeCfg[probe_cfg].warps;
-    const size_t probe_smem = kProbeCfg[probe_cfg].smem;
-    M3S_CUDA(h, cudaFuncSetAttribute(probe_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)probe_smem));
-    M3S_CUDA(h, cudaFuncSetAttribute(probe_fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ProbeSmem)));
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_probe, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_resolve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    typedef void (*ana_fn_t)(const int16_t *, const M3sEncClip *, const M3sEncWork *, const M3sDevTables *, const EncTables *, int, int64_t,
-                             int32_t *, M3sEncStats *, uint32_t);
-    static const struct { ana_fn_t fn; int warps; size_t smem; int run; } kAnaFold[] = {   // M3S_ENC_FOLD_CFG picks another shape for experiments
-#define ANA_CFG(G, W) {k_enc_analysis_fold<G, W>, W, sizeof(Ana3Smem<W>), Ana3Smem<W>::RUN}
-        ANA_CFG(0, 8), ANA_CFG(0, 4), ANA_CFG(1, 8), ANA_CFG(0, 16)};
-#undef ANA_CFG
-    int ana_cfg = getenv("M3S_ENC_FOLD_CFG") ? atoi(getenv("M3S_ENC_FOLD_CFG")) : 0;
-    if (ana_cfg < 0 || ana_cfg >= (int)(sizeof kAnaFold / sizeof kAnaFold[0])) ana_cfg = 0;
-    const ana_fn_t ana_fold = kAnaFold[ana_cfg].fn;
-    M3S_CUDA(h, cudaFuncSetAttribute(ana_fold, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kAnaFold[ana_cfg].smem));
-    M3S_CUDA(h, cudaFuncSetAttribute(ana_fold, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    // M3S_ENC_ANALYSIS_DIRECT=1 selects the direct-form analysis kernel (every product on its own) as a cross-check of the folded one
-    const bool ana_direct = getenv("M3S_ENC_ANALYSIS_DIRECT") != nullptr;
-    const int64_t ana_run = ana_direct ? ENC_RUN : kAnaFold[ana_cfg].run;
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis_fold, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Ana3Smem)));
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis_fold, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    const int64_t ana_run = Ana3Smem::RUN;   // granules per analysis work item
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PackSmem)));
     auto frames_in_chunk = [&](int i, int64_t c0) { return std::max<int64_t>(0, std::min<int64_t>(cf, clips[i].n_frames - c0)); };
     // host staging: per chunk every clip owns a region of cf * 1152 + 1056 stereo samples (1056 = the analysis history the
@@ -2290,14 +1803,9 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         M3sLaunchOn on_aux(h, h->aux);   // timing events of this launch go to the aux stream; restored on every return path
         if (g_enc_trace) tmark(tev[k].a0, h->aux);
         M3S_KBEGIN(h, M3S_K_ENC_ANALYSIS);
-        if (ana_direct)
-            k_enc_analysis<<<(unsigned)nw, ANA_THREADS, 0, h->aux>>>(
-                k_pcm, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips, (const M3sEncWork *)h->e_work.p + work_off[k], h->d_tab,
-                (const EncTables *)h->e_tabs.p, sri, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p);
-        else
-            ana_fold<<<(unsigned)nw, 32 * kAnaFold[ana_cfg].warps, kAnaFold[ana_cfg].smem, h->aux>>>(
-                k_pcm, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips, (const M3sEncWork *)h->e_work.p + work_off[k], h->d_tab,
-                (const EncTables *)h->e_tabs.p, sri, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p, 0u);
+        k_enc_analysis_fold<<<(unsigned)nw, 32 * ANA3_WARPS, sizeof(Ana3Smem), h->aux>>>(
+            k_pcm, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips, (const M3sEncWork *)h->e_work.p + work_off[k], h->d_tab,
+            (const EncTables *)h->e_tabs.p, sri, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p, 0u);
         M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].a1, h->aux);
         M3S_CUDA(h, cudaEventRecord(h->ev_ana[pb], h->aux));
@@ -2309,7 +1817,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     };
     // ---- software pipeline over the chunks (frames [k cf, (k+1) cf) of every clip); nothing in the loop blocks the host:
     //        copy_in   PCM of chunk k+2                       (host buffers only)
-    //        aux       analysis of chunk k+1                  fills the issue slots the latency-bound rate loop leaves idle
+    //        aux       analysis of chunk k+1                  queued behind the packing of chunk k
     //        stream    rate loop + packing of chunk k         the critical path: back to back, chunk after chunk
     //        copy_out  MP3 bytes of chunk k                   (host buffers only)
     if (host && n_chunks > 1) M3S_CUDA(h, stage_chunk(1));
@@ -2321,48 +1829,30 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         if (chunk_total == 0) break;
         const M3sEncClip *d_clips = (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips;
         M3S_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_ana[pb], 0));
-        // The sequential rate loop (latency chains) leaves issue slots for the next chunk's analysis, so that form overlaps the two
-        // (880 -> 741 ms/step); the parallel form and the analysis are both issue-bound and run back to back (measured: overlapping
-        // them gains nothing and stretches the analysis kernel's own time).  M3S_ENC_OVERLAP=0/1 and M3S_ENC_SERIAL override.
-        const bool overlap = getenv("M3S_ENC_SERIAL") ? false : (getenv("M3S_ENC_OVERLAP") ? atoi(getenv("M3S_ENC_OVERLAP")) != 0 : chain);
-        const bool serial = !overlap;
         const int64_t n_gran = 4 * chunk_total;
-        const int64_t probe_tiles = (n_gran + probe_warps * PROBE_G - 1) / (probe_warps * PROBE_G);
-        const int64_t probe_ctas = getenv("M3S_PROBE_CTAS") ? atoll(getenv("M3S_PROBE_CTAS")) : 0;
         M3S_KBEGIN(h, M3S_K_ENC_RATE);
-        if (chain)
-            k_enc_rate_chain<<<(unsigned)n_clips, 32 * RATE_WARPS, sizeof(RateSmem), h->stream>>>(
-                d_clips, (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p,
-                (const uint32_t *)h->e_pad.p, (const uint8_t *)h->e_payload.p, sri, whole, (int32_t)c0, (int32_t)cf, 0,
-                (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint32_t *)b_ix[pb]->p, (int32_t *)b_info[pb]->p,
-                (uint8_t *)b_scfsi[pb]->p, (uint32_t *)h->e_lastix.p);
-        else
-            probe_fn<<<(unsigned)std::min<int64_t>(probe_tiles, probe_ctas > 0 ? probe_ctas : probe_tiles), 32 * probe_warps, probe_smem, h->stream>>>(
-                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-                sri, whole, n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint4 *)b_var[pb]->p,
-                (uint32_t *)b_sum[pb]->p, (uint8_t *)b_scfsi[pb]->p);
+        k_enc_probe<<<(unsigned)((n_gran + PROBE_WARPS * PROBE_G - 1) / (PROBE_WARPS * PROBE_G)), 32 * PROBE_WARPS, sizeof(ProbeSmem), h->stream>>>(
+            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+            sri, whole, n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint4 *)b_var[pb]->p,
+            (uint32_t *)b_sum[pb]->p, (uint8_t *)b_scfsi[pb]->p);
         M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].r1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_rate[pb], h->stream));
-        // (overlapped order) queued behind the rate loop's CTAs on purpose: the next chunk's analysis takes what they leave free
-        if (!serial && k + 1 < n_chunks && (rc = launch_analysis(k + 1))) return rc;
         if (host && k + 2 < n_chunks) M3S_CUDA(h, stage_chunk(k + 2));
-        if (!chain) {
-            M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
-            k_enc_resolve<<<(unsigned)((n_clips + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
-                d_clips, n_clips, (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-                (const uint8_t *)h->e_payload.p, sri, whole, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
-                (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
-            M3S_LAUNCH_CHECK(h);
-            M3S_KBEGIN(h, M3S_K_ENC_AUX);
-            k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
-                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, sri, (int32_t)c0, (int32_t)cf,
-                n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
-                (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
-                (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
-                (uint32_t *)((char *)h->e_lastix.p + (size_t)((k + 1) & 1) * lastix_bytes));
-            M3S_LAUNCH_CHECK(h);
-        }
+        M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
+        k_enc_resolve<<<(unsigned)((n_clips + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
+            d_clips, n_clips, (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+            (const uint8_t *)h->e_payload.p, sri, whole, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
+            (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
+        M3S_LAUNCH_CHECK(h);
+        M3S_KBEGIN(h, M3S_K_ENC_AUX);
+        k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
+            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, sri, (int32_t)c0, (int32_t)cf,
+            n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
+            (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
+            (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
+            (uint32_t *)((char *)h->e_lastix.p + (size_t)((k + 1) & 1) * lastix_bytes));
+        M3S_LAUNCH_CHECK(h);
         // packing stays on the rate loop's stream
         M3S_KBEGIN(h, M3S_K_ENC_PACK);
         k_enc_pack<<<(unsigned)((chunk_total + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
@@ -2371,7 +1861,9 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].p1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_pack[pb], h->stream));
-        if (serial && k + 1 < n_chunks) {
+        // the rate loop and the analysis are both issue-bound: the next chunk's analysis waits for this chunk's packing (measured:
+        // overlapping them gains nothing and stretches the analysis kernel's own time)
+        if (k + 1 < n_chunks) {
             M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_pack[pb], 0));
             if ((rc = launch_analysis(k + 1))) return rc;
         }

@@ -1,4 +1,4 @@
-// m3s_hybrid_fast.cuh -- D2 + D3 of the decoder, FP32 instantiation (the default path; M3S_DEC_EXACT keeps k_hybrid<double>):
+// m3s_hybrid_fast.cuh -- D2 + D3 of the decoder, k_hybrid_fast in FP32 (the default path) or float64 (M3S_DEC_EXACT):
 // requantize -> MS stereo -> reorder / alias -> IMDCT + window + overlap -> frequency inversion -> polyphase synthesis -> int16.
 // (Frame.py:157-218 re_quantize, :561-572, :574-602, :604-622, :106-154 imdct, :624-631, :65-103 synth_filter_bank,
 //  :633-640 interleave, MP3_Parser.py:91 int16 conversion)

@@ -158,78 +158,48 @@ def test_chunked_equals_single(built, oracle):
     h.close()
 
 
-def test_sequential_rate_loop_equals_parallel(built, oracle, monkeypatch):
-    """M3S_ENC_CHAIN=1 selects the sequential form of the rate loop (one CTA per clip walking its granules in order); both forms
-    must produce the oracle's bytes, taps and offsets."""
-    from mp3stego_b200 import _lib
+def test_mixed_payload_batch_vs_oracle(handle, oracle):
+    """A tone hiding a long payload, quiet clicks hiding another and a short plain clip in one batch: the oracle's bytes, taps
+    and offsets."""
     clips = [synth_wav(21, 14), _clicks(5, 9 * 1152, 9), synth_wav(22, 5)]
     bits = ["011" * 200, "10" * 300, ""]
-    outs = {}
-    for mode in ("parallel", "chain"):
-        if mode == "chain":
-            monkeypatch.setenv("M3S_ENC_CHAIN", "1")
-        h = _lib.Handle(0)
-        outs[mode] = _encode(h, clips, 128, payloads=bits)
-        h.close()
-    monkeypatch.delenv("M3S_ENC_CHAIN")
-    for c, p, a, b in zip(clips, bits, outs["parallel"], outs["chain"]):
-        ref = oracle.encode(c, 44100, 128, p)
-        for g in (a, b):
-            _check_taps(g, ref)
-            assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
-
-
-@pytest.mark.parametrize("form", ["default", "direct", "cfg1", "cfg2", "cfg3"])
-def test_analysis_kernel_forms(built, oracle, monkeypatch, form):
-    """The analysis kernel ships in its folded form (equal truncated products computed once, k_enc_analysis_fold, 8 warps per CTA).
-    The direct form (M3S_ENC_ANALYSIS_DIRECT=1: every product on its own) and the other shapes of the folded one (M3S_ENC_FOLD_CFG:
-    4 / 16 warps per CTA, the xor guard) must give the oracle's MDCT lines, bytes and offsets too -- on clips long enough to span several
-    slot blocks and runs, with silence, a few-LSB stretch and clicks so that the folded form's correction pass runs
-    (MP3_Encoder.py:322-370, :652-758)."""
-    from mp3stego_b200 import _lib
-    if form == "direct":
-        monkeypatch.setenv("M3S_ENC_ANALYSIS_DIRECT", "1")
-    elif form != "default":
-        monkeypatch.setenv("M3S_ENC_FOLD_CFG", form[3:])
-    quiet = synth_wav(31, 40).copy()
-    quiet[1152 * 5:1152 * 9] = 0
-    quiet[1152 * 9:1152 * 12] = (quiet[1152 * 9:1152 * 12] >> 13).astype(np.int16)   # a few LSBs: windowed values with many zero low bits
-    clips = [synth_wav(30, 150), quiet, _clicks(11, 33 * 1152, 5), np.zeros((7 * 1152, 2), np.int16)]
-    bits = ["0110" * 900, "1" * 300, "10" * 200, ""]
-    h = _lib.Handle(0)
-    got = _encode(h, clips, 128, payloads=bits)
-    h.close()
-    for c, p, g in zip(clips, bits, got):
+    for c, p, g in zip(clips, bits, _encode(handle, clips, 128, payloads=bits)):
         ref = oracle.encode(c, 44100, 128, p)
         _check_taps(g, ref)
         assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
 
 
-@pytest.mark.parametrize("env", [{"M3S_PROBE_CTAS": "1"}, {"M3S_PROBE_CTAS": "7"}, {"M3S_PROBE_CFG": "1"}, {"M3S_PROBE_CFG": "2"},
-                                 {"M3S_ENC_OVERLAP": "1", "M3S_ENC_CHUNK_FRAMES": "64"},
-                                 {"M3S_ENC_SERIAL": "1", "M3S_ENC_CHAIN": "1", "M3S_ENC_CHUNK_FRAMES": "64"}],
-                         ids=["probe_ctas1", "probe_ctas7", "probe_cfg1", "probe_cfg2", "overlap", "serial_chain"])
-def test_encoder_switches(built, oracle, monkeypatch, env):
-    """The encoder's diagnostic switches (read per call) give the oracle's MDCT lines, bytes and offsets: a probe grid smaller than
-    the tile count (M3S_PROBE_CTAS, k_enc_probe's strided tile walk), the other probe CTA shapes (M3S_PROBE_CFG 1, 2), the analysis
-    of chunk k + 1 overlapped with the rate loop of chunk k (M3S_ENC_OVERLAP) and the serial sequential rate loop, both over
-    64-frame chunks (bytes and offsets; the taps need a single-chunk batch)."""
-    from mp3stego_b200 import _lib
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+def _analysis_edge_clips():
+    """Clips long enough to span several slot blocks and runs of the analysis kernel, with silence, a few-LSB stretch and clicks
+    so that the folded kernel's correction pass runs (MP3_Encoder.py:322-370, :652-758); and their payloads."""
     quiet = synth_wav(31, 40).copy()
     quiet[1152 * 5:1152 * 9] = 0
-    quiet[1152 * 9:1152 * 12] = (quiet[1152 * 9:1152 * 12] >> 13).astype(np.int16)
+    quiet[1152 * 9:1152 * 12] = (quiet[1152 * 9:1152 * 12] >> 13).astype(np.int16)   # a few LSBs: windowed values with many zero low bits
     clips = [synth_wav(30, 150), quiet, _clicks(11, 33 * 1152, 5), np.zeros((7 * 1152, 2), np.int16)]
-    bits = ["0110" * 900, "1" * 300, "10" * 200, ""]
-    taps = "M3S_ENC_CHUNK_FRAMES" not in env     # the taps of a batch need it in one chunk
+    return clips, ["0110" * 900, "1" * 300, "10" * 200, ""]
+
+
+def test_analysis_correction_pass(handle, oracle):
+    """The analysis kernel computes equal truncated products once and corrects the sums where an input has many zero low bits:
+    on the edge clips it gives the oracle's MDCT lines, taps, bytes and offsets."""
+    clips, bits = _analysis_edge_clips()
+    for c, p, g in zip(clips, bits, _encode(handle, clips, 128, payloads=bits)):
+        ref = oracle.encode(c, 44100, 128, p)
+        _check_taps(g, ref)
+        assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
+
+
+def test_edge_clips_in_64_frame_chunks(built, oracle, monkeypatch):
+    """The edge clips through the chunk pipeline (M3S_ENC_CHUNK_FRAMES=64: the analysis of chunk k + 1 queued behind the packing
+    of chunk k, the rate-loop state carried across chunks): the oracle's bytes and offsets (the taps need a single-chunk batch)."""
+    from mp3stego_b200 import _lib
+    monkeypatch.setenv("M3S_ENC_CHUNK_FRAMES", "64")
+    clips, bits = _analysis_edge_clips()
     h = _lib.Handle(0)
-    got = _encode(h, clips, 128, payloads=bits, taps=taps)
+    got = _encode(h, clips, 128, payloads=bits, taps=False)
     h.close()
     for c, p, g in zip(clips, bits, got):
-        ref = oracle.encode(c, 44100, 128, p, taps=taps)
-        if taps:
-            _check_taps(g, ref)
+        ref = oracle.encode(c, 44100, 128, p, taps=False)
         assert g["mp3"] == ref["mp3"] and g["hide_str_offset"] == ref["hide_str_offset"]
 
 
