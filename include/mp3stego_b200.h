@@ -172,6 +172,12 @@ M3S_API int64_t m3s_decode_bound(const uint8_t *bytes_host, const int64_t *file_
  *   mp3_out       output bytes, clip i at mp3_off[i]; capacity mp3_cap[i] >= m3s_encode_bound()
  *   out_len       [n_clips] host: bytes written (a multiple of 4, MP3_Encoder.py:1370-1392,1549-1552)
  *   hide_str_offset_out  [n_clips] host: MP3Encoder.hide_str_offset after the last frame
+ * A granule whose step search would quantise at a step above 0 (loud high-frequency input at low bitrates, e.g. a
+ * full-scale Nyquist-rate square at 44.1 kHz / 32 kbps) would make the reference read its 128-entry step table past
+ * the end (SURVEY A.E13); there is no defined output for it.  The kernels stop that search at step 0, and the call
+ * returns M3S_ERR_ARG with an m3s_last_error text naming the first such clip and frame ("clip %d frame %d: ... runs
+ * past the end of the step table").  The whole batch fails: no clip's output or hide_str_offset is valid, and the
+ * handle stays usable for the next call.
  */
 M3S_API int64_t m3s_encode_bound(int64_t n_samples, int32_t sample_rate, int32_t bitrate_kbps);
 /* Exact number of bytes MP3Encoder emits for a clip of n_samples per channel: the sum of the padded frame sizes

@@ -42,7 +42,8 @@ struct M3sEncState {       // E2 state carried from chunk to chunk (and between 
     int64_t hide_off;      // MP3Encoder.hide_str_offset
     int32_t a1[4], a2[4], a3[4], step[4];  // per (gr, ch) slot: address1..3 (stale when big_values == 0, A.E6), quantizerStepSize
     int32_t src[4];        // per slot: 1 + clip frame of the latest non-silent granule (0 = none yet); l3_enc keeps ITS values while silent
-    int32_t pad[2];
+    int32_t overrun;       // 1 + clip frame of the first granule whose step search runs past the step table (0 = none; SURVEY A.E13)
+    int32_t pad;
 };
 
 struct __align__(16) M3sEncStats {  // per granule-channel, written by E1
@@ -537,6 +538,7 @@ __device__ __forceinline__ void rate_tables_load(RateSmem &S, const M3sDevTables
 #define PROBE_CACHE 24       // distinct steps cached per granule; more than that (never seen) sends the granule to the resolve kernel
 #define VAR_SILENT 0x80000000u
 #define VAR_SLOW 0x40000000u
+#define VAR_OVERRUN (VAR_SLOW | VAR_SILENT)   // the walk needs step 1 (steptabi[128]): the resolve kernel's search finds it again and records it
 #define VAR_NONE 0xFFFFFFFFu
 
 // What a probe (one step of one granule) leaves for the variant walks: everything but the payload bits.  The table the
@@ -906,7 +908,7 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
         const uint32_t act = hiding ? (sure3 ? 0xFFu : 0x7FFFu) : 0x4000u;
         int next = -120, count = 120, step = 0, s = 0, nslots = 0, have = 0;
         uint32_t la = 0;
-        bool in_bin = true, slow = false, diverged = false;
+        bool in_bin = true, slow = false, diverged = false, overrun = false;
         for (;;) {
             int half = 0, nstep = step;
             bool ovf = false;
@@ -916,6 +918,7 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
                 ovf = s < s_min;
             } else {
                 nstep = max(step, s_min - 1) + 1;   // while quantize(step + 1) > 8192: step += 1; then step += 1
+                if (nstep > 0) { overrun = true; break; }   // the step table ends at step 0
                 s = nstep;
             }
             uint32_t lt = 0, le = 0, geo = 0, addr = 0;   // an overflowing probe counts 100000 bits: neither < nor <= max_bits
@@ -947,7 +950,7 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
         }
         // ---- ... and per lane from the first probe on which they disagree (that probe is taken again, lane by lane)
         if (diverged && !slow) {
-            bool done = !((act >> lane) & 1u);
+            bool done = !((act >> lane) & 1u), lane_over = false;
             for (;;) {
                 int half = 0;
                 bool ovf = false;
@@ -959,6 +962,7 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
                     } else {
                         step = max(step, s_min - 1) + 1;
                         s = step;
+                        if (step > 0) { lane_over = true; done = true; }   // the step table ends at step 0
                     }
                 }
                 // every step some lane needs and the cache lacks is probed once, by the whole warp
@@ -999,9 +1003,10 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
                 if (__any_sync(FULL, stray)) { slow = true; break; }
                 if (__all_sync(FULL, done)) break;
             }
+            overrun = __any_sync(FULL, lane_over);
         }
-        if (slow) {
-            if (lane == 0) sum[gs] = VAR_SLOW;
+        if (slow || overrun) {
+            if (lane == 0) sum[gs] = slow ? VAR_SLOW : VAR_OVERRUN;
             continue;
         }
         uint32_t cntw = 0;
@@ -1028,7 +1033,9 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
 
 
 // The reference's own sequential search for ONE granule with the true state (the slow path of k_enc_resolve).
-__device__ __noinline__ void search_granule(const RateSmem &S, const int32_t *__restrict__ mdct_g, int32_t xrmax, int max_bits, int hn,
+// Returns false, with step 0 and an empty granule, when the search would quantise at a step above 0 (steptabi[128], past the
+// end of the table: the reference has no defined output there, SURVEY A.E13).
+__device__ __noinline__ bool search_granule(const RateSmem &S, const int32_t *__restrict__ mdct_g, int32_t xrmax, int max_bits, int hn,
                                             uint32_t hb, int lane, int &a1, int &a2, int &a3, int &step, GranInfo &gi, int &part23)
 {
     uint32_t ax[9], ay[9], qx[9], qy[9], sg;
@@ -1043,7 +1050,13 @@ __device__ __noinline__ void search_granule(const RateSmem &S, const int32_t *__
             s = next + half;
             ovf = quant_max(S, xrmax, s) > 8192;
         } else {
-            while (quant_max(S, xrmax, step + 1) > 8192) step++;
+            while (step < 0 && quant_max(S, xrmax, step + 1) > 8192) step++;
+            if (step >= 0) {
+                gi.bv = 0; gi.count1 = 0; gi.c1sel = 0; gi.r0 = 0; gi.r1 = 0; gi.ts0 = 0; gi.ts1 = 0; gi.ts2 = 0;
+                step = 0;
+                part23 = 0;
+                return false;
+            }
             step++;
             s = step;
         }
@@ -1062,6 +1075,7 @@ __device__ __noinline__ void search_granule(const RateSmem &S, const int32_t *__
         } else if (bits <= max_bits) break;
     }
     part23 = bits;
+    return true;
 }
 
 // "latest value at or before my lane among the lanes of my slot" (lanes 4 apart), VAR_NONE where a lane has nothing to say
@@ -1102,6 +1116,7 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
     uint32_t car_a = (uint32_t)sp->a1[slot] | (uint32_t)sp->a2[slot] << 10 | (uint32_t)sp->a3[slot] << 20;
     uint32_t car_step = (uint32_t)(sp->step[slot] + 128);    // steps travel as step + 128 (8..128) so that none collides with VAR_NONE
     uint32_t car_src = (uint32_t)sp->src[slot];
+    int32_t overrun = sp->overrun;
 #pragma unroll 1
     for (int gb = 0; gb < ng; gb += 32) {
         const int i = gb + lane;
@@ -1185,7 +1200,8 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
                 const int max_bits = frame_max_bits(byteoff, fj, whole_slots, padding, mean_bits);
                 bits_at(off, hn, hb);
                 GranInfo gi;
-                search_granule(S, mdct + gsj * 576, stats[gsj].xrmax, max_bits, hn, hb, lane, a1, a2, a3, step, gi, part23);
+                if (!search_granule(S, mdct + gsj * 576, stats[gsj].xrmax, max_bits, hn, hb, lane, a1, a2, a3, step, gi, part23) && !overrun)
+                    overrun = fj + 1;
                 const int cnt = (gi.ts0 > 0) + (gi.ts1 > 0) + (gi.ts2 > 0);
                 const uint32_t na = (uint32_t)a1 | (uint32_t)a2 << 10 | (uint32_t)a3 << 20;
                 if (lane == j) {
@@ -1239,7 +1255,7 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
         sp->a1[slot] = (int32_t)(car_a & 1023u); sp->a2[slot] = (int32_t)((car_a >> 10) & 1023u); sp->a3[slot] = (int32_t)((car_a >> 20) & 1023u);
         sp->step[slot] = (int32_t)car_step - 128;
         sp->src[slot] = (int32_t)car_src;
-        if (lane == 0) sp->hide_off = off;
+        if (lane == 0) { sp->hide_off = off; sp->overrun = overrun; }
     }
 }
 
@@ -1907,6 +1923,10 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     M3S_CUDA(h, cudaStreamSynchronize(h->stream));
     if (hide_str_offset_out)
         for (int i = 0; i < n_clips; i++) hide_str_offset_out[i] = states[i].hide_off;
+    for (int i = 0; i < n_clips; i++)
+        if (states[i].overrun)
+            return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d frame %d: the step search runs past the end of the step table (quantize would "
+                            "read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)", i, states[i].overrun - 1);
     h->enc_taps_ok = single_chunk;
     h->enc_total_frames = total_frames;
     h->enc_n_clips = n_clips;

@@ -26,6 +26,8 @@ def raise_for_status(status: int, what: str = "file"):
         raise IndexError(f"{what}: big_values / region counts outside the band tables (Frame.py:461-478 raises IndexError)")
     if status & M3S_FILE_CHANNEL_SWITCH:
         raise ValueError(f"{what}: mono and stereo frames in one file (MP3_Parser.py:83: setting an array element with a sequence)")
+M3S_ERR_ARG = -2
+STEP_TABLE_OVERRUN = "runs past the end of the step table"   # in m3s_encode's error text for such a clip
 M3S_DEC_PCM_FLOAT = 1
 M3S_DEC_EXACT = 2
 
@@ -320,7 +322,8 @@ class Handle:
                compact=False, payload_packed=None):
         """E1-E3 over a batch of int16 stereo clips laid end to end in `pcm` (numpy or torch, host or cuda).
         compact=True lays the MP3s back to back at their exact sizes (m3s_encode_size), so that (mp3, mp3_off + [end])
-        can be fed straight to decode_scan.  payload_packed = (uint8 array of '0'/'1' chars, offsets[n+1]) avoids re-joining."""
+        can be fed straight to decode_scan.  payload_packed = (uint8 array of '0'/'1' chars, offsets[n+1]) avoids re-joining.
+        Raises IndexError, for the whole batch, when a clip drives the rate loop past the end of the step table."""
         L = self._L
         n = len(n_samples)
         ns, ns_p = _i64(n_samples)
@@ -356,6 +359,11 @@ class Handle:
         _ready(pcm, mp3_out)
         rc = L.m3s_encode(self._h, _ptr(pcm), mem, po_p, ns_p, n, sample_rate, bitrate_kbps, pl_p, ploff_p, _ptr(mp3_out),
                           mo_p, mc_p, out_len.ctypes.data_as(_c_i64p), hoff.ctypes.data_as(_c_i64p))
+        if rc == M3S_ERR_ARG:
+            msg = L.m3s_last_error(self._h).decode()
+            if STEP_TABLE_OVERRUN in msg:
+                # the reference's quantize() indexes its step table past the end for this input (SURVEY A.E13): no output
+                raise IndexError(f"index out of bounds: {msg}")
         self._check(rc, "m3s_encode")
         res = dict(mp3=mp3_out, mp3_off=mo, out_len=out_len, hide_str_offset=hoff)
         if taps:

@@ -7,7 +7,7 @@
                  (encoder.py:22-51, WAV_Reader.py:30-110), same structure around one m3s_encode call per sample rate
 
 torch is used for pinned host memory only.  Per-file failures follow the reference: sys.exit messages for missing files / bad
-WAV headers, IndexError for input the reference's encoder cannot read (mono, length not a multiple of 1152)."""
+WAV headers, IndexError for input the reference's encoder cannot read (mono, length not a multiple of 1152, a clip that drives the rate loop past the step table)."""
 import os
 import struct
 import sys

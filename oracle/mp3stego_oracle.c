@@ -709,7 +709,7 @@ typedef struct ora_enc_result {
     int32_t *ix;   /* [n_frames][ch][gr][576] signed, as written */
     int32_t *info; /* [n_frames][gr][ch][ORA_ENC_FIELDS] */
     int32_t *scfsi; /* [n_frames][ch][4] */
-    int status;
+    int status;     /* 0; -1 mono; -2 bad rate; -3 step table overrun (A.E13): no bytes, n_frames = that frame */
 } ora_enc_result;
 #define ORA_ENC_FIELDS 16
 
@@ -989,12 +989,15 @@ static int bin_search_step_size(enc_t *e, int desired, int32_t *ix, grinfo_t *ci
 }
 
 /* MP3_Encoder.py:1064-1095 */
+/* Returns -1 instead of a bit count when the search would quantise at a step above 0: quantize() would read steptabi[128],
+ * past the end of the 128-entry table, and the reference has no defined output there (SURVEY A.E13). */
 static int inner_loop(enc_t *e, int32_t *ix, int max_bits, grinfo_t *ci)
 {
     int bits;
     if (max_bits < 0) ci->quantizerStepSize -= 1;
     do {
-        while (quantize(e, ix, ci->quantizerStepSize + 1) > 8192) ci->quantizerStepSize += 1;
+        while (ci->quantizerStepSize < 0 && quantize(e, ix, ci->quantizerStepSize + 1) > 8192) ci->quantizerStepSize += 1;
+        if (ci->quantizerStepSize >= 0) return -1;
         ci->quantizerStepSize += 1;
         bits = probe_bits(e, ix, ci);
     } while (bits > max_bits);
@@ -1068,7 +1071,8 @@ static void resv_frame_end(enc_t *e)
 }
 
 /* MP3_Encoder.py:760-815 */
-static void iteration_loop(enc_t *e)
+/* Returns 0, or -1 when a granule's step search runs past the step table (inner_loop). */
+static int iteration_loop(enc_t *e)
 {
     for (int ch = 0; ch < e->nch; ch++)
         for (int gr = 0; gr < 2; gr++) {
@@ -1094,6 +1098,7 @@ static void iteration_loop(enc_t *e)
                 ci->quantizerStepSize = bin_search_step_size(e, max_bits, ix, ci);
                 ci->part2_length = 0;
                 int bits = inner_loop(e, ix, max_bits - ci->part2_length, ci);
+                if (bits < 0) return -1;
                 ci->part2_3_length = ci->part2_length + bits;
                 e->hide_off += (ci->table_select[0] > 0) + (ci->table_select[1] > 0) + (ci->table_select[2] > 0);
             }
@@ -1101,6 +1106,7 @@ static void iteration_loop(enc_t *e)
             ci->global_gain = ci->quantizerStepSize + 210;
         }
     resv_frame_end(e);
+    return 0;
 }
 
 /* MP3_Encoder.py:1448-1513 */
@@ -1265,7 +1271,12 @@ ORA_API ora_enc_result *ora_encode(const int16_t *pcm, int64_t pcm_len, int64_t 
         e->bits_per_frame = 8 * (e->whole_slots_per_frame + e->padding);
         e->mean_bits = (int)((e->bits_per_frame - e->side_info_len) / 2.0);
         mdct_sub(e);
-        iteration_loop(e);
+        if (iteration_loop(e)) { /* step table overrun: no bytes, n_frames = the frame it happened in */
+            r->status = -3;
+            r->n_frames = f;
+            free(e->out.p); free(e);
+            return r;
+        }
         format_bitstream(e);
         if (want_taps) {
             memcpy(r->mdct + f * 4 * 576, e->mdct_freq, sizeof e->mdct_freq);

@@ -113,7 +113,8 @@ def decode(data: bytes, offset: int = 0, taps: bool = True) -> dict:
 
 def encode(pcm: np.ndarray, samplerate: int = 44100, bitrate: int = 320, hide_bits: str = "",
            taps: bool = True) -> dict:
-    """Encode interleaved int16 stereo PCM [n, 2] the way MP3Encoder.encode does (MP3_Encoder.py:596-621)."""
+    """Encode interleaved int16 stereo PCM [n, 2] the way MP3Encoder.encode does (MP3_Encoder.py:596-621).
+    status -3: a granule's step search ran past the step table (SURVEY A.E13); no bytes, n_frames = the frame it happened in."""
     L = lib()
     pcm = np.ascontiguousarray(pcm, dtype=np.int16)
     nch = pcm.shape[1] if pcm.ndim == 2 else 1

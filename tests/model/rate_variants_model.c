@@ -7,12 +7,15 @@
  * ("probe"), and a sequential pass that only looks results up ("resolve", redoing the flagged granules with the true state)
  * reproduces the reference's side info, step sizes, addresses and hide_str_offset exactly.
  *
- * usage: rate_variants_model pcm.raw n_frames bitrate_kbps payload.txt [payload_len]   ->  "granules N silent S slow R bad B"
- * (bad = granules where the model and the oracle disagree; must be 0) */
+ * usage: rate_variants_model pcm.raw n_frames bitrate_kbps payload.txt [payload_len|-1 [sample_rate]]
+ *   ->  "granules N silent S slow R bad B maxsteps M"
+ * (bad = granules where the model and the oracle disagree; must be 0.  maxsteps = the most distinct steps the active variants of
+ * one granule probe together, which k_enc_probe caches in PROBE_CACHE = 24 rows before it sends the granule to the slow path.)
+ * Clips whose step search runs past the step table (SURVEY A.E13) are outside the model: it stops with "overrun". */
 #include "../../oracle/mp3stego_oracle.c"
 #include <stdio.h>
-static int g_slow, g_have; static int g_la[3];
-static int my_probe(enc_t*e,int32_t*ix,grinfo_t*ci){ int b=probe_bits(e,ix,ci); if(ci->big_values==0&&ci->count1>0&&!g_have) g_slow=1; if(ci->big_values>0){g_have=1;g_la[0]=ci->address1;g_la[1]=ci->address2;g_la[2]=ci->address3;} return b;}
+static int g_slow, g_have; static int g_la[3]; static unsigned char g_seen[128]; static int g_nseen;
+static int my_probe(enc_t*e,int32_t*ix,grinfo_t*ci,int step){ if(!g_seen[step+127]){g_seen[step+127]=1;g_nseen++;} int b=probe_bits(e,ix,ci); if(ci->big_values==0&&ci->count1>0&&!g_have) g_slow=1; if(ci->big_values>0){g_have=1;g_la[0]=ci->address1;g_la[1]=ci->address2;g_la[2]=ci->address3;} return b;}
 static void run_variant(enc_t *e, grinfo_t ci0, int max_bits, const char *bits, int hn, grinfo_t *out, int *outbits)
 {
     static int32_t ix[576];
@@ -22,13 +25,14 @@ static void run_variant(enc_t *e, grinfo_t ci0, int max_bits, const char *bits, 
     g_slow=0; g_have=0;
     int next=-120,count=120;
     do{int half=count/2,bit; int s=next+half;
-       if(quantize(e,ix,s)>8192) bit=100000; else bit=my_probe(e,ix,&ci);
+       if(quantize(e,ix,s)>8192) bit=100000; else bit=my_probe(e,ix,&ci,s);
        if(bit<max_bits) count=half; else {next+=half;count-=half;}
     }while(count>1);
     ci.quantizerStepSize=next;
     int b;
-    do{ while(quantize(e,ix,ci.quantizerStepSize+1)>8192) ci.quantizerStepSize++;
-        ci.quantizerStepSize++; b=my_probe(e,ix,&ci);
+    do{ while(ci.quantizerStepSize<0&&quantize(e,ix,ci.quantizerStepSize+1)>8192) ci.quantizerStepSize++;
+        if(ci.quantizerStepSize>=0){printf("overrun\n");exit(0);}
+        ci.quantizerStepSize++; b=my_probe(e,ix,&ci,ci.quantizerStepSize);
     }while(b>max_bits);
     e->hide_str=sv_s; e->hide_len=sv_l; e->hide_off=sv_o;
     *out=ci; *outbits=b;
@@ -37,18 +41,19 @@ int main(int argc,char**argv){
     int nfr=atoi(argv[2]); int br=atoi(argv[3]);
     FILE*f=fopen(argv[1],"rb"); int16_t*pcm=malloc((size_t)nfr*1152*2*2); if(fread(pcm,2,(size_t)nfr*1152*2,f)){} fclose(f);
     f=fopen(argv[4],"rb"); char*pay=malloc(1<<20); int64_t plen=fread(pay,1,1<<20,f); fclose(f);
-    if(argc>5) plen=atoi(argv[5]);
+    if(argc>5&&atoi(argv[5])>=0) plen=atoi(argv[5]);
+    int sr=argc>6?atoi(argv[6]):44100;
     enc_t*e=calloc(1,sizeof*e);
-    e->nch=2;e->samplerate=44100;e->bitrate=br;e->sr_index=0;
+    e->nch=2;e->samplerate=sr;e->bitrate=br;e->sr_index=sr==44100?0:sr==48000?1:2;
     e->buffer=pcm;e->buffer_len=(int64_t)nfr*1152*2;e->buffer_pos[0]=0;e->buffer_pos[1]=1;
     e->hide_str=pay;e->hide_len=plen;e->cache=0;e->cache_bits=32;
     for(int i=0;i<10000;i++) e->int2idx[i]=(int32_t)(sqrt(sqrt((double)i)*(double)i)-0.0946+0.5);
-    double avg=(2.0*576/44100.0)*(1000*(double)br/8.0);
+    double avg=(2.0*576/(double)sr)*(1000*(double)br/8.0);
     e->whole_slots_per_frame=(int)avg;e->frac_slots_per_frame=avg-(double)e->whole_slots_per_frame;e->slot_lag=-e->frac_slots_per_frame;
     e->side_info_len=288;
     /* emulated state */
     int st_a[2][2][3]={{{0}}}, st_step[2][2]={{0}}; int64_t off=0;
-    long ngr=0,nslow=0,nsil=0,bad=0;
+    long ngr=0,nslow=0,nsil=0,bad=0; int maxsteps=0;
     for(int fr=0;fr<nfr;fr++){
         if(e->frac_slots_per_frame!=0){e->padding=e->slot_lag<=(e->frac_slots_per_frame-1.0)?1:0;e->slot_lag+=e->padding-e->frac_slots_per_frame;}
         e->bits_per_frame=8*(e->whole_slots_per_frame+e->padding);
@@ -66,6 +71,7 @@ int main(int argc,char**argv){
             if(e->xrmax){
                 int q=2*ch+gr; int hiding=plen>0; int sure3=plen-3*(4*(int64_t)fr+q)>=3;
                 grinfo_t rec[15]; int rbits[15]; int rhave[15]; int rla[15][3]; int slow=0;
+                memset(g_seen,0,sizeof g_seen); g_nseen=0;
                 for(int v=0;v<15;v++){
                     int active=hiding?(v<(sure3?8:15)):(v==14); if(!active) continue;
                     int hn; int hb; if(v<8){hn=3;hb=v;}else if(v<12){hn=2;hb=v-8;}else if(v<14){hn=1;hb=v-12;}else{hn=0;hb=0;}
@@ -73,6 +79,7 @@ int main(int argc,char**argv){
                     grinfo_t z=*ci; z.address1=z.address2=z.address3=0;
                     run_variant(e,z,max_bits,b,hn,&rec[v],&rbits[v]); if(g_slow) slow=1; rhave[v]=g_have; memcpy(rla[v],g_la,sizeof g_la);
                 }
+                if(g_nseen>maxsteps) maxsteps=g_nseen;
                 /* resolve */
                 int hn=0; int hb=0; if(hiding){int64_t left=plen-off; hn=left>3?3:(left<0?0:(int)left); for(int k=0;k<hn;k++) if(pay[off+k]=='1') hb|=1<<k;}
                 int v=hn==3?hb:hn==2?8+hb:hn==1?12+hb:14;
@@ -96,6 +103,6 @@ int main(int argc,char**argv){
             if(!ok){bad++; if(bad<5) printf("BAD fr %d ch %d gr %d: ts %d %d %d vs %d %d %d p23 %d vs %d a %d %d %d vs %d %d %d off %ld vs %ld\n",fr,ch,gr,em_ts[0],em_ts[1],em_ts[2],ci->table_select[0],ci->table_select[1],ci->table_select[2],em_p23,ci->part2_3_length,st_a[gr][ch][0],st_a[gr][ch][1],st_a[gr][ch][2],ci->address1,ci->address2,ci->address3,(long)off,(long)e->hide_off);}
         }
     }
-    printf("granules %ld silent %ld slow %ld bad %ld\n",ngr,nsil,nslow,bad);
+    printf("granules %ld silent %ld slow %ld bad %ld maxsteps %d\n",ngr,nsil,nslow,bad,maxsteps);
     return 0;
 }
