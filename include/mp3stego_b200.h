@@ -187,7 +187,20 @@ M3S_API int m3s_encode(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
                        int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
                        const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
                        int64_t *out_len, int64_t *hide_str_offset_out);
-/* Parity taps of the last m3s_encode call (host buffers): mdct int32 [frames][ch][gr][576] (MP3_Encoder.py:652),
+/* m3s_encode with a rate pair per clip: clips of different sample rates and bitrates in ONE call (a mixed MP3 collection
+ * re-encoded at each file's own rates needs no grouping by the caller).
+ *   sample_rate   [n_clips] host: 32000, 44100 or 48000 per clip
+ *   bitrate_kbps  [n_clips] host: one of the 14 MPEG-1 Layer III bitrates per clip
+ * Everything else as m3s_encode, per clip: clip i's bytes, out_len and hide_str_offset are what m3s_encode gives for it at its own
+ * pair.  A clip with an unsupported rate fails the call with M3S_ERR_ARG before anything is queued, the text naming the clip
+ * ("clip %d: sample rate ..." / "clip %d: bitrate ...").  The step-table failure above names the caller's clip index and frame.
+ * m3s_encode_taps works after a single-chunk call, frames in the caller's clip order.  m3s_encode is this function with its two
+ * rates broadcast to every clip. */
+M3S_API int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                             int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
+                             const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
+                             int64_t *out_len, int64_t *hide_str_offset_out);
+/* Parity taps of the last m3s_encode / m3s_encode_mixed call (host buffers): mdct int32 [frames][ch][gr][576] (MP3_Encoder.py:652),
  * ix int32 [frames][ch][gr][576] signed as written (:1272-1276), info int32 [frames][gr][ch][16]:
  * part2_3_length, big_values, count1, global_gain, table_select[3], region0_count, region1_count,
  * count1table_select, address1..3, quantizerStepSize, padding, hide_str_offset-after-frame. */

@@ -236,7 +236,7 @@ struct m3s_ctx {
     int64_t enc_chunk_budget = 0;   // frames of intermediates kept per chunk (0 = default; M3S_ENC_CHUNK_FRAMES overrides)
     int64_t enc_total_frames = 0;
     int32_t enc_n_clips = 0;
-    std::vector<int64_t> enc_frame_base;
+    std::vector<int64_t> enc_tap_runs;   // last encode: (device frame, caller frame, frames) triples, the taps' way back to the caller's clip order
 };
 
 int m3s_fail(m3s_ctx *h, int code, const char *fmt, ...);

@@ -233,7 +233,7 @@ static void build_tables(M3sDevTables *T)
 
 static_assert(sizeof(M3S_HUFF_PACKED) / sizeof(uint32_t) == 1410, "packed code book size");
 
-extern "C" int m3s_version(void) { return 200; }
+extern "C" int m3s_version(void) { return 300; }
 
 extern "C" int m3s_create(int device, m3s_handle_t *out)
 {

@@ -35,7 +35,10 @@ struct M3sEncClip {
     int64_t payload_base;  // first payload char
     int64_t payload_len;   // number of payload chars ('0'/'1'); 0 = plain encode
     int32_t n_frames;
-    int32_t pad;
+    int32_t pad_base;      // first entry of the clip's frame byte offsets in the padding tables of the call (one table per rate pair)
+    int32_t whole_slots;   // whole bytes of a frame at the clip's rate pair (a padded frame has one more)
+    int16_t sr_idx;        // 0 = 44.1, 1 = 48, 2 = 32 kHz (the header's sampling_frequency field)
+    int16_t bitrate_idx;   // the header's bitrate_index, 1..14
 };
 
 struct M3sEncState {       // E2 state carried from chunk to chunk (and between frames inside the kernel)
@@ -142,7 +145,7 @@ struct Ana3LoadSb {  // input j of the MDCT: slot j of the previous granule (j <
 // each product once instead of recomputing it per use, and the add folds into the multiply's addend
 __global__ void __launch_bounds__(32 * ANA3_WARPS, 2)
 k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restrict__ clips, const M3sEncWork *__restrict__ work,
-                    const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET, int sr_idx, int64_t chunk_frame0,
+                    const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET, int64_t chunk_frame0,
                     int32_t *__restrict__ mdct, M3sEncStats *__restrict__ stats, const uint32_t zero)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -153,7 +156,7 @@ k_enc_analysis_fold(const int16_t *__restrict__ pcm, const M3sEncClip *__restric
     const M3sEncWork wk = work[blockIdx.x];
     const M3sEncClip cl = clips[wk.clip];
     const int ch = wk.ch;
-    for (int i = tid; i < 576; i += ANA3_THREADS) S.sfb[i] = T->long_sfb_of[sr_idx][i];
+    for (int i = tid; i < 576; i += ANA3_THREADS) S.sfb[i] = T->long_sfb_of[cl.sr_idx][i];
     if (tid < 8) { S.ca[tid] = T->enc_ca[tid]; S.cs[tid] = T->enc_cs[tid]; }
     if (tid < 32) S.en_thresh[tid] = ET->en_thresh[tid];
     if (tid < 24 * ANA3_WARPS) (&S.bins[0][0])[tid] = 0u;
@@ -497,9 +500,10 @@ __device__ __forceinline__ void quantize_all(const RateSmem &S, const uint32_t (
     }
 }
 
-// the shared-memory tables of k_enc_resolve and k_enc_emit
+// the shared-memory tables of k_enc_resolve and k_enc_emit; the band bounds S.sfb depend on the sample rate and only the
+// resolve kernel reads them (it loads them itself, once per sample-rate group)
 __device__ __forceinline__ void rate_tables_load(RateSmem &S, const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET,
-                                                 int sr_idx, int tid, int nthr)
+                                                 int tid, int nthr)
 {
     for (int i = tid; i < 10000; i += nthr) S.i2i[i] = (uint16_t)T->int2idx[i];
     for (int i = tid; i < 256; i += nthr) {
@@ -507,7 +511,6 @@ __device__ __forceinline__ void rate_tables_load(RateSmem &S, const M3sDevTables
         S.hlc[i] = make_uint2(ET->hl4[i], (uint32_t)(x != 0) + (uint32_t)(y != 0) + (((uint32_t)(x > 14) + (uint32_t)(y > 14)) << 16));
     }
     for (int i = tid; i < 128; i += nthr) { S.steptabi[i] = T->steptabi[i]; S.steptab[i] = T->steptab[i]; }
-    if (tid < 24) S.sfb[tid] = tid < 23 ? T->sfb_long[sr_idx][tid] : 576;
     if (tid < 32) {
         S.linmax[tid] = T->enc_linmax[tid];
         S.linbits[tid] = T->enc_linbits[tid];
@@ -584,10 +587,12 @@ __device__ __forceinline__ void load_granule(const int32_t *__restrict__ mdct_g,
     }
 }
 
-__device__ __forceinline__ int frame_max_bits(const uint32_t *__restrict__ byteoff, int f, int whole_slots, int &padding, int &mean_bits)
+// max_bits of frame f of clip `cl` (its own rate pair); `byteoff` = the padding tables of the call
+__device__ __forceinline__ int frame_max_bits(const uint32_t *__restrict__ byteoff, const M3sEncClip &cl, int f, int &padding, int &mean_bits)
 {
-    padding = (int)(byteoff[f + 1] - byteoff[f]) - whole_slots;
-    const int bits_per_frame = 8 * (whole_slots + padding);
+    const uint32_t *bo = byteoff + cl.pad_base;
+    padding = (int)(bo[f + 1] - bo[f]) - cl.whole_slots;
+    const int bits_per_frame = 8 * (cl.whole_slots + padding);
     mean_bits = (bits_per_frame - 288) / 2;                  // :634-636 (side info 8 * (4 + 32) bits)
     return min(mean_bits / 2, 4095);                         // :894-912 with the reservoir never enabled (A.E7)
 }
@@ -804,10 +809,10 @@ __device__ __forceinline__ bool probe_row(const ProbeTab &T, const uint32_t (&ax
 
 __global__ void __launch_bounds__(32 * PROBE_WARPS, 2)
 k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ frame_clip, const M3sDevTables *__restrict__ DT,
-            const EncTables *__restrict__ ET, const uint32_t *__restrict__ byteoff, int sr_idx, int whole_slots, int64_t n_gran,
+            const EncTables *__restrict__ ET, const uint32_t *__restrict__ byteoff, int sr_idx, int64_t g_begin, int64_t g_end,
             const int32_t *__restrict__ mdct, const M3sEncStats *__restrict__ stats, uint4 *__restrict__ var,
             uint32_t *__restrict__ sum, uint8_t *__restrict__ scfsi_out)
-{
+{   // granule slots [g_begin, g_end) of the chunk: the frames of the clips at sample rate sr_idx (their tables are per CTA)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ProbeSmem &PS = *reinterpret_cast<ProbeSmem *>(smem_raw);
     ProbeTab &T = PS.T;
@@ -855,15 +860,15 @@ k_enc_probe(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fr
     // one tile of PROBE_WARPS * PROBE_G granules per CTA: warp w takes granules w, w + PROBE_WARPS, ... of tile blockIdx.x
 #pragma unroll 1
     for (int it = 0; it < PROBE_G; it++) {
-        const int64_t gs = (int64_t)blockIdx.x * (PROBE_WARPS * PROBE_G) + warp + it * PROBE_WARPS;
-        if (gs >= n_gran) break;
+        const int64_t gs = g_begin + (int64_t)blockIdx.x * (PROBE_WARPS * PROBE_G) + warp + it * PROBE_WARPS;
+        if (gs >= g_end) break;
         const int64_t fl_ = gs >> 2;
         const int q = (int)(gs & 3);                         // position in the reference's order: (ch0,gr0) (ch0,gr1) (ch1,gr0) (ch1,gr1)
         const int c = frame_clip[fl_];
         const int64_t payload_len = clips[c].payload_len;
         const int f = (int)(fl_ - clips[c].frame_base);      // frame index inside the clip
         int padding, mean_bits;
-        const int max_bits = frame_max_bits(byteoff, f, whole_slots, padding, mean_bits);
+        const int max_bits = frame_max_bits(byteoff, clips[c], f, padding, mean_bits);
         const int32_t xrmax = stats[gs].xrmax;
         if (q & 1) {
             // ---- calc_scfsi (:862-892) of this channel: needs the statistics of both granules
@@ -1091,19 +1096,20 @@ __device__ __forceinline__ uint32_t slot_scan(uint32_t v, int lane)
 
 #define RESOLVE_WARPS 2
 __global__ void __launch_bounds__(32 * RESOLVE_WARPS)
-k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__restrict__ states, const M3sDevTables *__restrict__ T,
+k_enc_resolve(const M3sEncClip *__restrict__ clips, int c_begin, int c_end, M3sEncState *__restrict__ states, const M3sDevTables *__restrict__ T,
               const EncTables *__restrict__ ET, const uint32_t *__restrict__ byteoff, const uint8_t *__restrict__ payload, int sr_idx,
-              int whole_slots, int32_t chunk_first, int32_t chunk_frames, const int32_t *__restrict__ mdct,
+              int32_t chunk_first, int32_t chunk_frames, const int32_t *__restrict__ mdct,
               const M3sEncStats *__restrict__ stats, const uint4 *__restrict__ var, uint32_t *__restrict__ sum, int32_t *__restrict__ info)
-{
+{   // clips [c_begin, c_end): the clips at sample rate sr_idx
     extern __shared__ __align__(16) unsigned char smem_raw[];
     RateSmem &S = *reinterpret_cast<RateSmem *>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t FULL = 0xFFFFFFFFu;
-    rate_tables_load(S, T, ET, sr_idx, tid, 32 * RESOLVE_WARPS);
+    rate_tables_load(S, T, ET, tid, 32 * RESOLVE_WARPS);
+    if (tid < 24) S.sfb[tid] = tid < 23 ? T->sfb_long[sr_idx][tid] : 576;
     __syncthreads();
-    const int c = blockIdx.x * RESOLVE_WARPS + warp;
-    if (c >= n_clips) return;
+    const int c = c_begin + blockIdx.x * RESOLVE_WARPS + warp;
+    if (c >= c_end) return;
     const M3sEncClip cl = clips[c];
     const int f_end = min(cl.n_frames, chunk_first + chunk_frames);
     if (f_end <= chunk_first) return;
@@ -1197,7 +1203,7 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
                 const int64_t gsj = (cl.frame_base + fj) * 4 + jq;
                 int padding, mean_bits, hn, part23 = 0;
                 uint32_t hb;
-                const int max_bits = frame_max_bits(byteoff, fj, whole_slots, padding, mean_bits);
+                const int max_bits = frame_max_bits(byteoff, cl, fj, padding, mean_bits);
                 bits_at(off, hn, hb);
                 GranInfo gi;
                 if (!search_granule(S, mdct + gsj * 576, stats[gsj].xrmax, max_bits, hn, hb, lane, a1, a2, a3, step, gi, part23) && !overrun)
@@ -1217,7 +1223,7 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
         // ---- per frame (4 lanes): resv_frame_end (:1097-1145) -- every unused bit of the frame becomes stuffing -- and the records
         {
             int padding = 0, mean_bits = 0;
-            if (valid) frame_max_bits(byteoff, f, whole_slots, padding, mean_bits);
+            if (valid) frame_max_bits(byteoff, cl, f, padding, mean_bits);
             const int base = lane & ~3;
             // part2_3_length in the order gr0ch0, gr0ch1, gr1ch0, gr1ch1 = my positions 0, 2, 1, 3
             int p23[4];
@@ -1266,7 +1272,7 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int n_clips, M3sEncState *__
 #define EMIT_G 8
 __global__ void __launch_bounds__(32 * EMIT_WARPS, 3)
 k_enc_emit(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ frame_clip, const M3sDevTables *__restrict__ T,
-           const EncTables *__restrict__ ET, int sr_idx, int32_t chunk_first, int32_t chunk_frames, int64_t n_gran,
+           const EncTables *__restrict__ ET, int32_t chunk_first, int32_t chunk_frames, int64_t n_gran,
            const int32_t *__restrict__ mdct, const M3sEncStats *__restrict__ stats, const uint32_t *__restrict__ srcs,
            const int32_t *__restrict__ info, uint32_t *__restrict__ ixout, const uint32_t *__restrict__ last_in,
            uint32_t *__restrict__ last_out)
@@ -1274,7 +1280,7 @@ k_enc_emit(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fra
     extern __shared__ __align__(16) unsigned char smem_raw[];
     RateSmem &S = *reinterpret_cast<RateSmem *>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    rate_tables_load(S, T, ET, sr_idx, tid, 32 * EMIT_WARPS);
+    rate_tables_load(S, T, ET, tid, 32 * EMIT_WARPS);
     __syncthreads();
     const int64_t g0 = (int64_t)blockIdx.x * (EMIT_WARPS * EMIT_G) + warp;
 #pragma unroll 1
@@ -1330,7 +1336,7 @@ struct PackSmem {
     uint32_t code[1410];
     uint16_t hoff[34];
     uint8_t linbits[34];
-    uint16_t sfb[24];
+    uint16_t sfb[3][24];     // per sample rate: the two warps of a CTA may pack frames of clips at different rates
     uint32_t frame[PACK_WARPS][PACK_WORDS];
     uint32_t ix[PACK_WARPS][288];
 };
@@ -1347,9 +1353,8 @@ __device__ __forceinline__ void put_bits_at(uint32_t *buf, int pos, uint32_t v, 
 
 __global__ void __launch_bounds__(32 * PACK_WARPS)
 k_enc_pack(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ frame_clip, const M3sDevTables *__restrict__ T,
-           const uint32_t *__restrict__ byteoff, int sr_idx, int bitrate_idx, int whole_slots, int64_t chunk_frame0,
-           int64_t chunk_total_frames, const uint32_t *__restrict__ ixin, const int32_t *__restrict__ info,
-           const uint8_t *__restrict__ scfsi, uint8_t *__restrict__ out)
+           const uint32_t *__restrict__ byteoff, int64_t chunk_frame0, int64_t chunk_total_frames, const uint32_t *__restrict__ ixin,
+           const int32_t *__restrict__ info, const uint8_t *__restrict__ scfsi, uint8_t *__restrict__ out)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     PackSmem &S = *reinterpret_cast<PackSmem *>(smem_raw);
@@ -1357,15 +1362,17 @@ k_enc_pack(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fra
     const uint32_t FULL = 0xFFFFFFFFu;
     for (int i = tid; i < 1410; i += 32 * PACK_WARPS) S.code[i] = T->enc_hpacked[i];
     if (tid < 34) { S.hoff[tid] = T->enc_hoff[tid]; S.linbits[tid] = T->enc_linbits[tid]; }
-    if (tid < 24) S.sfb[tid] = tid < 23 ? T->sfb_long[sr_idx][tid] : 576;
+    for (int i = tid; i < 3 * 24; i += 32 * PACK_WARPS) S.sfb[i / 24][i % 24] = i % 24 < 23 ? T->sfb_long[i / 24][i % 24] : 576;
     __syncthreads();
     const int64_t fl_ = (int64_t)blockIdx.x * PACK_WARPS + warp;
     if (fl_ >= chunk_total_frames) return;
     const int c = frame_clip[fl_];
     const M3sEncClip cl = clips[c];
     const int f = (int)(chunk_frame0 + fl_ - cl.frame_base);
-    const int fbytes = (int)(byteoff[f + 1] - byteoff[f]);
-    const int padding = fbytes - whole_slots;
+    const uint32_t *bo = byteoff + cl.pad_base;
+    const uint16_t *sfb = S.sfb[cl.sr_idx];
+    const int fbytes = (int)(bo[f + 1] - bo[f]);
+    const int padding = fbytes - cl.whole_slots;
     uint32_t *buf = S.frame[warp];
     for (int i = lane; i < PACK_WORDS; i += 32) buf[i] = 0u;
     __syncwarp();
@@ -1374,7 +1381,7 @@ k_enc_pack(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fra
     if (lane == 0) {
         int pos = 0;
         auto put = [&](uint32_t v, int n) { put_bits_at(buf, pos, v, n); pos += n; };
-        put(0x7ff, 11); put(3, 2); put(1, 2); put(1, 1); put((uint32_t)bitrate_idx, 4); put((uint32_t)(sr_idx % 3), 2);
+        put(0x7ff, 11); put(3, 2); put(1, 2); put(1, 1); put((uint32_t)cl.bitrate_idx, 4); put((uint32_t)cl.sr_idx, 2);
         put((uint32_t)padding, 1); put(0, 1); put(0, 2); put(0, 2); put(0, 1); put(1, 1); put(0, 2);
         put(0, 9); put(0, 3);
         for (int ch = 0; ch < 2; ch++)
@@ -1393,7 +1400,7 @@ k_enc_pack(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fra
         for (int ch = 0; ch < 2; ch++) {
             const int32_t *r = inf + (2 * gr + ch) * ENC_INFO_FIELDS;
             const int part23 = r[0], bv = r[1], count1 = r[2], ts[3] = {r[4], r[5], r[6]}, c1sel = r[9];
-            const int r1 = S.sfb[r[7] + 1], r2 = S.sfb[min(r[7] + 1 + r[8] + 1, 23)];
+            const int r1 = sfb[r[7] + 1], r2 = sfb[min(r[7] + 1 + r[8] + 1, 23)];
             const uint32_t *src = ixin + ((fl_ * 2 + ch) * 2 + gr) * 288;
             uint32_t *ix = S.ix[warp];
             for (int j = 0; j < 9; j++) ix[32 * j + lane] = __ldg(src + 32 * j + lane);
@@ -1486,7 +1493,7 @@ k_enc_pack(const M3sEncClip *__restrict__ clips, const int32_t *__restrict__ fra
         }
     __syncwarp();
     // ---- copy out, clipped to what the reference's word-granular writer emits for the whole clip (A.E8)
-    const int64_t fo = byteoff[f];
+    const int64_t fo = bo[f];
     const uint8_t *bb = (const uint8_t *)buf;
     for (int i = lane; i < fbytes; i += 32)
         if (fo + i < cl.out_len) out[cl.out_base + fo + i] = bb[i ^ 3];   // big-endian words -> byte stream
@@ -1580,22 +1587,47 @@ static void build_enc_tables(const M3sDevTables *T, EncTables *E)
 }
 
 static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                       int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
+                       int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
                        const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
                        int64_t *out_len, int64_t *hide_str_offset_out);
+
+// both entry points run here: an early return may leave work of the call on the helper streams, drained before the caller reuses buffers
+static int encode_call(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples, int32_t n_clips,
+                       const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits, const int64_t *payload_off,
+                       uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap, int64_t *out_len, int64_t *hide_str_offset_out)
+{
+    const int rc = encode_impl(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out,
+                               mp3_off, mp3_cap, out_len, hide_str_offset_out);
+    if (rc != M3S_OK && h) {
+        cudaStreamSynchronize(h->stream);
+        if (h->copy_in) { cudaStreamSynchronize(h->copy_in); cudaStreamSynchronize(h->copy_out); cudaStreamSynchronize(h->aux); }
+    }
+    return rc;
+}
 
 extern "C" int m3s_encode(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
                           int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
                           const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
                           int64_t *out_len, int64_t *hide_str_offset_out)
 {
-    const int rc = encode_impl(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out,
-                               mp3_off, mp3_cap, out_len, hide_str_offset_out);
-    if (rc != M3S_OK && h) {   // an early return may leave work of this call on the helper streams: drain them before the caller reuses buffers
-        cudaStreamSynchronize(h->stream);
-        if (h->copy_in) { cudaStreamSynchronize(h->copy_in); cudaStreamSynchronize(h->copy_out); cudaStreamSynchronize(h->aux); }
-    }
-    return rc;
+    if (!h) return M3S_ERR_ARG;
+    h->enc_taps_ok = false;
+    if (sr_index_of(sample_rate) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: sample rate %d is not an MPEG-1 rate", sample_rate);
+    if (br_index_of(bitrate_kbps) < 0)
+        return m3s_fail(h, M3S_ERR_ARG, "encode: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", bitrate_kbps);
+    // the batch's one rate pair, broadcast to every clip
+    const std::vector<int32_t> srs((size_t)std::max(n_clips, 0), sample_rate), brs((size_t)std::max(n_clips, 0), bitrate_kbps);
+    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, srs.data(), brs.data(), payload_bits, payload_off, mp3_out, mp3_off,
+                       mp3_cap, out_len, hide_str_offset_out);
+}
+
+extern "C" int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                                int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
+                                const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
+                                int64_t *out_len, int64_t *hide_str_offset_out)
+{
+    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out, mp3_off,
+                       mp3_cap, out_len, hide_str_offset_out);
 }
 
 static const bool g_enc_trace = getenv("M3S_TRACE") != nullptr;   // host-clock stage timing of the encode call (diagnostic)
@@ -1608,49 +1640,86 @@ static double enc_now_ms()
 #define M3S_ENC_MARK(tag) do { if (g_enc_trace) { const double t__ = enc_now_ms(); fprintf(stderr, "[m3s enc] %-22s +%.2f ms\n", tag, t__ - tr_t); tr_t = t__; } } while (0)
 
 static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                       int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
+                       int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
                        const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
                        int64_t *out_len, int64_t *hide_str_offset_out)
 {
     if (!h) return M3S_ERR_ARG;
     double tr_t = g_enc_trace ? enc_now_ms() : 0.0;
     h->enc_taps_ok = false;
-    if (!pcm || !n_samples || n_clips <= 0 || !mp3_out || !mp3_off) return m3s_fail(h, M3S_ERR_ARG, "encode: null argument");
+    if (!pcm || !n_samples || n_clips <= 0 || !mp3_out || !mp3_off || !sample_rate || !bitrate_kbps)
+        return m3s_fail(h, M3S_ERR_ARG, "encode: null argument");
     if ((uintptr_t)pcm & 3) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm must be 4-byte aligned (one stereo sample per word)");
-    const int sri = sr_index_of(sample_rate), bri = br_index_of(bitrate_kbps);
-    if (sri < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: sample rate %d is not an MPEG-1 rate", sample_rate);
-    if (bri < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", bitrate_kbps);
+    // ---- per-clip checks, in the caller's order, before anything is queued
+    for (int j = 0; j < n_clips; j++) {
+        if (sr_index_of(sample_rate[j]) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: sample rate %d is not an MPEG-1 rate", j, sample_rate[j]);
+        if (br_index_of(bitrate_kbps[j]) < 0)
+            return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", j, bitrate_kbps[j]);
+        if (n_samples[j] < 0 || n_samples[j] % 1152) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d has %lld samples per channel, not a multiple of 1152 (the reference raises IndexError, MP3_Encoder.py:611-614)", j, (long long)n_samples[j]);
+        if (pcm_off && (pcm_off[j] & 1)) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm_off must be even (stereo samples)");
+    }
     M3S_CUDA(h, cudaSetDevice(h->device));
     int rc;
+    // ---- the library's clip order: grouped by sample rate (stable), so that in every chunk the frame slots of one sample rate are
+    //      contiguous and the kernels that stage per-rate tables once per CTA (probe, resolve) run once per group.  Clip i of that
+    //      order is the caller's clip order[i]; every output goes back by the caller's index.
+    std::vector<int> order(n_clips), inv(n_clips);
+    for (int i = 0; i < n_clips; i++) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return sr_index_of(sample_rate[a]) < sr_index_of(sample_rate[b]); });
+    for (int i = 0; i < n_clips; i++) inv[order[i]] = i;
+    int grp[4];   // clips of sample rate index s: [grp[s], grp[s + 1])
+    for (int s = 0, i = 0; s < 4; s++) {
+        while (s < 3 && i < n_clips && sr_index_of(sample_rate[order[i]]) < s) i++;
+        grp[s] = s < 3 ? i : n_clips;
+    }
     // ---- clip table
     std::vector<M3sEncClip> clips(n_clips);
-    int64_t total_frames = 0, pcm_elems = 0, max_frames = 0, out_total = 0, pay_total = 0;
+    int64_t total_frames = 0, max_frames = 0, out_total = 0, pay_total = 0;
     for (int i = 0; i < n_clips; i++) {
-        if (n_samples[i] < 0 || n_samples[i] % 1152) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d has %lld samples per channel, not a multiple of 1152 (the reference raises IndexError, MP3_Encoder.py:611-614)", i, (long long)n_samples[i]);
+        const int j = order[i];
         M3sEncClip &c = clips[i];
-        c.pcm_base = pcm_off ? pcm_off[i] : pcm_elems;
-        if (c.pcm_base & 1) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm_off must be even (stereo samples)");
-        c.n_frames = (int32_t)(n_samples[i] / 1152);
+        c.pcm_base = pcm_off ? pcm_off[j] : 0;
+        c.n_frames = (int32_t)(n_samples[j] / 1152);
         c.frame_base = total_frames;
-        c.out_base = mp3_off[i];
-        c.payload_base = payload_bits && payload_off ? payload_off[i] : 0;
-        c.payload_len = payload_bits && payload_off ? payload_off[i + 1] - payload_off[i] : 0;
-        c.pad = 0;
+        c.out_base = mp3_off[j];
+        c.payload_base = payload_bits && payload_off ? payload_off[j] : 0;
+        c.payload_len = payload_bits && payload_off ? payload_off[j + 1] - payload_off[j] : 0;
+        c.sr_idx = (int16_t)sr_index_of(sample_rate[j]);
+        c.bitrate_idx = (int16_t)br_index_of(bitrate_kbps[j]);
         total_frames += c.n_frames;
-        pcm_elems = std::max(pcm_elems, c.pcm_base + 2 * n_samples[i]);
         max_frames = std::max<int64_t>(max_frames, c.n_frames);
         pay_total = std::max(pay_total, c.payload_base + c.payload_len);
     }
-    std::vector<uint32_t> byteoff;
-    int whole = 0;
-    padding_prefix(sample_rate, bitrate_kbps, max_frames, byteoff, whole);
-    for (int i = 0; i < n_clips; i++) {
-        M3sEncClip &c = clips[i];
-        c.out_len = (int64_t)(byteoff[c.n_frames] / 4) * 4;
-        if (mp3_cap && mp3_cap[i] < c.out_len) return m3s_fail(h, M3S_ERR_CAPACITY, "encode: clip %d needs %lld output bytes, capacity %lld", i, (long long)c.out_len, (long long)mp3_cap[i]);
+    if (!pcm_off) {   // back to back in the caller's order
+        int64_t e = 0;
+        for (int j = 0; j < n_clips; j++) { clips[inv[j]].pcm_base = e; e += 2 * n_samples[j]; }
+    }
+    // ---- padding tables: one per rate pair of the batch, sized to its longest clip, back to back
+    int64_t pair_frames[3][16];
+    for (auto &r : pair_frames) for (int64_t &v : r) v = -1;
+    for (const M3sEncClip &c : clips) pair_frames[c.sr_idx][c.bitrate_idx] = std::max<int64_t>(pair_frames[c.sr_idx][c.bitrate_idx], c.n_frames);
+    static const int kRates[3] = {44100, 48000, 32000};
+    std::vector<uint32_t> byteoff, tab;
+    int pair_base[3][16] = {}, pair_whole[3][16] = {};
+    for (int s = 0; s < 3; s++)
+        for (int b = 1; b < 15; b++) {
+            if (pair_frames[s][b] < 0) continue;
+            padding_prefix(kRates[s], kBitrates[b], pair_frames[s][b], tab, pair_whole[s][b]);
+            if (byteoff.size() + tab.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode: too many frames in one call");
+            pair_base[s][b] = (int)byteoff.size();
+            byteoff.insert(byteoff.end(), tab.begin(), tab.end());
+        }
+    for (M3sEncClip &c : clips) {
+        c.pad_base = pair_base[c.sr_idx][c.bitrate_idx];
+        c.whole_slots = pair_whole[c.sr_idx][c.bitrate_idx];
+        c.out_len = (int64_t)(byteoff[(size_t)c.pad_base + c.n_frames] / 4) * 4;
         out_total = std::max(out_total, c.out_base + c.out_len);
-        if (out_len) out_len[i] = c.out_len;
-        if (hide_str_offset_out) hide_str_offset_out[i] = 0;
+    }
+    for (int j = 0; j < n_clips; j++) {
+        const M3sEncClip &c = clips[inv[j]];
+        if (mp3_cap && mp3_cap[j] < c.out_len) return m3s_fail(h, M3S_ERR_CAPACITY, "encode: clip %d needs %lld output bytes, capacity %lld", j, (long long)c.out_len, (long long)mp3_cap[j]);
+        if (out_len) out_len[j] = c.out_len;
+        if (hide_str_offset_out) hide_str_offset_out[j] = 0;
     }
     if (total_frames == 0) return M3S_OK;
     M3S_ENC_MARK("clip table");
@@ -1762,10 +1831,13 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     std::vector<int32_t> fc_count((size_t)n_clips * n_chunks);   // frame_clip array, whose chunk k is [slot_off[k], slot_off[k+1])
     std::vector<M3sEncClip> cclips((size_t)n_clips * n_chunks);   // chunk-local clip records
     std::vector<int64_t> work_off(n_chunks + 1, 0), slot_off(n_chunks + 1, 0);
+    std::vector<int64_t> grp_slot((size_t)n_chunks * 4);   // chunk k: the frame slots of sample rate index s are [grp_slot[4k + s], grp_slot[4k + s + 1])
     for (int64_t k = 0; k < n_chunks; k++) {
         const int64_t c0 = k * cf;
         int64_t base = 0;
         for (int i = 0; i < n_clips; i++) {
+            for (int s = 0; s < 4; s++)
+                if (grp[s] == i) grp_slot[(size_t)k * 4 + s] = base;
             const int64_t nfc = frames_in_chunk(i, c0);
             M3sEncClip &cc = cclips[(size_t)k * n_clips + i];
             cc = clips[i];
@@ -1783,6 +1855,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             fc_count[(size_t)k * n_clips + i] = (int32_t)nfc;
             base += nfc;
         }
+        for (int s = 0; s < 4; s++)
+            if (grp[s] == n_clips) grp_slot[(size_t)k * 4 + s] = base;
         work_off[k + 1] = (int64_t)work.size();
         slot_off[k + 1] = slot_off[k] + base;
     }
@@ -1821,7 +1895,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         M3S_KBEGIN(h, M3S_K_ENC_ANALYSIS);
         k_enc_analysis_fold<<<(unsigned)nw, 32 * ANA3_WARPS, sizeof(Ana3Smem), h->aux>>>(
             k_pcm, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips, (const M3sEncWork *)h->e_work.p + work_off[k], h->d_tab,
-            (const EncTables *)h->e_tabs.p, sri, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p, 0u);
+            (const EncTables *)h->e_tabs.p, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p, 0u);
         M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].a1, h->aux);
         M3S_CUDA(h, cudaEventRecord(h->ev_ana[pb], h->aux));
@@ -1836,6 +1910,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     //        aux       analysis of chunk k+1                  queued behind the packing of chunk k
     //        stream    rate loop + packing of chunk k         the critical path: back to back, chunk after chunk
     //        copy_out  MP3 bytes of chunk k                   (host buffers only)
+    //      The probe and resolve kernels stage per-sample-rate tables once per CTA: they run once per sample rate present in the
+    //      chunk, over its frame slots / clips.  The other kernels read the rate from the clip record and run once per chunk.
     if (host && n_chunks > 1) M3S_CUDA(h, stage_chunk(1));
     if ((rc = launch_analysis(0))) return rc;
     for (int64_t k = 0; k < n_chunks; k++) {
@@ -1844,26 +1920,34 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         const int64_t chunk_total = slot_off[k + 1] - slot_off[k];
         if (chunk_total == 0) break;
         const M3sEncClip *d_clips = (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips;
+        const int64_t *gsl = &grp_slot[(size_t)k * 4];
         M3S_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_ana[pb], 0));
         const int64_t n_gran = 4 * chunk_total;
-        M3S_KBEGIN(h, M3S_K_ENC_RATE);
-        k_enc_probe<<<(unsigned)((n_gran + PROBE_WARPS * PROBE_G - 1) / (PROBE_WARPS * PROBE_G)), 32 * PROBE_WARPS, sizeof(ProbeSmem), h->stream>>>(
-            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-            sri, whole, n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint4 *)b_var[pb]->p,
-            (uint32_t *)b_sum[pb]->p, (uint8_t *)b_scfsi[pb]->p);
-        M3S_LAUNCH_CHECK(h);
+        for (int s = 0; s < 3; s++) {
+            const int64_t g0 = 4 * gsl[s], g1 = 4 * gsl[s + 1];
+            if (g1 == g0) continue;
+            M3S_KBEGIN(h, M3S_K_ENC_RATE);
+            k_enc_probe<<<(unsigned)((g1 - g0 + PROBE_WARPS * PROBE_G - 1) / (PROBE_WARPS * PROBE_G)), 32 * PROBE_WARPS, sizeof(ProbeSmem), h->stream>>>(
+                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+                s, g0, g1, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint4 *)b_var[pb]->p,
+                (uint32_t *)b_sum[pb]->p, (uint8_t *)b_scfsi[pb]->p);
+            M3S_LAUNCH_CHECK(h);
+        }
         if (g_enc_trace) tmark(tev[k].r1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_rate[pb], h->stream));
         if (host && k + 2 < n_chunks) M3S_CUDA(h, stage_chunk(k + 2));
-        M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
-        k_enc_resolve<<<(unsigned)((n_clips + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
-            d_clips, n_clips, (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-            (const uint8_t *)h->e_payload.p, sri, whole, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
-            (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
-        M3S_LAUNCH_CHECK(h);
+        for (int s = 0; s < 3; s++) {
+            if (gsl[s + 1] == gsl[s]) continue;   // no clip of this sample rate has a frame in the chunk
+            M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
+            k_enc_resolve<<<(unsigned)((grp[s + 1] - grp[s] + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
+                d_clips, grp[s], grp[s + 1], (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+                (const uint8_t *)h->e_payload.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
+                (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
+            M3S_LAUNCH_CHECK(h);
+        }
         M3S_KBEGIN(h, M3S_K_ENC_AUX);
         k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
-            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, sri, (int32_t)c0, (int32_t)cf,
+            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (int32_t)c0, (int32_t)cf,
             n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
             (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
             (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
@@ -1872,8 +1956,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         // packing stays on the rate loop's stream
         M3S_KBEGIN(h, M3S_K_ENC_PACK);
         k_enc_pack<<<(unsigned)((chunk_total + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
-            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const uint32_t *)h->e_pad.p, sri, bri, whole, 0,
-            chunk_total, (const uint32_t *)b_ix[pb]->p, (const int32_t *)b_info[pb]->p, (const uint8_t *)b_scfsi[pb]->p, d_out);
+            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const uint32_t *)h->e_pad.p, 0, chunk_total,
+            (const uint32_t *)b_ix[pb]->p, (const int32_t *)b_info[pb]->p, (const uint8_t *)b_scfsi[pb]->p, d_out);
         M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].p1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_pack[pb], h->stream));
@@ -1889,7 +1973,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             for (int i = 0; i < n_clips; i++) {
                 const int64_t nfc = frames_in_chunk(i, c0);
                 if (nfc == 0) continue;
-                const int64_t b0 = byteoff[c0], b1 = std::min<int64_t>(byteoff[c0 + nfc], clips[i].out_len);
+                const uint32_t *bo = byteoff.data() + clips[i].pad_base;
+                const int64_t b0 = bo[c0], b1 = std::min<int64_t>(bo[c0 + nfc], clips[i].out_len);
                 if (b1 <= b0) continue;
                 M3sRow r;
                 r.dst = (char *)mp3_out + clips[i].out_base + b0;
@@ -1917,16 +2002,27 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         for (int64_t k = 0; k < n_chunks; k++)
             for (cudaEvent_t e : {tev[k].c0, tev[k].c1, tev[k].a0, tev[k].a1, tev[k].r1, tev[k].p1, tev[k].o1}) if (e) cudaEventDestroy(e);
     }
-    // ---- results
+    // ---- results, by the caller's clip index
     std::vector<M3sEncState> states(n_clips);
     M3S_CUDA(h, cudaMemcpyAsync(states.data(), h->e_state.p, sizeof(M3sEncState) * n_clips, cudaMemcpyDeviceToHost, h->stream));
     M3S_CUDA(h, cudaStreamSynchronize(h->stream));
     if (hide_str_offset_out)
-        for (int i = 0; i < n_clips; i++) hide_str_offset_out[i] = states[i].hide_off;
-    for (int i = 0; i < n_clips; i++)
-        if (states[i].overrun)
+        for (int j = 0; j < n_clips; j++) hide_str_offset_out[j] = states[inv[j]].hide_off;
+    for (int j = 0; j < n_clips; j++)
+        if (states[inv[j]].overrun)
             return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d frame %d: the step search runs past the end of the step table (quantize would "
-                            "read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)", i, states[i].overrun - 1);
+                            "read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)", j, states[inv[j]].overrun - 1);
+    // taps: the device holds the frames in the library's clip order; (device frame, caller frame, frames) runs map them back
+    h->enc_tap_runs.clear();
+    std::vector<int64_t> caller_fb(n_clips + 1, 0);
+    for (int j = 0; j < n_clips; j++) caller_fb[j + 1] = caller_fb[j] + n_samples[j] / 1152;
+    for (int i = 0; i < n_clips; i++) {
+        const int64_t src = clips[i].frame_base, dst = caller_fb[order[i]], n = clips[i].n_frames;
+        std::vector<int64_t> &R = h->enc_tap_runs;
+        if (n == 0) continue;
+        if (!R.empty() && R[R.size() - 3] + R.back() == src && R[R.size() - 2] + R.back() == dst) R.back() += n;
+        else R.insert(R.end(), {src, dst, n});
+    }
     h->enc_taps_ok = single_chunk;
     h->enc_total_frames = total_frames;
     h->enc_n_clips = n_clips;
@@ -1939,12 +2035,16 @@ extern "C" int m3s_encode_taps(m3s_handle_t h, int32_t *mdct, int32_t *ix, int32
     if (!h->enc_taps_ok) return m3s_fail(h, M3S_ERR_STATE, "encode_taps: the last m3s_encode ran in several chunks (or failed); taps need a single-chunk batch");
     M3S_CUDA(h, cudaSetDevice(h->device));
     const int64_t nf = h->enc_total_frames;
-    if (mdct) M3S_CUDA(h, cudaMemcpyAsync(mdct, h->e_mdct.p, (size_t)nf * 4 * 576 * 4, cudaMemcpyDeviceToHost, h->stream));
-    if (info) M3S_CUDA(h, cudaMemcpyAsync(info, h->e_info.p, (size_t)nf * 4 * ENC_INFO_FIELDS * 4, cudaMemcpyDeviceToHost, h->stream));
+    const std::vector<int64_t> &R = h->enc_tap_runs;   // (device frame, caller frame, frames): one run when the order is the caller's
+    const size_t NM = 4 * 576, NI = 4 * ENC_INFO_FIELDS;   // values per frame
+    for (size_t r = 0; r < R.size(); r += 3) {
+        if (mdct) M3S_CUDA(h, cudaMemcpyAsync(mdct + R[r + 1] * NM, (const int32_t *)h->e_mdct.p + R[r] * NM, R[r + 2] * NM * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (info) M3S_CUDA(h, cudaMemcpyAsync(info + R[r + 1] * NI, (const int32_t *)h->e_info.p + R[r] * NI, R[r + 2] * NI * 4, cudaMemcpyDeviceToHost, h->stream));
+    }
     std::vector<int16_t> ix16;
     std::vector<uint8_t> sc8;
     if (ix) {
-        ix16.resize((size_t)nf * 4 * 576);
+        ix16.resize((size_t)nf * NM);
         M3S_CUDA(h, cudaMemcpyAsync(ix16.data(), h->e_ix.p, ix16.size() * 2, cudaMemcpyDeviceToHost, h->stream));
     }
     if (scfsi) {
@@ -1952,7 +2052,9 @@ extern "C" int m3s_encode_taps(m3s_handle_t h, int32_t *mdct, int32_t *ix, int32
         M3S_CUDA(h, cudaMemcpyAsync(sc8.data(), h->e_scfsi.p, sc8.size(), cudaMemcpyDeviceToHost, h->stream));
     }
     M3S_CUDA(h, cudaStreamSynchronize(h->stream));
-    if (ix) for (size_t i = 0; i < ix16.size(); i++) ix[i] = ix16[i];
-    if (scfsi) for (size_t i = 0; i < sc8.size(); i++) scfsi[i] = sc8[i];
+    for (size_t r = 0; r < R.size(); r += 3) {
+        if (ix) for (size_t i = 0; i < (size_t)R[r + 2] * NM; i++) ix[R[r + 1] * NM + i] = ix16[R[r] * NM + i];
+        if (scfsi) for (size_t i = 0; i < (size_t)R[r + 2] * 8; i++) scfsi[R[r + 1] * 8 + i] = sc8[R[r] * 8 + i];
+    }
     return M3S_OK;
 }

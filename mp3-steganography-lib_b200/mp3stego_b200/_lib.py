@@ -60,6 +60,9 @@ SYMBOLS = [
     ("m3s_encode", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, _c_i64p, _c_i64p, ctypes.c_int32,
                                   ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, _c_i64p, ctypes.c_void_p, _c_i64p,
                                   _c_i64p, _c_i64p, _c_i64p]),
+    ("m3s_encode_mixed", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, _c_i64p, _c_i64p, ctypes.c_int32,
+                                        _c_i32p, _c_i32p, ctypes.c_void_p, _c_i64p, ctypes.c_void_p, _c_i64p,
+                                        _c_i64p, _c_i64p, _c_i64p]),
     ("m3s_encode_taps", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                        ctypes.c_void_p]),
     ("m3s_table_export", ctypes.c_int64, [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64]),
@@ -321,20 +324,29 @@ class Handle:
     def encode(self, pcm, n_samples, sample_rate, bitrate_kbps, payloads=None, pcm_off=None, mp3_out=None, taps=False,
                compact=False, payload_packed=None):
         """E1-E3 over a batch of int16 stereo clips laid end to end in `pcm` (numpy or torch, host or cuda).
-        compact=True lays the MP3s back to back at their exact sizes (m3s_encode_size), so that (mp3, mp3_off + [end])
-        can be fed straight to decode_scan.  payload_packed = (uint8 array of '0'/'1' chars, offsets[n+1]) avoids re-joining.
-        Raises IndexError, for the whole batch, when a clip drives the rate loop past the end of the step table."""
+        sample_rate and bitrate_kbps are ints (one rate pair for the batch, m3s_encode) or sequences with one entry per clip
+        (m3s_encode_mixed: clips of different rates in one call).
+        compact=True lays the MP3s back to back at their exact sizes (m3s_encode_size at each clip's pair), so that
+        (mp3, mp3_off + [end]) can be fed straight to decode_scan.  payload_packed = (uint8 array of '0'/'1' chars, offsets[n+1])
+        avoids re-joining.  Raises IndexError, for the whole batch, when a clip drives the rate loop past the end of the step table."""
         L = self._L
         n = len(n_samples)
         ns, ns_p = _i64(n_samples)
         if pcm_off is None:
             pcm_off = np.concatenate([[0], np.cumsum(ns * 2)])[:-1]
         po, po_p = _i64(pcm_off)
+        mixed = not (np.isscalar(sample_rate) and np.isscalar(bitrate_kbps))
+        if mixed:
+            srs = np.ascontiguousarray(np.broadcast_to(np.asarray(sample_rate, np.int32), (n,)))
+            brs = np.ascontiguousarray(np.broadcast_to(np.asarray(bitrate_kbps, np.int32), (n,)))
+            keys = list(zip(ns.tolist(), srs.tolist(), brs.tolist()))
+        else:
+            keys = [(int(s), sample_rate, bitrate_kbps) for s in ns]
         size_fn = L.m3s_encode_size if compact else L.m3s_encode_bound
-        uniq = {int(s): size_fn(int(s), sample_rate, bitrate_kbps) for s in set(int(v) for v in ns)}
-        bounds = np.array([uniq[int(s)] for s in ns], np.int64)
+        uniq = {k: size_fn(*k) for k in set(keys)}
+        bounds = np.array([uniq[k] for k in keys], np.int64)
         if (bounds < 0).any():
-            raise M3SError("encode: unsupported sample count / sample rate / bitrate")
+            raise M3SError(f"encode: clip {int(np.argmax(bounds < 0))}: unsupported sample count / sample rate / bitrate")
         mo, mo_p = _i64(np.concatenate([[0], np.cumsum(bounds)])[:-1])
         mc, mc_p = _i64(bounds)
         mem = _mem_of(pcm)
@@ -357,14 +369,19 @@ class Handle:
         out_len = np.zeros(n, np.int64)
         hoff = np.zeros(n, np.int64)
         _ready(pcm, mp3_out)
-        rc = L.m3s_encode(self._h, _ptr(pcm), mem, po_p, ns_p, n, sample_rate, bitrate_kbps, pl_p, ploff_p, _ptr(mp3_out),
-                          mo_p, mc_p, out_len.ctypes.data_as(_c_i64p), hoff.ctypes.data_as(_c_i64p))
+        if mixed:
+            rc = L.m3s_encode_mixed(self._h, _ptr(pcm), mem, po_p, ns_p, n, srs.ctypes.data_as(_c_i32p), brs.ctypes.data_as(_c_i32p),
+                                    pl_p, ploff_p, _ptr(mp3_out), mo_p, mc_p, out_len.ctypes.data_as(_c_i64p),
+                                    hoff.ctypes.data_as(_c_i64p))
+        else:
+            rc = L.m3s_encode(self._h, _ptr(pcm), mem, po_p, ns_p, n, sample_rate, bitrate_kbps, pl_p, ploff_p, _ptr(mp3_out),
+                              mo_p, mc_p, out_len.ctypes.data_as(_c_i64p), hoff.ctypes.data_as(_c_i64p))
         if rc == M3S_ERR_ARG:
             msg = L.m3s_last_error(self._h).decode()
             if STEP_TABLE_OVERRUN in msg:
                 # the reference's quantize() indexes its step table past the end for this input (SURVEY A.E13): no output
                 raise IndexError(f"index out of bounds: {msg}")
-        self._check(rc, "m3s_encode")
+        self._check(rc, "m3s_encode_mixed" if mixed else "m3s_encode")
         res = dict(mp3=mp3_out, mp3_off=mo, out_len=out_len, hide_str_offset=hoff)
         if taps:
             nf = int((ns // 1152).sum())

@@ -4,7 +4,8 @@ call and without leaving the GPU between the decode and the encode half of the c
   reveal_batch   reveal_massage for N files: frame walk + side-info scan + reveal bits only (D0 + D4, ~36 B/frame of traffic);
                  no Huffman decode, no synthesis, no temp WAV
   hide_batch     hide_message for N files: decode (float64 instantiation, so the int16 PCM equals the reference's WAV sample
-                 for sample) -> encode + hide at each file's own bitrate; the PCM stays in HBM
+                 for sample) -> encode + hide at each file's own sample rate and bitrate, all files in one encode call; the PCM
+                 stays in HBM
   clear_batch    clear_file: the same with no payload
 The semantics per file are the facade's: message framing '<len>#<message>' as utf-8 bits (steganography.py:10-24,88-90),
 bitrate of the last frame (MP3_Parser.py:93-97), too_long = hide_str_offset < len(bits) - 1 (encoder.py:49-51),
@@ -103,27 +104,20 @@ def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[in
             raise IndexError(f"file {i}: the reference encoder only handles stereo input (WAV_Reader / MP3_Encoder.py:611-614)")
     rows = sc["pcm_rows"].astype(np.int64)
     pcm_off = sc["pcm_off"]
-    out: List[bytes] = [b""] * n
-    hoff = [0] * n
-    # one encode call per (sample rate, bitrate) group: the encoder takes one rate pair per batch
-    key = sc["sample_rate"].astype(np.int64) * 1000 + sc["bitrate"].astype(np.int64) // 1000
-    for k in np.unique(key):
-        idx = np.nonzero(key == k)[0]
-        sr, kbps = int(k) // 1000, int(k) % 1000
-        res = handle.encode(pcm, rows[idx], sr, kbps, payloads=[payloads[i] for i in idx], pcm_off=pcm_off[idx], compact=True)
-        mark("encode")
-        nbytes = int(res["mp3_off"][-1] + res["out_len"][-1])
-        back = _pinned(handle, "out", nbytes)
-        back[:nbytes].copy_(res["mp3"][:nbytes], non_blocking=True)
-        torch.cuda.current_stream(dev).synchronize()
-        mark("download")
-        mv = memoryview(back.numpy())
-        for m, i in enumerate(idx):
-            o = int(res["mp3_off"][m])
-            out[i] = bytes(mv[o:o + int(res["out_len"][m])])
-            hoff[i] = int(res["hide_str_offset"][m])
-        mark("cut")
-    return out, hoff, [int(b) // 1000 for b in sc["bitrate"]]
+    kbps = sc["bitrate"].astype(np.int64) // 1000
+    # one encode call for the whole batch, every file at its own sample rate and last-frame bitrate
+    res = handle.encode(pcm, rows, sc["sample_rate"], kbps, payloads=list(payloads), pcm_off=pcm_off[:n], compact=True)
+    mark("encode")
+    nbytes = int(res["mp3_off"][-1] + res["out_len"][-1])
+    back = _pinned(handle, "out", nbytes)
+    back[:nbytes].copy_(res["mp3"][:nbytes], non_blocking=True)
+    torch.cuda.current_stream(dev).synchronize()
+    mark("download")
+    mv = memoryview(back.numpy())
+    out = [bytes(mv[o:o + ln]) for o, ln in zip(res["mp3_off"].tolist(), res["out_len"].tolist())]
+    hoff = res["hide_str_offset"].tolist()
+    mark("cut")
+    return out, hoff, kbps.tolist()
 
 
 def hide_batch(handle: "_lib.Handle", blobs: Sequence[bytes], messages: Sequence[str]) -> Tuple[List[bytes], List[bool]]:

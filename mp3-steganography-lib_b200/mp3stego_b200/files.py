@@ -4,7 +4,8 @@
                  ID3v2 skip, parse, write_to_wav via scipy's layout, optional reveal text), with the reads on a thread pool into
                  ONE pinned buffer, one self-pipelining m3s_decode call for the whole batch, and the WAV writes on the pool again
   encode_files   WAV files -> MP3 files (optionally hiding one message per file): what Encoder.encode does per file
-                 (encoder.py:22-51, WAV_Reader.py:30-110), same structure around one m3s_encode call per sample rate
+                 (encoder.py:22-51, WAV_Reader.py:30-110), same structure around one m3s_encode_mixed call for all files, each
+                 at its own sample rate and bitrate
 
 torch is used for pinned host memory only.  Per-file failures follow the reference: sys.exit messages for missing files / bad
 WAV headers, IndexError for input the reference's encoder cannot read (mono, length not a multiple of 1152, a clip that drives the rate loop past the step table)."""
@@ -12,7 +13,7 @@ import os
 import struct
 import sys
 from concurrent.futures import ThreadPoolExecutor
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Union
 
 import numpy as np
 
@@ -96,48 +97,51 @@ def decode_files(handle: "_lib.Handle", mp3_paths: Sequence[str], wav_paths: Opt
     return out
 
 
-def encode_files(handle: "_lib.Handle", wav_paths: Sequence[str], mp3_paths: Sequence[str], bitrate: int = 320,
+def encode_files(handle: "_lib.Handle", wav_paths: Sequence[str], mp3_paths: Sequence[str], bitrate: Union[int, Sequence[int]] = 320,
                  messages: Optional[Sequence[str]] = None, threads: int = 8) -> List[bool]:
-    """Encode N WAV files to MP3 files at `bitrate` kbps, hiding messages[i] ('' or None = plain encode) in file i with the facade's
-    '<len>#<message>' framing (steganography.py:44-47).  Returns the too_long flags (encoder.py:49-51)."""
+    """Encode N WAV files to MP3 files at `bitrate` kbps -- one int for every file, or one entry per file (the reference's
+    Encoder(file, out, bitrate=...) sets it per file) -- hiding messages[i] ('' or None = plain encode) in file i with the facade's
+    '<len>#<message>' framing (steganography.py:44-47).  All files go through one encode call whatever their sample rates and
+    bitrates.  Returns the too_long flags (encoder.py:49-51)."""
     n = len(wav_paths)
     if n == 0:
         return []
     if len(mp3_paths) != n or (messages is not None and len(messages) != n):
         raise ValueError("one output path (and one message) per input file")
+    rates = [bitrate] * n if isinstance(bitrate, (int, np.integer)) else list(bitrate)
+    if len(rates) != n:
+        raise ValueError("one bitrate per input file")
     for p in wav_paths:
         if not os.path.exists(p):
             sys.exit(f"File {p} not found.")
-    if bitrate not in MPEG1_L3_BITRATES:
-        sys.exit("Unsupported bitrate configuration.")
+    for b in rates:
+        if b not in MPEG1_L3_BITRATES:
+            sys.exit("Unsupported bitrate configuration.")
     with ThreadPoolExecutor(max(1, threads)) as pool:
-        readers = list(pool.map(lambda p: WavReader(p, bitrate), wav_paths))   # header checks + sample buffer, reference semantics
+        readers = list(pool.map(WavReader, wav_paths, rates))   # header checks + sample buffer, reference semantics
         for w in readers:
             if w.num_of_channels != 2:
                 raise IndexError("index out of bounds: the reference encoder only works on 16-bit stereo input")
             if w.num_of_samples % 1152 or len(w.buffer) < 2 * w.num_of_samples:
                 raise IndexError("index out of bounds: sample count is not a multiple of 1152")
         bits = [str_to_binary_str(str(len(m)) + "#" + m) if m else "" for m in (messages or [""] * n)]
-        too_long = [False] * n
-        for sr in sorted({w.samplerate for w in readers}):
-            idx = [i for i in range(n) if readers[i].samplerate == sr]
-            ns = [readers[i].num_of_samples for i in idx]
-            po = np.concatenate([[0], np.cumsum([2 * s for s in ns])]).astype(np.int64)
-            stage = _pinned(2 * int(po[-1])).view(dtype=__import__("torch").int16)
-            sv = stage.numpy()
+        ns = [w.num_of_samples for w in readers]
+        po = np.concatenate([[0], np.cumsum([2 * s for s in ns])]).astype(np.int64)
+        stage = _pinned(2 * int(po[-1])).view(dtype=__import__("torch").int16)
+        sv = stage.numpy()
 
-            def fill(k):
-                sv[po[k]:po[k + 1]] = readers[idx[k]].buffer[: 2 * ns[k]]
+        def fill(i):
+            sv[po[i]:po[i + 1]] = readers[i].buffer[: 2 * ns[i]]
 
-            list(pool.map(fill, range(len(idx))))
-            res = handle.encode(stage[: int(po[-1])], ns, sr, bitrate, payloads=[bits[i] for i in idx], pcm_off=po[:-1], compact=True)
-            mp3 = res["mp3"]
+        list(pool.map(fill, range(n)))
+        res = handle.encode(stage[: int(po[-1])], ns, [w.samplerate for w in readers], rates, payloads=bits, pcm_off=po[:-1],
+                            compact=True)
+        mp3 = res["mp3"]
 
-            def write(k):
-                o, ln = int(res["mp3_off"][k]), int(res["out_len"][k])
-                with open(mp3_paths[idx[k]], "wb") as f:
-                    f.write(memoryview(np.ascontiguousarray(mp3[o:o + ln])).cast("B"))
-                too_long[idx[k]] = int(res["hide_str_offset"][k]) < len(bits[idx[k]]) - 1
+        def write(i):
+            o, ln = int(res["mp3_off"][i]), int(res["out_len"][i])
+            with open(mp3_paths[i], "wb") as f:
+                f.write(memoryview(np.ascontiguousarray(mp3[o:o + ln])).cast("B"))
 
-            list(pool.map(write, range(len(idx))))
-    return too_long
+        list(pool.map(write, range(n)))
+    return [int(res["hide_str_offset"][i]) < len(bits[i]) - 1 for i in range(n)]
