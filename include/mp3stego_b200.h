@@ -200,6 +200,28 @@ M3S_API int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, const 
                              int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
                              const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
                              int64_t *out_len, int64_t *hide_str_offset_out);
+/* hide_str_offset of many candidate payloads per clip, without writing MP3 bytes: how much of a message fits in a clip, answered
+ * for every prefix at once.  The analysis and the rate loop's probe of every payload variant run once per clip; only the offset
+ * chain runs per candidate, so the call costs about one encode without the quantisation and the bit packing.
+ *   pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps   as m3s_encode_mixed (pcm host or device per mem)
+ *   body          host bytes; clip i's body is body[body_off[i] .. body_off[i+1])
+ *   body_off      [n_clips+1] host
+ *   cand_off      [n_clips+1] host, cand_off[0] = 0: the candidates of clip i are c in [cand_off[i], cand_off[i+1]); a clip may have none
+ *   head          host bytes; candidate c's head is head[head_off[c] .. head_off[c+1]), at most 32 bytes
+ *   head_off      [n_cand+1] host, n_cand = cand_off[n_clips]
+ *   body_len      [n_cand] host: candidate c hides the MSB-first bits of its head followed by the first body_len[c] bytes of its
+ *                 clip's body.  (The facade frames message[:n] as head "<n>#" and body = the message's utf-8 bytes.)
+ *   hide_str_offset_out  [n_cand] host: what m3s_encode_mixed returns as clip i's hide_str_offset with that payload as '0'/'1'
+ *                 chars; an empty payload gets the plain encode's offset.
+ * The clip checks of m3s_encode_mixed apply; a head over 32 bytes, a body_len past the clip's body or bad offsets fail with
+ * M3S_ERR_ARG before anything is queued, the text naming the clip and the candidate.  A step-table overrun (see m3s_encode) under
+ * any candidate fails the whole call, the text naming the caller's clip, the candidate and the frame ("clip %d candidate %lld
+ * frame %d: ... runs past the end of the step table"); the handle stays usable.  m3s_encode_taps fails after this call. */
+M3S_API int m3s_encode_offsets(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                               int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps,
+                               const uint8_t *body, const int64_t *body_off, const int64_t *cand_off,
+                               const uint8_t *head, const int64_t *head_off, const int64_t *body_len,
+                               int64_t *hide_str_offset_out);
 /* Parity taps of the last m3s_encode / m3s_encode_mixed call (host buffers): mdct int32 [frames][ch][gr][576] (MP3_Encoder.py:652),
  * ix int32 [frames][ch][gr][576] signed as written (:1272-1276), info int32 [frames][gr][ch][16]:
  * part2_3_length, big_values, count1, global_gain, table_select[3], region0_count, region1_count,
@@ -224,6 +246,7 @@ enum {
     M3S_K_ENC_RESOLVE,   /* E2b per-clip sequential offset scan over granule variants */
     M3S_K_ENC_PACK,      /* E3 side-info + main-data bit packing */
     M3S_K_ENC_AUX,       /* E2c quantisation at the chosen step (k_enc_emit) */
+    M3S_K_ENC_OFFSETS,   /* E2d m3s_encode_offsets: the offset chains of many candidate payloads per clip (k_enc_offsets) */
     M3S_K_COUNT
 };
 M3S_API int m3s_timing_enable(m3s_handle_t h, int on);

@@ -231,6 +231,7 @@ struct m3s_ctx {
     // ---- encode state
     M3sBuf e_clips2, e_mdct2, e_gran2, e_ix2, e_info2, e_scfsi2;   // second set of the buffers the analysis writes ahead
     M3sBuf e_var, e_var2, e_sum, e_sum2;   // per-granule variant records / summaries of the parallel rate loop (k_enc_probe -> k_enc_resolve)
+    M3sBuf e_cand;   // m3s_encode_offsets: candidate records, work items, heads and bodies
     M3sBuf e_pcm, e_clips, e_mdct, e_ix, e_info, e_gran, e_out, e_payload, e_misc, e_pad, e_tabs, e_state, e_lastix, e_scfsi, e_work;
     bool enc_taps_ok = false;
     int64_t enc_chunk_budget = 0;   // frames of intermediates kept per chunk (0 = default; M3S_ENC_CHUNK_FRAMES overrides)

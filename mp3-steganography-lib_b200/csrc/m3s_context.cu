@@ -233,7 +233,7 @@ static void build_tables(M3sDevTables *T)
 
 static_assert(sizeof(M3S_HUFF_PACKED) / sizeof(uint32_t) == 1410, "packed code book size");
 
-extern "C" int m3s_version(void) { return 300; }
+extern "C" int m3s_version(void) { return 400; }
 
 extern "C" int m3s_create(int device, m3s_handle_t *out)
 {
@@ -392,7 +392,7 @@ extern "C" int m3s_destroy(m3s_handle_t h)
                       &h->b_work, &h->b_spec_export, &h->e_pcm, &h->e_clips, &h->e_mdct,
                       &h->e_ix, &h->e_info, &h->e_gran, &h->e_out, &h->e_payload, &h->e_misc, &h->e_pad, &h->e_tabs, &h->e_state,
                       &h->e_lastix, &h->e_scfsi, &h->e_work, &h->e_clips2, &h->e_mdct2, &h->e_gran2, &h->e_ix2, &h->e_info2, &h->e_scfsi2,
-                      &h->e_var, &h->e_var2, &h->e_sum, &h->e_sum2};
+                      &h->e_var, &h->e_var2, &h->e_sum, &h->e_sum2, &h->e_cand};
     for (M3sBuf *b : bufs) free_buf(*b);
     for (M3sScanSet &ss : h->ss) {
         M3sBuf *sb[] = {&ss.files, &ss.fouts, &ss.tmp_pos, &ss.fr_pos, &ss.fr_P, &ss.fr_meta, &ss.fr_carry, &ss.fr_reveal, &ss.fr_file,
@@ -513,7 +513,8 @@ extern "C" int m3s_timing_get(m3s_handle_t h, int kernel_id, double *total_ms, i
 extern "C" const char *m3s_kernel_name(int kernel_id)
 {
     static const char *names[M3S_K_COUNT] = {"k_walk", "k_fscan", "k_sideinfo", "k_strip", "k_huff", "k_spec_export", "k_hybrid",
-                                             "k_enc_analysis", "k_enc_rate", "k_enc_resolve", "k_enc_pack", "k_enc_emit"};
+                                             "k_enc_analysis", "k_enc_rate", "k_enc_resolve", "k_enc_pack", "k_enc_emit",
+                                             "k_enc_offsets"};
     return kernel_id >= 0 && kernel_id < M3S_K_COUNT ? names[kernel_id] : "?";
 }
 

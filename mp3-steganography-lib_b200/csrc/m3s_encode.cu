@@ -1265,6 +1265,144 @@ k_enc_resolve(const M3sEncClip *__restrict__ clips, int c_begin, int c_end, M3sE
     }
 }
 
+// ================================================================================================
+// E2 for many payloads: k_enc_offsets (m3s_encode_offsets).  hide_str_offset of up to 32 candidate payloads of ONE clip per warp,
+// lane = candidate, against the one probe pass of the clip: per granule every lane reads the same summary word, takes the <= 3
+// bits at its own offset, and adds the count of its variant.  It writes nothing but the candidates' carried state: `sum` and
+// `var` are read by every warp of the clip.
+// ================================================================================================
+struct M3sOffCand {        // candidate payload: the MSB-first bits of head[0 .. head_len) followed by body[body_base .. body_base + body_len)
+    int64_t body_base;     // first body byte in the call's body buffer
+    int64_t nbits;         // 8 * (head_len + body_len)
+    int32_t head_base;     // first head byte in the call's head buffer
+    int32_t head_len;      // <= 32
+};
+struct M3sOffWork {        // one warp: candidates [cand_first, cand_first + count) of library clip `clip`, count <= 32
+    int32_t clip;
+    int32_t count;
+    int64_t cand_first;
+};
+
+#define OFFSETS_WARPS 2
+__global__ void __launch_bounds__(32 * OFFSETS_WARPS)
+k_enc_offsets(const M3sEncClip *__restrict__ clips, const M3sOffWork *__restrict__ work, int w_begin, int w_end,
+              const M3sOffCand *__restrict__ cands, const uint8_t *__restrict__ head, const uint8_t *__restrict__ body,
+              M3sEncState *__restrict__ states, const M3sDevTables *__restrict__ T, const EncTables *__restrict__ ET,
+              const uint32_t *__restrict__ byteoff, int sr_idx, int32_t chunk_first, int32_t chunk_frames,
+              const int32_t *__restrict__ mdct, const M3sEncStats *__restrict__ stats, const uint4 *__restrict__ var,
+              const uint32_t *__restrict__ sum)
+{   // work items [w_begin, w_end): the candidates of the clips at sample rate sr_idx
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    RateSmem &S = *reinterpret_cast<RateSmem *>(smem_raw);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t FULL = 0xFFFFFFFFu;
+    rate_tables_load(S, T, ET, tid, 32 * OFFSETS_WARPS);
+    if (tid < 24) S.sfb[tid] = tid < 23 ? T->sfb_long[sr_idx][tid] : 576;
+    __syncthreads();
+    const int w = w_begin + blockIdx.x * OFFSETS_WARPS + warp;
+    if (w >= w_end) return;
+    const M3sOffWork wk = work[w];
+    const M3sEncClip cl = clips[wk.clip];
+    const int f_end = min(cl.n_frames, chunk_first + chunk_frames);
+    if (f_end <= chunk_first) return;
+    const bool mine = lane < wk.count;
+    const int64_t ci = wk.cand_first + (mine ? lane : 0);
+    const M3sOffCand cd = cands[ci];
+    M3sEncState *sp = states + ci;
+    int64_t off = sp->hide_off;
+    uint32_t car_a[4];
+    int car_step[4];
+#pragma unroll
+    for (int s = 0; s < 4; s++) {
+        car_a[s] = (uint32_t)sp->a1[s] | (uint32_t)sp->a2[s] << 10 | (uint32_t)sp->a3[s] << 20;
+        car_step[s] = sp->step[s];
+    }
+    int32_t overrun = sp->overrun;
+    // the payload bits [wbase, wbase + 64) MSB first; a granule reads 3 bits at `off`, so the window moves every ~20 granules
+    const int64_t nbytes = cd.nbits >> 3;
+    uint64_t win = 0;
+    int64_t wbase = INT64_MIN / 2;
+    auto bits_at = [&](int64_t o, int &hn, uint32_t &hb) {   // hb bit j = payload bit o + j, as k_enc_resolve's payload window
+        const int64_t left = cd.nbits - o;
+        hn = left > 3 ? 3 : (left < 0 ? 0 : (int)left);
+        hb = 0u;
+        if (hn == 0) return;
+        if (o + 3 > wbase + 64) {
+            wbase = o & ~(int64_t)7;
+            win = 0;
+#pragma unroll 1
+            for (int b = 0; b < 8; b++) {
+                const int64_t k = (wbase >> 3) + b;
+                const uint32_t v = k >= nbytes ? 0u : (k < cd.head_len ? __ldg(head + cd.head_base + k) : __ldg(body + cd.body_base + k - cd.head_len));
+                win |= (uint64_t)v << (56 - 8 * b);
+            }
+        }
+        const int rel = (int)(o - wbase);
+        const uint32_t top = (uint32_t)(win >> (61 - rel)) & 7u;   // bits rel, rel + 1, rel + 2 as b0 b1 b2 (MSB first)
+        hb = (((top >> 2) & 1u) | (top & 2u) | ((top & 1u) << 2)) & ((1u << hn) - 1u);
+    };
+#pragma unroll 1
+    for (int f = chunk_first; f < f_end; f++) {
+        const int64_t fl_ = cl.frame_base + f;
+        const uint4 ws4 = *(const uint4 *)(sum + fl_ * 4);   // the frame's four summary words, the same for every lane
+#pragma unroll
+        for (int q = 0; q < 4; q++) {   // the reference's order (ch0,gr0) (ch0,gr1) (ch1,gr0) (ch1,gr1); slot = 2 gr + ch
+            const int slot = 2 * (q & 1) + (q >> 1);
+            const int64_t gs = fl_ * 4 + q;
+            const uint32_t ws = q == 0 ? ws4.x : (q == 1 ? ws4.y : (q == 2 ? ws4.z : ws4.w));
+            int hn;
+            uint32_t hb;
+            if (ws & VAR_SLOW) {
+                // the probe could not settle this granule (stale addresses, or the step table's end): the reference's search with each
+                // lane's true state, served one lane at a time by the whole warp
+                bits_at(off, hn, hb);
+                int padding, mean_bits;
+                const int max_bits = frame_max_bits(byteoff, cl, f, padding, mean_bits);
+                const int32_t xrmax = stats[gs].xrmax;
+                uint32_t new_a = car_a[slot];
+                int new_step = car_step[slot], cnt = 0;
+                bool over = false;
+                for (uint32_t pend = __ballot_sync(FULL, mine); pend; pend &= pend - 1) {
+                    const int src = __ffs(pend) - 1;
+                    const uint32_t sa = __shfl_sync(FULL, car_a[slot], src);
+                    int step = __shfl_sync(FULL, car_step[slot], src);
+                    const int lhn = __shfl_sync(FULL, hn, src);
+                    const uint32_t lhb = __shfl_sync(FULL, hb, src);
+                    int a1 = (int)(sa & 1023u), a2 = (int)((sa >> 10) & 1023u), a3 = (int)((sa >> 20) & 1023u), part23 = 0;
+                    GranInfo gi;
+                    const bool ok = search_granule(S, mdct + gs * 576, xrmax, max_bits, lhn, lhb, lane, a1, a2, a3, step, gi, part23);
+                    if (lane == src) {
+                        new_a = (uint32_t)a1 | (uint32_t)a2 << 10 | (uint32_t)a3 << 20;
+                        new_step = step;
+                        cnt = (gi.ts0 > 0) + (gi.ts1 > 0) + (gi.ts2 > 0);
+                        over = !ok;
+                    }
+                }
+                car_a[slot] = new_a;
+                car_step[slot] = new_step;
+                if (over && !overrun) overrun = f + 1;
+                off += cnt;
+            } else if (!(ws & VAR_SILENT)) {
+                bits_at(off, hn, hb);
+                const int v = variant_index(hn, hb);
+                off += (ws >> (2 * v)) & 3u;
+                const uint4 r = var[gs * 16 + v];   // k_enc_probe's record of the variant: .y = step + 128 | ... | have << 30, .z = addresses
+                car_step[slot] = (int)(r.y & 0xFFu) - 128;
+                if ((r.y >> 30) & 1u) car_a[slot] = r.z;
+            }
+        }
+    }
+    if (mine) {
+#pragma unroll
+        for (int s = 0; s < 4; s++) {
+            sp->a1[s] = (int32_t)(car_a[s] & 1023u); sp->a2[s] = (int32_t)((car_a[s] >> 10) & 1023u); sp->a3[s] = (int32_t)((car_a[s] >> 20) & 1023u);
+            sp->step[s] = car_step[s];
+        }
+        sp->hide_off = off;
+        sp->overrun = overrun;
+    }
+}
+
 // One warp per granule-channel: quantise at the chosen step and write the signed values format_bitstream codes (:1272-1276).
 // A silent granule keeps what l3_enc held for its slot (never coded: big_values = count1 = 0): the values of the latest
 // non-silent granule of the slot, re-derived from that granule's spectra, or read from `last_in` when it lies in an earlier chunk.
@@ -1586,18 +1724,28 @@ static void build_enc_tables(const M3sDevTables *T, EncTables *E)
     }
 }
 
+// The candidate payloads of m3s_encode_offsets (see the header).  With them the encoder runs in offsets mode: analysis and probe as
+// always, then k_enc_offsets instead of resolve, emit and pack; hide_str_offset_out is indexed by candidate.
+struct EncOffsets {
+    const uint8_t *body;
+    const int64_t *body_off, *cand_off;
+    const uint8_t *head;
+    const int64_t *head_off, *body_len;
+};
+
 static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
                        int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
                        const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                       int64_t *out_len, int64_t *hide_str_offset_out);
+                       int64_t *out_len, int64_t *hide_str_offset_out, const EncOffsets *ox);
 
-// both entry points run here: an early return may leave work of the call on the helper streams, drained before the caller reuses buffers
+// every entry point runs here: an early return may leave work of the call on the helper streams, drained before the caller reuses buffers
 static int encode_call(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples, int32_t n_clips,
                        const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits, const int64_t *payload_off,
-                       uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap, int64_t *out_len, int64_t *hide_str_offset_out)
+                       uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap, int64_t *out_len, int64_t *hide_str_offset_out,
+                       const EncOffsets *ox = nullptr)
 {
     const int rc = encode_impl(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out,
-                               mp3_off, mp3_cap, out_len, hide_str_offset_out);
+                               mp3_off, mp3_cap, out_len, hide_str_offset_out, ox);
     if (rc != M3S_OK && h) {
         cudaStreamSynchronize(h->stream);
         if (h->copy_in) { cudaStreamSynchronize(h->copy_in); cudaStreamSynchronize(h->copy_out); cudaStreamSynchronize(h->aux); }
@@ -1630,6 +1778,16 @@ extern "C" int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, con
                        mp3_cap, out_len, hide_str_offset_out);
 }
 
+extern "C" int m3s_encode_offsets(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                                  int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *body,
+                                  const int64_t *body_off, const int64_t *cand_off, const uint8_t *head, const int64_t *head_off,
+                                  const int64_t *body_len, int64_t *hide_str_offset_out)
+{
+    const EncOffsets ox{body, body_off, cand_off, head, head_off, body_len};
+    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, nullptr, nullptr, nullptr, nullptr, nullptr,
+                       nullptr, hide_str_offset_out, &ox);
+}
+
 static const bool g_enc_trace = getenv("M3S_TRACE") != nullptr;   // host-clock stage timing of the encode call (diagnostic)
 static double enc_now_ms()
 {
@@ -1639,17 +1797,36 @@ static double enc_now_ms()
 }
 #define M3S_ENC_MARK(tag) do { if (g_enc_trace) { const double t__ = enc_now_ms(); fprintf(stderr, "[m3s enc] %-22s +%.2f ms\n", tag, t__ - tr_t); tr_t = t__; } } while (0)
 
+// Offsets mode: the payload length k_enc_probe prunes the variants of caller clip j with (`sure3`).  It is the shortest hiding
+// candidate's: with a longer one the probe would skip end-of-payload variants that a shorter candidate meets.  An empty candidate
+// next to hiding ones needs variant 14 (no bits left) at every granule, which only a payload shorter than 3 bits keeps active.
+// 0 when no candidate hides.
+static int64_t offsets_probe_len(const EncOffsets &ox, int j)
+{
+    int64_t shortest = INT64_MAX;
+    bool empty = false;
+    for (int64_t c = ox.cand_off[j]; c < ox.cand_off[j + 1]; c++) {
+        const int64_t nbits = 8 * (ox.head_off[c + 1] - ox.head_off[c] + ox.body_len[c]);
+        if (nbits == 0) empty = true;
+        else shortest = std::min(shortest, nbits);
+    }
+    if (shortest == INT64_MAX) return 0;
+    return empty ? 1 : shortest;
+}
+
 static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
                        int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
                        const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                       int64_t *out_len, int64_t *hide_str_offset_out)
+                       int64_t *out_len, int64_t *hide_str_offset_out, const EncOffsets *ox)
 {
     if (!h) return M3S_ERR_ARG;
     double tr_t = g_enc_trace ? enc_now_ms() : 0.0;
     h->enc_taps_ok = false;
-    if (!pcm || !n_samples || n_clips <= 0 || !mp3_out || !mp3_off || !sample_rate || !bitrate_kbps)
+    if (!pcm || !n_samples || n_clips <= 0 || !sample_rate || !bitrate_kbps || (!ox && (!mp3_out || !mp3_off)) ||
+        (ox && (!ox->body_off || !ox->cand_off || !ox->head_off || !ox->body_len || !hide_str_offset_out)))
         return m3s_fail(h, M3S_ERR_ARG, "encode: null argument");
     if ((uintptr_t)pcm & 3) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm must be 4-byte aligned (one stereo sample per word)");
+    if (ox && ox->cand_off[0] != 0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: cand_off[0] is %lld, not 0", (long long)ox->cand_off[0]);
     // ---- per-clip checks, in the caller's order, before anything is queued
     for (int j = 0; j < n_clips; j++) {
         if (sr_index_of(sample_rate[j]) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: sample rate %d is not an MPEG-1 rate", j, sample_rate[j]);
@@ -1657,6 +1834,19 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", j, bitrate_kbps[j]);
         if (n_samples[j] < 0 || n_samples[j] % 1152) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d has %lld samples per channel, not a multiple of 1152 (the reference raises IndexError, MP3_Encoder.py:611-614)", j, (long long)n_samples[j]);
         if (pcm_off && (pcm_off[j] & 1)) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm_off must be even (stereo samples)");
+        if (!ox) continue;
+        const int64_t c0 = ox->cand_off[j], c1 = ox->cand_off[j + 1], b0 = ox->body_off[j], b1 = ox->body_off[j + 1];
+        if (c1 < c0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: cand_off decreases (%lld -> %lld)", j, (long long)c0, (long long)c1);
+        if (b0 < 0 || b1 < b0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: bad body range [%lld, %lld)", j, (long long)b0, (long long)b1);
+        if (b1 > b0 && !ox->body) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: body is NULL", j);
+        for (int64_t c = c0; c < c1; c++) {
+            const int64_t h0 = ox->head_off[c], h1 = ox->head_off[c + 1], bl = ox->body_len[c];
+            if (h0 < 0 || h1 < h0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: bad head range [%lld, %lld)", j, (long long)c, (long long)h0, (long long)h1);
+            if (h1 - h0 > 32) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head of %lld bytes, more than 32", j, (long long)c, (long long)(h1 - h0));
+            if (h1 > h0 && !ox->head) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head is NULL", j, (long long)c);
+            if (bl < 0 || bl > b1 - b0)
+                return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: body_len %lld outside the clip's body of %lld bytes", j, (long long)c, (long long)bl, (long long)(b1 - b0));
+        }
     }
     M3S_CUDA(h, cudaSetDevice(h->device));
     int rc;
@@ -1681,9 +1871,9 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         c.pcm_base = pcm_off ? pcm_off[j] : 0;
         c.n_frames = (int32_t)(n_samples[j] / 1152);
         c.frame_base = total_frames;
-        c.out_base = mp3_off[j];
+        c.out_base = ox ? 0 : mp3_off[j];
         c.payload_base = payload_bits && payload_off ? payload_off[j] : 0;
-        c.payload_len = payload_bits && payload_off ? payload_off[j + 1] - payload_off[j] : 0;
+        c.payload_len = ox ? offsets_probe_len(*ox, j) : (payload_bits && payload_off ? payload_off[j + 1] - payload_off[j] : 0);
         c.sr_idx = (int16_t)sr_index_of(sample_rate[j]);
         c.bitrate_idx = (int16_t)br_index_of(bitrate_kbps[j]);
         total_frames += c.n_frames;
@@ -1715,13 +1905,15 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         c.out_len = (int64_t)(byteoff[(size_t)c.pad_base + c.n_frames] / 4) * 4;
         out_total = std::max(out_total, c.out_base + c.out_len);
     }
+    const int64_t n_cand = ox ? ox->cand_off[n_clips] : 0;
     for (int j = 0; j < n_clips; j++) {
         const M3sEncClip &c = clips[inv[j]];
         if (mp3_cap && mp3_cap[j] < c.out_len) return m3s_fail(h, M3S_ERR_CAPACITY, "encode: clip %d needs %lld output bytes, capacity %lld", j, (long long)c.out_len, (long long)mp3_cap[j]);
         if (out_len) out_len[j] = c.out_len;
-        if (hide_str_offset_out) hide_str_offset_out[j] = 0;
+        if (hide_str_offset_out && !ox) hide_str_offset_out[j] = 0;
     }
-    if (total_frames == 0) return M3S_OK;
+    for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = 0;
+    if (total_frames == 0 || (ox && n_cand == 0)) return M3S_OK;
     M3S_ENC_MARK("clip table");
     // ---- encoder constant tables (once per handle)
     if (!h->e_tabs.p) {
@@ -1741,18 +1933,63 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     const int16_t *d_pcm = pcm;
     uint8_t *d_out = mp3_out;
     if ((rc = m3s_pipeline_init(h))) return rc;
-    if (host) {
+    if (host && !ox) {
         if ((rc = m3s_buf_reserve(h, h->e_out, (size_t)out_total + 16))) return rc;
         d_out = (uint8_t *)h->e_out.p;
     }
-    if ((rc = m3s_buf_reserve(h, h->e_payload, (size_t)pay_total + 16))) return rc;
-    if (pay_total > 0) M3S_CUDA(h, cudaMemcpyAsync(h->e_payload.p, payload_bits, (size_t)pay_total, cudaMemcpyHostToDevice, h->stream));
+    // offsets mode: the candidates, k_enc_offsets' work items (32 candidates of one clip each, in the library's clip order, so that
+    // the items of one sample rate are [ogrp[s], ogrp[s + 1])), the heads and the bodies, in one buffer
+    std::vector<M3sOffCand> cands;
+    std::vector<M3sOffWork> owork;
+    int ogrp[4] = {0, 0, 0, 0};
+    const M3sOffCand *d_cands = nullptr;
+    const M3sOffWork *d_owork = nullptr;
+    const uint8_t *d_head = nullptr, *d_body = nullptr;
+    if (ox) {
+        cands.resize((size_t)n_cand);
+        int64_t body_total = 0;
+        for (int i = 0; i < n_clips; i++) {
+            const int j = order[i];
+            for (int s = 0; s < 4; s++)
+                if (grp[s] == i) ogrp[s] = (int)owork.size();
+            body_total = std::max(body_total, ox->body_off[j + 1]);
+            for (int64_t c = ox->cand_off[j]; c < ox->cand_off[j + 1]; c++) {
+                M3sOffCand &d = cands[(size_t)c];
+                d.head_base = (int32_t)ox->head_off[c];
+                d.head_len = (int32_t)(ox->head_off[c + 1] - ox->head_off[c]);
+                d.body_base = ox->body_off[j];
+                d.nbits = 8 * (d.head_len + ox->body_len[c]);
+                if ((c - ox->cand_off[j]) % 32 == 0) owork.push_back(M3sOffWork{i, (int32_t)std::min<int64_t>(32, ox->cand_off[j + 1] - c), c});
+            }
+        }
+        for (int s = 0; s < 4; s++)
+            if (grp[s] == n_clips) ogrp[s] = (int)owork.size();
+        const int64_t head_total = ox->head_off[n_cand];
+        if (head_total > INT32_MAX || owork.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: too many candidates in one call");
+        auto al16 = [](size_t b) { return (b + 15) / 16 * 16; };
+        const size_t o_work = al16(sizeof(M3sOffCand) * cands.size()), o_head = o_work + al16(sizeof(M3sOffWork) * owork.size());
+        const size_t o_body = o_head + al16((size_t)head_total);
+        if ((rc = m3s_buf_reserve(h, h->e_cand, o_body + (size_t)body_total + 16))) return rc;
+        char *base = (char *)h->e_cand.p;
+        M3S_CUDA(h, cudaMemcpyAsync(base, cands.data(), sizeof(M3sOffCand) * cands.size(), cudaMemcpyHostToDevice, h->stream));
+        M3S_CUDA(h, cudaMemcpyAsync(base + o_work, owork.data(), sizeof(M3sOffWork) * owork.size(), cudaMemcpyHostToDevice, h->stream));
+        if (head_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_head, ox->head, (size_t)head_total, cudaMemcpyHostToDevice, h->stream));
+        if (body_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_body, ox->body, (size_t)body_total, cudaMemcpyHostToDevice, h->stream));
+        d_cands = (const M3sOffCand *)base;
+        d_owork = (const M3sOffWork *)(base + o_work);
+        d_head = (const uint8_t *)(base + o_head);
+        d_body = (const uint8_t *)(base + o_body);
+    } else {
+        if ((rc = m3s_buf_reserve(h, h->e_payload, (size_t)pay_total + 16))) return rc;
+        if (pay_total > 0) M3S_CUDA(h, cudaMemcpyAsync(h->e_payload.p, payload_bits, (size_t)pay_total, cudaMemcpyHostToDevice, h->stream));
+    }
     if ((rc = m3s_buf_reserve(h, h->e_pad, sizeof(uint32_t) * byteoff.size()))) return rc;
     M3S_CUDA(h, cudaMemcpyAsync(h->e_pad.p, byteoff.data(), sizeof(uint32_t) * byteoff.size(), cudaMemcpyHostToDevice, h->stream));
-    if ((rc = m3s_buf_reserve(h, h->e_state, sizeof(M3sEncState) * n_clips))) return rc;
-    M3S_CUDA(h, cudaMemsetAsync(h->e_state.p, 0, sizeof(M3sEncState) * n_clips, h->stream));
+    const int64_t n_states = ox ? n_cand : n_clips;   // the carried state is per candidate in offsets mode
+    if ((rc = m3s_buf_reserve(h, h->e_state, sizeof(M3sEncState) * n_states))) return rc;
+    M3S_CUDA(h, cudaMemsetAsync(h->e_state.p, 0, sizeof(M3sEncState) * n_states, h->stream));
     const size_t lastix_bytes = (size_t)n_clips * 4 * 288 * 4;
-    if ((rc = m3s_buf_reserve(h, h->e_lastix, 2 * lastix_bytes))) return rc;   // two sets: chunk k reads set k & 1 and writes the other
+    if (!ox && (rc = m3s_buf_reserve(h, h->e_lastix, 2 * lastix_bytes))) return rc;   // two sets: chunk k reads set k & 1 and writes the other
 
     // ---- chunking: all clips advance together through windows of `cf` frames so that the intermediates
     //      (MDCT spectra 9.2 KB/frame, quantised values 4.6 KB/frame) stay bounded while every clip keeps its warp busy
@@ -1771,8 +2008,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     for (int q = 0; q < nset; q++) {
         if ((rc = m3s_buf_reserve(h, *b_mdct[q], (size_t)chunk_cap * 4 * 576 * 4))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_gran[q], (size_t)chunk_cap * 4 * sizeof(M3sEncStats)))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_ix[q], (size_t)chunk_cap * 4 * 288 * 4))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_info[q], (size_t)chunk_cap * 4 * ENC_INFO_FIELDS * 4))) return rc;
+        if (!ox && (rc = m3s_buf_reserve(h, *b_ix[q], (size_t)chunk_cap * 4 * 288 * 4))) return rc;
+        if (!ox && (rc = m3s_buf_reserve(h, *b_info[q], (size_t)chunk_cap * 4 * ENC_INFO_FIELDS * 4))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_scfsi[q], (size_t)chunk_cap * 8))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_var[q], (size_t)chunk_cap * 4 * 16 * sizeof(uint4)))) return rc;
         if ((rc = m3s_buf_reserve(h, *b_sum[q], (size_t)chunk_cap * 4 * sizeof(uint32_t)))) return rc;
@@ -1786,6 +2023,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis_fold, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     const int64_t ana_run = Ana3Smem::RUN;   // granules per analysis work item
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PackSmem)));
+    if (ox) M3S_CUDA(h, cudaFuncSetAttribute(k_enc_offsets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
     auto frames_in_chunk = [&](int i, int64_t c0) { return std::max<int64_t>(0, std::min<int64_t>(cf, clips[i].n_frames - c0)); };
     // host staging: per chunk every clip owns a region of cf * 1152 + 1056 stereo samples (1056 = the analysis history the
     // first granule of the chunk reaches back to: 480 window taps + one warm-up granule), two region sets for double buffering
@@ -1936,29 +2174,41 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         if (g_enc_trace) tmark(tev[k].r1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_rate[pb], h->stream));
         if (host && k + 2 < n_chunks) M3S_CUDA(h, stage_chunk(k + 2));
-        for (int s = 0; s < 3; s++) {
-            if (gsl[s + 1] == gsl[s]) continue;   // no clip of this sample rate has a frame in the chunk
-            M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
-            k_enc_resolve<<<(unsigned)((grp[s + 1] - grp[s] + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
-                d_clips, grp[s], grp[s + 1], (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-                (const uint8_t *)h->e_payload.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
-                (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
+        if (ox) {   // offsets mode: every candidate's offset chain instead of resolve, emit and pack
+            for (int s = 0; s < 3; s++) {
+                if (gsl[s + 1] == gsl[s] || ogrp[s + 1] == ogrp[s]) continue;
+                M3S_KBEGIN(h, M3S_K_ENC_OFFSETS);
+                k_enc_offsets<<<(unsigned)((ogrp[s + 1] - ogrp[s] + OFFSETS_WARPS - 1) / OFFSETS_WARPS), 32 * OFFSETS_WARPS, sizeof(RateSmem), h->stream>>>(
+                    d_clips, d_owork, ogrp[s], ogrp[s + 1], d_cands, d_head, d_body, (M3sEncState *)h->e_state.p, h->d_tab,
+                    (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
+                    (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (const uint32_t *)b_sum[pb]->p);
+                M3S_LAUNCH_CHECK(h);
+            }
+        } else {
+            for (int s = 0; s < 3; s++) {
+                if (gsl[s + 1] == gsl[s]) continue;   // no clip of this sample rate has a frame in the chunk
+                M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
+                k_enc_resolve<<<(unsigned)((grp[s + 1] - grp[s] + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
+                    d_clips, grp[s], grp[s + 1], (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+                    (const uint8_t *)h->e_payload.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
+                    (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
+                M3S_LAUNCH_CHECK(h);
+            }
+            M3S_KBEGIN(h, M3S_K_ENC_AUX);
+            k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
+                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (int32_t)c0, (int32_t)cf,
+                n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
+                (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
+                (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
+                (uint32_t *)((char *)h->e_lastix.p + (size_t)((k + 1) & 1) * lastix_bytes));
+            M3S_LAUNCH_CHECK(h);
+            // packing stays on the rate loop's stream
+            M3S_KBEGIN(h, M3S_K_ENC_PACK);
+            k_enc_pack<<<(unsigned)((chunk_total + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
+                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const uint32_t *)h->e_pad.p, 0, chunk_total,
+                (const uint32_t *)b_ix[pb]->p, (const int32_t *)b_info[pb]->p, (const uint8_t *)b_scfsi[pb]->p, d_out);
             M3S_LAUNCH_CHECK(h);
         }
-        M3S_KBEGIN(h, M3S_K_ENC_AUX);
-        k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
-            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (int32_t)c0, (int32_t)cf,
-            n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
-            (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
-            (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
-            (uint32_t *)((char *)h->e_lastix.p + (size_t)((k + 1) & 1) * lastix_bytes));
-        M3S_LAUNCH_CHECK(h);
-        // packing stays on the rate loop's stream
-        M3S_KBEGIN(h, M3S_K_ENC_PACK);
-        k_enc_pack<<<(unsigned)((chunk_total + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
-            d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const uint32_t *)h->e_pad.p, 0, chunk_total,
-            (const uint32_t *)b_ix[pb]->p, (const int32_t *)b_info[pb]->p, (const uint8_t *)b_scfsi[pb]->p, d_out);
-        M3S_LAUNCH_CHECK(h);
         if (g_enc_trace) tmark(tev[k].p1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_pack[pb], h->stream));
         // the rate loop and the analysis are both issue-bound: the next chunk's analysis waits for this chunk's packing (measured:
@@ -1967,7 +2217,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_pack[pb], 0));
             if ((rc = launch_analysis(k + 1))) return rc;
         }
-        if (host) {   // this chunk's bytes of every clip go home behind the pack kernel
+        if (host && !ox) {   // this chunk's bytes of every clip go home behind the pack kernel
             M3S_CUDA(h, cudaStreamWaitEvent(h->copy_out, h->ev_pack[pb], 0));
             rows.clear();
             for (int i = 0; i < n_clips; i++) {
@@ -2001,6 +2251,19 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         }
         for (int64_t k = 0; k < n_chunks; k++)
             for (cudaEvent_t e : {tev[k].c0, tev[k].c1, tev[k].a0, tev[k].a1, tev[k].r1, tev[k].p1, tev[k].o1}) if (e) cudaEventDestroy(e);
+    }
+    if (ox) {   // ---- offsets mode: results by the caller's candidate index
+        std::vector<M3sEncState> states((size_t)n_cand);
+        M3S_CUDA(h, cudaMemcpyAsync(states.data(), h->e_state.p, sizeof(M3sEncState) * n_cand, cudaMemcpyDeviceToHost, h->stream));
+        M3S_CUDA(h, cudaStreamSynchronize(h->stream));
+        for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = states[(size_t)c].hide_off;
+        for (int j = 0; j < n_clips; j++)
+            for (int64_t c = ox->cand_off[j]; c < ox->cand_off[j + 1]; c++)
+                if (states[(size_t)c].overrun)
+                    return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld frame %d: the step search runs past the end of the step "
+                                    "table (quantize would read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)",
+                                    j, (long long)c, states[(size_t)c].overrun - 1);
+        return M3S_OK;
     }
     // ---- results, by the caller's clip index
     std::vector<M3sEncState> states(n_clips);

@@ -63,6 +63,9 @@ SYMBOLS = [
     ("m3s_encode_mixed", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, _c_i64p, _c_i64p, ctypes.c_int32,
                                         _c_i32p, _c_i32p, ctypes.c_void_p, _c_i64p, ctypes.c_void_p, _c_i64p,
                                         _c_i64p, _c_i64p, _c_i64p]),
+    ("m3s_encode_offsets", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, _c_i64p, _c_i64p, ctypes.c_int32,
+                                          _c_i32p, _c_i32p, ctypes.c_void_p, _c_i64p, _c_i64p, ctypes.c_void_p, _c_i64p, _c_i64p,
+                                          _c_i64p]),
     ("m3s_encode_taps", ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                        ctypes.c_void_p]),
     ("m3s_table_export", ctypes.c_int64, [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64]),
@@ -70,7 +73,7 @@ SYMBOLS = [
     ("m3s_timing_get", ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_double), _c_i64p]),
     ("m3s_kernel_name", ctypes.c_char_p, [ctypes.c_int]),
 ]
-M3S_K_COUNT = 12
+M3S_K_COUNT = 13
 
 _lib = None
 
@@ -392,6 +395,41 @@ class Handle:
             self._check(L.m3s_encode_taps(self._h, _ptr(res["mdct"]), _ptr(res["ix"]), _ptr(res["info"]), _ptr(res["scfsi"])),
                         "m3s_encode_taps")
         return res
+
+    def encode_offsets(self, pcm, n_samples, sample_rate, bitrate_kbps, bodies, candidates, pcm_off=None):
+        """m3s_encode_offsets: hide_str_offset of many candidate payloads per clip, from one analysis + probe pass per clip and
+        without writing MP3 bytes.  `pcm`, `n_samples`, `pcm_off` as encode(); sample_rate and bitrate_kbps are ints or one entry
+        per clip.  bodies[i] is the bytes of clip i; candidates[i] is a list of (head: bytes, body_len: int), each hiding the
+        MSB-first bits of head + bodies[i][:body_len].  Returns one int64 array of offsets per clip, in candidate order.
+        Raises IndexError, for the whole call, when a candidate drives the rate loop past the end of the step table."""
+        L = self._L
+        n = len(n_samples)
+        if len(bodies) != n or len(candidates) != n:
+            raise ValueError("encode_offsets: one body and one candidate list per clip")
+        ns, ns_p = _i64(n_samples)
+        if pcm_off is None:
+            pcm_off = np.concatenate([[0], np.cumsum(ns * 2)])[:-1]
+        po, po_p = _i64(pcm_off)
+        srs = np.ascontiguousarray(np.broadcast_to(np.asarray(sample_rate, np.int32), (n,)))
+        brs = np.ascontiguousarray(np.broadcast_to(np.asarray(bitrate_kbps, np.int32), (n,)))
+        body = np.frombuffer(b"".join(bodies) + b"\0", np.uint8)
+        bo, bo_p = _i64(np.concatenate([[0], np.cumsum([len(b) for b in bodies])]))
+        co, co_p = _i64(np.concatenate([[0], np.cumsum([len(c) for c in candidates])]))
+        heads = [hd for cs in candidates for hd, _ in cs]
+        head = np.frombuffer(b"".join(heads) + b"\0", np.uint8)
+        ho, ho_p = _i64(np.concatenate([[0], np.cumsum([len(hd) for hd in heads])]))
+        bl, bl_p = _i64([b for cs in candidates for _, b in cs] or [0])
+        out = np.zeros(max(int(co[-1]), 1), np.int64)
+        _ready(pcm)
+        rc = L.m3s_encode_offsets(self._h, _ptr(pcm), _mem_of(pcm), po_p, ns_p, n, srs.ctypes.data_as(_c_i32p),
+                                  brs.ctypes.data_as(_c_i32p), _ptr(body), bo_p, co_p, _ptr(head), ho_p, bl_p,
+                                  out.ctypes.data_as(_c_i64p))
+        if rc == M3S_ERR_ARG:
+            msg = L.m3s_last_error(self._h).decode()
+            if STEP_TABLE_OVERRUN in msg:
+                raise IndexError(f"index out of bounds: {msg}")
+        self._check(rc, "m3s_encode_offsets")
+        return [out[co[i]:co[i + 1]].copy() for i in range(n)]
 
 
 _default = {}

@@ -7,6 +7,9 @@ call and without leaving the GPU between the decode and the encode half of the c
                  for sample) -> encode + hide at each file's own sample rate and bitrate, all files in one encode call; the PCM
                  stays in HBM
   clear_batch    clear_file: the same with no payload
+  capacity_batch   the longest prefix of each message that hide_message would hide whole (every prefix resolved in ONE
+                   m3s_encode_offsets call against one analysis + probe pass per file)
+  hide_batch_fit   hide_batch of those prefixes, from the same decode
 The semantics per file are the facade's: message framing '<len>#<message>' as utf-8 bits (steganography.py:10-24,88-90),
 bitrate of the last frame (MP3_Parser.py:93-97), too_long = hide_str_offset < len(bits) - 1 (encoder.py:49-51),
 ID3v2 skip (decoder.py:29-33).  torch is used for the device buffers only."""
@@ -53,12 +56,10 @@ def _pinned(handle, name: str, nbytes: int):
     return buf
 
 
-def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[int]]:
-    """decode (exact) -> encode for N files, bytes in -> bytes out.  The host side moves every byte exactly twice: the files are
-    gathered straight into a pinned buffer (one pass) that crosses PCIe in one asynchronous copy, and the MP3s come back into a
-    pinned buffer from which the per-file `bytes` are cut (one pass); everything in between stays in HBM."""
+def _marker():
+    """mark(tag): host wall clock of the batch stages on stderr when M3S_TRACE is set (diagnostic)."""
     import torch
-    trace = os.environ.get("M3S_TRACE") is not None   # host wall clock of the stages (diagnostic)
+    trace = os.environ.get("M3S_TRACE") is not None
     t_last = [time.perf_counter()]
 
     def mark(tag):
@@ -67,6 +68,15 @@ def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[in
             t = time.perf_counter()
             print("[m3s batch] %-14s +%.1f ms" % (tag, 1e3 * (t - t_last[0])), file=sys.stderr)
             t_last[0] = t
+    return mark
+
+
+def _decode_exact(handle, blobs, mark):
+    """The decode half of the composites: N files -> int16 PCM in HBM (float64 instantiation, so that it equals the reference's
+    WAV sample for sample).  The files are gathered straight into a pinned buffer that crosses PCIe in one asynchronous copy.
+    Returns dict(pcm, rows, pcm_off, sample_rate, kbps): what the encode calls take, every file at its own sample rate and
+    last-frame bitrate."""
+    import torch
     n = len(blobs)
     sizes = np.fromiter((len(b) for b in blobs), np.int64, n)
     off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
@@ -102,11 +112,17 @@ def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[in
             raise ValueError(f"file {i}: not an MPEG-1 Layer III stream the reference can decode")
         if nchan[i] != 2:
             raise IndexError(f"file {i}: the reference encoder only handles stereo input (WAV_Reader / MP3_Encoder.py:611-614)")
-    rows = sc["pcm_rows"].astype(np.int64)
-    pcm_off = sc["pcm_off"]
-    kbps = sc["bitrate"].astype(np.int64) // 1000
-    # one encode call for the whole batch, every file at its own sample rate and last-frame bitrate
-    res = handle.encode(pcm, rows, sc["sample_rate"], kbps, payloads=list(payloads), pcm_off=pcm_off[:n], compact=True)
+    return dict(pcm=pcm, rows=sc["pcm_rows"].astype(np.int64), pcm_off=sc["pcm_off"][:n], sample_rate=sc["sample_rate"],
+                kbps=sc["bitrate"].astype(np.int64) // 1000)
+
+
+def _encode_cut(handle, dec, payloads, mark) -> Tuple[List[bytes], List[int], List[int]]:
+    """The encode half: one encode call for the whole batch, then the MP3s come back into a pinned buffer from which the per-file
+    `bytes` are cut (one pass)."""
+    import torch
+    dev = torch.device("cuda", handle.device)
+    kbps = dec["kbps"]
+    res = handle.encode(dec["pcm"], dec["rows"], dec["sample_rate"], kbps, payloads=list(payloads), pcm_off=dec["pcm_off"], compact=True)
     mark("encode")
     nbytes = int(res["mp3_off"][-1] + res["out_len"][-1])
     back = _pinned(handle, "out", nbytes)
@@ -120,6 +136,13 @@ def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[in
     return out, hoff, kbps.tolist()
 
 
+def _transcode(handle, blobs, payloads) -> Tuple[List[bytes], List[int], List[int]]:
+    """decode (exact) -> encode for N files, bytes in -> bytes out.  The host side moves every byte exactly twice (gather, cut);
+    everything in between stays in HBM."""
+    mark = _marker()
+    return _encode_cut(handle, _decode_exact(handle, blobs, mark), payloads, mark)
+
+
 def hide_batch(handle: "_lib.Handle", blobs: Sequence[bytes], messages: Sequence[str]) -> Tuple[List[bytes], List[bool]]:
     """hide_message for N (mp3 bytes, message) pairs -> (new mp3 bytes, too_long flags)."""
     if len(blobs) != len(messages):
@@ -129,6 +152,65 @@ def hide_batch(handle: "_lib.Handle", blobs: Sequence[bytes], messages: Sequence
     bits = [str_to_binary_str(str(len(m)) + "#" + m) for m in messages]
     out, hoff, _ = _transcode(handle, blobs, bits)
     return out, [hoff[i] < len(bits[i]) - 1 for i in range(len(blobs))]
+
+
+def capacity_candidates(message: str, max_bits: int = None) -> Tuple[bytes, List[Tuple[bytes, int]]]:
+    """The candidates of one message for m3s_encode_offsets: the body is the message's utf-8 bytes, and candidate n (n = 0 ..
+    len(message)) is (head f"{n}#", the utf-8 length of message[:n]), whose bits are str_to_binary_str(f"{n}#{message[:n]}"), the
+    framing hide_message gives message[:n].  The framed length grows with n, so the list stops before the first prefix of more
+    than max_bits bits (None: no limit); candidate n is the list's entry n.  Returns (body, [(head, body_len), ...])."""
+    body = message.encode("utf-8")
+    ends = np.cumsum([0] + [len(ch.encode("utf-8")) for ch in message]).tolist()
+    cands = []
+    for n, bl in enumerate(ends):
+        head = b"%d#" % n
+        if max_bits is not None and 8 * (len(head) + bl) > max_bits:
+            break
+        cands.append((head, bl))
+    return body, cands
+
+
+def _capacity(handle, dec, messages) -> List[int]:
+    # hide_str_offset is at most 3 per granule of a channel (the three regions' tables) and a payload fits when the offset reaches
+    # its length - 1: a longer candidate cannot fit and is not evaluated
+    limits = [12 * (int(r) // 1152) + 1 for r in dec["rows"]]
+    bodies, cands = zip(*[capacity_candidates(m, lim) for m, lim in zip(messages, limits)])
+    offs = handle.encode_offsets(dec["pcm"], dec["rows"], dec["sample_rate"], dec["kbps"], list(bodies), list(cands),
+                                 pcm_off=dec["pcm_off"])
+    best = []
+    for cs, off in zip(cands, offs):
+        fit = [n for n, ((head, bl), o) in enumerate(zip(cs, off.tolist())) if o >= 8 * (len(head) + bl) - 1]
+        best.append(max(fit) if fit else -1)
+    return best
+
+
+def capacity_batch(handle: "_lib.Handle", blobs: Sequence[bytes], messages: Sequence[str]) -> List[int]:
+    """For each file the largest n in [0, len(message)] for which hide_message(file, message[:n]) would not report too_long, i.e.
+    its hide_str_offset reaches len(bits) - 1 under the framing f"{n}#{message[:n]}"; -1 when not even "0#" fits.  Every n is
+    evaluated, so the answer is exact where fitting is not monotone in n (the stego swap steers quantisation).  One exact decode
+    and one m3s_encode_offsets call for the batch."""
+    if len(blobs) != len(messages):
+        raise ValueError("one message per file")
+    if not blobs:
+        return []
+    return _capacity(handle, _decode_exact(handle, blobs, _marker()), messages)
+
+
+def hide_batch_fit(handle: "_lib.Handle", blobs: Sequence[bytes], messages: Sequence[str]) -> Tuple[List[bytes], List[int]]:
+    """hide_batch of message[:n*] for each file, n* = capacity_batch(...): the longest prefix that is hidden whole.  Where n* is -1
+    the file gets hide_batch's output for the empty message.  The files are decoded once; the PCM feeds both the offsets call and
+    the encode.  Returns (new mp3 bytes, n*)."""
+    if len(blobs) != len(messages):
+        raise ValueError("one message per file")
+    if not blobs:
+        return [], []
+    mark = _marker()
+    dec = _decode_exact(handle, blobs, mark)
+    best = _capacity(handle, dec, messages)
+    mark("offsets")
+    fit = [m[:max(n, 0)] for m, n in zip(messages, best)]
+    out, _, _ = _encode_cut(handle, dec, [str_to_binary_str(str(len(m)) + "#" + m) for m in fit], mark)
+    return out, best
 
 
 def clear_batch(handle: "_lib.Handle", blobs: Sequence[bytes]) -> List[bytes]:
