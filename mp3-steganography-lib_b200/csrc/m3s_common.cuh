@@ -188,17 +188,23 @@ struct M3sScanSet {
     size_t pin_cap = 0;
 };
 
+// One encode chunk's intermediates: MDCT spectra, granule statistics, quantised values, side info, scfsi, and the per-granule
+// variant records / summaries of the parallel rate loop (k_enc_probe -> k_enc_resolve).
+struct M3sEncSet {
+    M3sBuf mdct, gran, ix, info, scfsi, var, sum;
+};
+
 struct m3s_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t own_stream = nullptr;
     // copy streams + events of the host-buffer pipelines (created on first use): PCIe transfers of chunk k+1 / k-1 overlap the kernels of chunk k
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
-    cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr}, ev_done = nullptr;
+    cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     cudaEvent_t ev_pace[3] = {nullptr, nullptr, nullptr};   // m3s_copy_paced
     // encoder: the analysis of chunk k+1 runs on `aux` next to the rate loop of chunk k (ev_ana[buf] = its spectra are ready)
     cudaStream_t aux = nullptr, launch_stream = nullptr;   // launch_stream: where the kernel being timed is launched (NULL = stream)
-    cudaEvent_t ev_ana[2] = {nullptr, nullptr}, ev_rate[2] = {nullptr, nullptr}, ev_pack[2] = {nullptr, nullptr};
+    cudaEvent_t ev_ana[2] = {nullptr, nullptr}, ev_pack[2] = {nullptr, nullptr};
     std::string err;
     int64_t launches = 0;
     // ---- optional per-kernel device timing (m3s_timing_enable): cudaEvent pairs on the launching stream
@@ -228,15 +234,13 @@ struct m3s_ctx {
                 ev_d_out[2] = {nullptr, nullptr};
     uint8_t *rev_mapped = nullptr, *rev_dev = nullptr;   // m3s_decode_reveal to host memory: mapped pinned staging filled by a copy KERNEL
     size_t rev_cap = 0;
-    // ---- encode state
-    M3sBuf e_clips2, e_mdct2, e_gran2, e_ix2, e_info2, e_scfsi2;   // second set of the buffers the analysis writes ahead
-    M3sBuf e_var, e_var2, e_sum, e_sum2;   // per-granule variant records / summaries of the parallel rate loop (k_enc_probe -> k_enc_resolve)
+    // ---- encode state.  The per-chunk intermediates exist twice: chunk k uses set k & 1, so that the analysis writes ahead.
+    M3sEncSet es[2];
     M3sBuf e_cand;   // m3s_encode_offsets: candidate records, work items, heads and bodies
-    M3sBuf e_pcm, e_clips, e_mdct, e_ix, e_info, e_gran, e_out, e_payload, e_misc, e_pad, e_tabs, e_state, e_lastix, e_scfsi, e_work;
+    M3sBuf e_pcm, e_clips, e_out, e_payload, e_misc, e_pad, e_tabs, e_state, e_lastix, e_work;
     bool enc_taps_ok = false;
     int64_t enc_chunk_budget = 0;   // frames of intermediates kept per chunk (0 = default; M3S_ENC_CHUNK_FRAMES overrides)
     int64_t enc_total_frames = 0;
-    int32_t enc_n_clips = 0;
     std::vector<int64_t> enc_tap_runs;   // last encode: (device frame, caller frame, frames) triples, the taps' way back to the caller's clip order
 };
 
@@ -245,6 +249,10 @@ void m3s_time_begin(m3s_ctx *h, int id);
 void m3s_time_end(m3s_ctx *h);
 int m3s_buf_reserve(m3s_ctx *h, M3sBuf &b, size_t bytes);
 int m3s_pipeline_init(m3s_ctx *h);   // creates copy_in / copy_out and their events
+int m3s_sync_streams(m3s_ctx *h);    // waits for the main stream and, once created, copy_in / copy_out / aux
+// M3S_TRACE set: host-clock stage marks and per-chunk / per-wave device timelines of the pipelined calls on stderr (diagnostic)
+extern const bool m3s_trace;
+double m3s_now_ms();
 // a batch of (dst, src, bytes) row copies on one stream: one cudaMemcpy2DAsync when the rows are equally long and equally spaced
 struct M3sRow { char *dst; const char *src; size_t bytes; };
 // blocking-call flavour: at most two pieces are queued at a time, so copies of OTHER handles (whose host threads wait on them)

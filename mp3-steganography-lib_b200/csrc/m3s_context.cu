@@ -4,6 +4,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <chrono>
+
 #include "m3s_common.cuh"
 #include "m3s_tables_data.h"
 
@@ -18,16 +20,28 @@ int m3s_fail(m3s_ctx *h, int code, const char *fmt, ...)
     return code;
 }
 
+const bool m3s_trace = getenv("M3S_TRACE") != nullptr;
+
+double m3s_now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+int m3s_sync_streams(m3s_ctx *h)
+{
+    M3S_CUDA(h, cudaStreamSynchronize(h->stream));
+    if (h->copy_in) {
+        M3S_CUDA(h, cudaStreamSynchronize(h->copy_in));
+        M3S_CUDA(h, cudaStreamSynchronize(h->copy_out));
+        M3S_CUDA(h, cudaStreamSynchronize(h->aux));
+    }
+    return M3S_OK;
+}
+
 int m3s_buf_reserve(m3s_ctx *h, M3sBuf &b, size_t bytes)
 {
     if (bytes <= b.cap) return M3S_OK;
     if (b.p) {
-        M3S_CUDA(h, cudaStreamSynchronize(h->stream));
-        if (h->copy_in) {   // the helper streams of the pipelines may still reference the buffer (e.g. after an early error return)
-            M3S_CUDA(h, cudaStreamSynchronize(h->copy_in));
-            M3S_CUDA(h, cudaStreamSynchronize(h->copy_out));
-            M3S_CUDA(h, cudaStreamSynchronize(h->aux));
-        }
+        // the helper streams of the pipelines may still reference the buffer (e.g. after an early error return)
+        const int rc = m3s_sync_streams(h);
+        if (rc) return rc;
         M3S_CUDA(h, cudaFree(b.p));
         b.p = nullptr;
         b.cap = 0;
@@ -303,14 +317,12 @@ int m3s_pipeline_init(m3s_ctx *h)
     M3S_CUDA(h, cudaStreamCreateWithFlags(&h->aux, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
         M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_ana[i], cudaEventDisableTiming));
-        M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_rate[i], cudaEventDisableTiming));
         M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_pack[i], cudaEventDisableTiming));
     }
     for (int i = 0; i < 2; i++) {
         M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_in[i], cudaEventDisableTiming));
         M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_free[i], cudaEventDisableTiming));
     }
-    M3S_CUDA(h, cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
     return M3S_OK;
 }
 
@@ -385,15 +397,14 @@ extern "C" int m3s_destroy(m3s_handle_t h)
 {
     if (!h) return M3S_ERR_ARG;
     cudaSetDevice(h->device);
-    cudaStreamSynchronize(h->stream);
-    if (h->copy_in) { cudaStreamSynchronize(h->copy_in); cudaStreamSynchronize(h->copy_out); cudaStreamSynchronize(h->aux); }
+    m3s_sync_streams(h);
     M3sBuf *bufs[] = {&h->b_stage_in[0], &h->b_stage_in[1], &h->b_pcm_stage[0], &h->b_pcm_stage[1],
                       &h->b_sf, &h->b_S, &h->b_spec,
-                      &h->b_work, &h->b_spec_export, &h->e_pcm, &h->e_clips, &h->e_mdct,
-                      &h->e_ix, &h->e_info, &h->e_gran, &h->e_out, &h->e_payload, &h->e_misc, &h->e_pad, &h->e_tabs, &h->e_state,
-                      &h->e_lastix, &h->e_scfsi, &h->e_work, &h->e_clips2, &h->e_mdct2, &h->e_gran2, &h->e_ix2, &h->e_info2, &h->e_scfsi2,
-                      &h->e_var, &h->e_var2, &h->e_sum, &h->e_sum2, &h->e_cand};
+                      &h->b_work, &h->b_spec_export, &h->e_pcm, &h->e_clips, &h->e_out, &h->e_payload, &h->e_misc, &h->e_pad,
+                      &h->e_tabs, &h->e_state, &h->e_lastix, &h->e_work, &h->e_cand};
     for (M3sBuf *b : bufs) free_buf(*b);
+    for (M3sEncSet &es : h->es)
+        for (M3sBuf *b : {&es.mdct, &es.gran, &es.ix, &es.info, &es.scfsi, &es.var, &es.sum}) free_buf(*b);
     for (M3sScanSet &ss : h->ss) {
         M3sBuf *sb[] = {&ss.files, &ss.fouts, &ss.tmp_pos, &ss.fr_pos, &ss.fr_P, &ss.fr_meta, &ss.fr_carry, &ss.fr_reveal, &ss.fr_file,
                         &ss.units, &ss.tabids, &ss.reveal, &ss.layout, &ss.irr};
@@ -414,12 +425,11 @@ extern "C" int m3s_destroy(m3s_handle_t h)
     if (h->copy_out) cudaStreamDestroy(h->copy_out);
     if (h->aux) cudaStreamDestroy(h->aux);
     for (int i = 0; i < 2; i++)
-        if (h->ev_ana[i]) { cudaEventDestroy(h->ev_ana[i]); cudaEventDestroy(h->ev_rate[i]); cudaEventDestroy(h->ev_pack[i]); }
+        if (h->ev_ana[i]) { cudaEventDestroy(h->ev_ana[i]); cudaEventDestroy(h->ev_pack[i]); }
     for (int i = 0; i < 2; i++) {
         if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
         if (h->ev_free[i]) cudaEventDestroy(h->ev_free[i]);
     }
-    if (h->ev_done) cudaEventDestroy(h->ev_done);
     for (int i = 0; i < 3; i++)
         if (h->ev_pace[i]) cudaEventDestroy(h->ev_pace[i]);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);

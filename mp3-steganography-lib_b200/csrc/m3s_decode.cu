@@ -1054,29 +1054,15 @@ int m3s_upload_fast_const()
 // ================================================================================================
 // host orchestration
 // ================================================================================================
-#include <chrono>
-static const bool g_trace = getenv("M3S_TRACE") != nullptr;   // host-clock stage timing of the decode calls (diagnostic)
-static inline double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-#define M3S_TRACE_MARK(tag) do { if (g_trace) { const double t__ = now_ms(); fprintf(stderr, "[m3s %p] %-18s +%.2f ms\n", (void *)h, tag, t__ - tr_t); tr_t = t__; } } while (0)
+#define M3S_TRACE_MARK(tag) do { if (m3s_trace) { const double t__ = m3s_now_ms(); fprintf(stderr, "[m3s %p] %-18s +%.2f ms\n", (void *)h, tag, t__ - tr_t); tr_t = t__; } } while (0)
 
 static inline int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
-
-static int sync_all_streams(m3s_ctx *h)
-{
-    M3S_CUDA(h, cudaStreamSynchronize(h->stream));
-    if (h->copy_in) {
-        M3S_CUDA(h, cudaStreamSynchronize(h->copy_in));
-        M3S_CUDA(h, cudaStreamSynchronize(h->copy_out));
-        M3S_CUDA(h, cudaStreamSynchronize(h->aux));
-    }
-    return M3S_OK;
-}
 
 // grow-only reserve that is safe while other streams of the handle may still use the buffer
 static int reserve_quiet(m3s_ctx *h, M3sBuf &b, size_t bytes)
 {
     if (bytes <= b.cap) return M3S_OK;
-    int rc = sync_all_streams(h);
+    int rc = m3s_sync_streams(h);
     if (rc) return rc;
     return m3s_buf_reserve(h, b, bytes);
 }
@@ -1086,7 +1072,7 @@ static int reserve_quiet(m3s_ctx *h, M3sBuf &b, size_t bytes)
 static int pin_reserve(m3s_ctx *h, void *&p, size_t &cap, size_t bytes)
 {
     if (bytes <= cap) return M3S_OK;
-    int rc = sync_all_streams(h);
+    int rc = m3s_sync_streams(h);
     if (rc) return rc;
     if (p) M3S_CUDA(h, cudaFreeHost(p));
     p = nullptr;
@@ -1169,7 +1155,7 @@ static int scan_enqueue(m3s_ctx *h, M3sScanSet &ss, cudaStream_t s, const uint8_
         if ((rc = reserve_quiet(h, ss.tmp_pos, sizeof(uint32_t) * (size_t)(tb + 32)))) return rc;
         if ((rc = scan_reserve_frames(h, ss, est + 8))) return rc;
         if ((size_t)n_files > ss.fouts_cap) {
-            if ((rc = sync_all_streams(h))) return rc;
+            if ((rc = m3s_sync_streams(h))) return rc;
             if (ss.fouts_mapped) M3S_CUDA(h, cudaFreeHost(ss.fouts_mapped));
             ss.fouts_mapped = nullptr;
             ss.fouts_cap = 0;
@@ -1272,7 +1258,7 @@ extern "C" int m3s_decode_scan(m3s_handle_t h, const uint8_t *bytes, int mem, co
     h->scanned = false;
     if (!bytes || !file_off || n_files <= 0) return m3s_fail(h, M3S_ERR_ARG, "decode_scan: bytes/file_off/n_files");
     M3S_CUDA(h, cudaSetDevice(h->device));
-    double tr_t = g_trace ? now_ms() : 0.0;
+    double tr_t = m3s_trace ? m3s_now_ms() : 0.0;
     for (int i = 0; i < n_files; i++)
         if (file_off[i + 1] < file_off[i] || (audio_start && (audio_start[i] < 0)))
             return m3s_fail(h, M3S_ERR_ARG, "decode_scan: file_off must be non-decreasing, audio_start >= 0");
@@ -1505,7 +1491,7 @@ extern "C" int m3s_decode_run(m3s_handle_t h, void *pcm, int mem, const int64_t 
     M3sScanSet &ss = *h->cur;
     const int64_t nf = ss.total_frames;
     if (nf == 0) return M3S_OK;
-    double tr_t = g_trace ? now_ms() : 0.0;
+    double tr_t = m3s_trace ? m3s_now_ms() : 0.0;
     const bool fl = (flags & M3S_DEC_PCM_FLOAT) != 0;
     const size_t esz = fl ? 4 : 2;
     int rc;
@@ -1536,7 +1522,7 @@ extern "C" int m3s_decode_run(m3s_handle_t h, void *pcm, int mem, const int64_t 
     if (spectra && mem == M3S_MEM_HOST)
         M3S_CUDA(h, m3s_copy_bulk(spectra, d_sp, (size_t)nf * 4 * 576 * 2, cudaMemcpyDeviceToHost, h->stream));
     M3S_TRACE_MARK("run.launched");
-    if (g_trace) { cudaStreamSynchronize(h->stream); M3S_TRACE_MARK("run.kernels_done"); }
+    if (m3s_trace) { cudaStreamSynchronize(h->stream); M3S_TRACE_MARK("run.kernels_done"); }
     if (mem == M3S_MEM_HOST) {
         bool dense = true;   // one paced transfer when the caller's layout is the staging layout
         for (int i = 0; i < ss.n_files; i++) dense = dense && user_base[i] == ss.files_h[i].pcm_base;
@@ -1615,8 +1601,8 @@ extern "C" int m3s_decode(m3s_handle_t h, const uint8_t *bytes, int mem, const i
     // M3S_TRACE=1: a timeline of the call (timing events on every stream; printed at the end, relative to the first upload)
     struct WaveEv { cudaEvent_t h2d0, h2d1, scan1, comp0, comp1, out0, out1; double host_scan_wait_ms; };
     std::vector<WaveEv> tev;
-    auto mark = [&](cudaEvent_t &e, cudaStream_t st) { if (g_trace) { cudaEventCreate(&e); cudaEventRecord(e, st); } };
-    if (g_trace) { tev.assign(W, WaveEv()); }
+    auto mark = [&](cudaEvent_t &e, cudaStream_t st) { if (m3s_trace) { cudaEventCreate(&e); cudaEventRecord(e, st); } };
+    if (m3s_trace) { tev.assign(W, WaveEv()); }
     int err = M3S_OK;
     for (int k = 0; k <= W && err == M3S_OK; k++) {
         // ------------------------------------------------------------ A(k): bytes of wave k up, scan of wave k
@@ -1635,25 +1621,25 @@ extern "C" int m3s_decode(m3s_handle_t h, const uint8_t *bytes, int mem, const i
                 if (host) M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_d_out[b], 0));
             }
             if (host) {
-                if (g_trace) mark(tev[k].h2d0, h->copy_in);
+                if (m3s_trace) mark(tev[k].h2d0, h->copy_in);
                 M3S_CUDA(h, cudaMemcpyAsync((void *)d_bytes, bytes + file_off[f0], (size_t)nbytes, cudaMemcpyHostToDevice, h->copy_in));
-                if (g_trace) mark(tev[k].h2d1, h->copy_in);
+                if (m3s_trace) mark(tev[k].h2d1, h->copy_in);
                 M3S_CUDA(h, cudaEventRecord(h->ev_d_h2d[b], h->copy_in));
                 M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_d_h2d[b], 0));
             }
             if ((err = scan_enqueue(h, ss, h->aux, d_bytes, host ? bytes + file_off[f0] : nullptr, file_off + f0,
                                     audio_start ? audio_start + f0 : nullptr, nfl)))
                 break;
-            if (g_trace) mark(tev[k].scan1, h->aux);
+            if (m3s_trace) mark(tev[k].scan1, h->aux);
             M3S_CUDA(h, cudaEventRecord(h->ev_d_scan[b], h->aux));
         }
         // ------------------------------------------------------------ B(k - 1): kernels of wave k - 1, results home
         if (k >= 1) {
             const int j = k - 1, b = j & 1, f0 = wave_first[j];
             M3sScanSet &ss = h->ss[b];
-            const double tw0 = g_trace ? now_ms() : 0.0;
+            const double tw0 = m3s_trace ? m3s_now_ms() : 0.0;
             M3S_CUDA(h, cudaEventSynchronize(h->ev_d_scan[b]));
-            if (g_trace) tev[j].host_scan_wait_ms = now_ms() - tw0;
+            if (m3s_trace) tev[j].host_scan_wait_ms = m3s_now_ms() - tw0;
             if ((err = scan_finish(h, ss, h->aux, file_off + f0, audio_start ? audio_start + f0 : nullptr))) break;
             int64_t wave_elems = 0;
             for (int i = 0; i < ss.n_files; i++) {
@@ -1687,9 +1673,9 @@ extern "C" int m3s_decode(m3s_handle_t h, const uint8_t *bytes, int mem, const i
                 if (j >= 2) M3S_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_d_out[b], 0));   // the staging buffer's previous wave is home
             }
             M3S_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_d_scan[b], 0));
-            if (g_trace) mark(tev[j].comp0, h->stream);
+            if (m3s_trace) mark(tev[j].comp0, h->stream);
             if ((err = run_enqueue(h, ss, d_pcm, nullptr, flags, b))) break;
-            if (g_trace) mark(tev[j].comp1, h->stream);
+            if (m3s_trace) mark(tev[j].comp1, h->stream);
             const size_t nb = (size_t)12 * (size_t)ss.total_frames;
             if (!host && nb) {
                 if (table_ids) M3S_CUDA(h, cudaMemcpyAsync(table_ids + 12 * frames_before, ss.tabids.p, nb, cudaMemcpyDeviceToDevice, h->stream));
@@ -1701,10 +1687,10 @@ extern "C" int m3s_decode(m3s_handle_t h, const uint8_t *bytes, int mem, const i
                 if (nb && table_ids) M3S_CUDA(h, cudaMemcpyAsync(table_ids + 12 * frames_before, ss.tabids.p, nb, cudaMemcpyDeviceToHost, h->copy_out));
                 if (nb && reveal_bits) M3S_CUDA(h, cudaMemcpyAsync(reveal_bits + 12 * frames_before, ss.reveal.p, nb, cudaMemcpyDeviceToHost, h->copy_out));
                 M3S_CUDA(h, cudaStreamWaitEvent(h->copy_out, h->ev_d_comp[b], 0));
-                if (g_trace) mark(tev[j].out0, h->copy_out);
+                if (m3s_trace) mark(tev[j].out0, h->copy_out);
                 if (wave_elems)
                     M3S_CUDA(h, cudaMemcpyAsync((char *)pcm + elems_before * esz, d_pcm, (size_t)wave_elems * esz, cudaMemcpyDeviceToHost, h->copy_out));
-                if (g_trace) mark(tev[j].out1, h->copy_out);
+                if (m3s_trace) mark(tev[j].out1, h->copy_out);
                 M3S_CUDA(h, cudaEventRecord(h->ev_d_out[b], h->copy_out));
             }
             frames_before += ss.total_frames;
@@ -1713,8 +1699,8 @@ extern "C" int m3s_decode(m3s_handle_t h, const uint8_t *bytes, int mem, const i
     }
     if (err == M3S_OK && pcm_off) pcm_off[n_files] = elems_before;
     const std::string keep = h->err;
-    const int rc2 = sync_all_streams(h);
-    if (g_trace && err == M3S_OK && host && W > 0) {
+    const int rc2 = m3s_sync_streams(h);
+    if (m3s_trace && err == M3S_OK && host && W > 0) {
         auto rel = [&](cudaEvent_t e) { float ms = 0.f; if (e) cudaEventElapsedTime(&ms, tev[0].h2d0, e); return ms; };
         fprintf(stderr, "[m3s_decode] %d waves; per wave (ms since the first upload): h2d [start end] scan_end comp [start end] d2h [start end] | host wait for the scan\n", W);
         for (int k = 0; k < W; k++)

@@ -17,9 +17,9 @@
 // double-precision fallback in quantize (:401-407) and the padding recurrence (:504-513, :630-632) done on the host.
 #include <math.h>
 #include <string.h>
-#include <time.h>
 
 #include <algorithm>
+#include <functional>
 #include <vector>
 
 #include "m3s_common.cuh"
@@ -1724,8 +1724,7 @@ static void build_enc_tables(const M3sDevTables *T, EncTables *E)
     }
 }
 
-// The candidate payloads of m3s_encode_offsets (see the header).  With them the encoder runs in offsets mode: analysis and probe as
-// always, then k_enc_offsets instead of resolve, emit and pack; hide_str_offset_out is indexed by candidate.
+// The candidate payloads of m3s_encode_offsets (see the header).
 struct EncOffsets {
     const uint8_t *body;
     const int64_t *body_off, *cand_off;
@@ -1733,188 +1732,129 @@ struct EncOffsets {
     const int64_t *head_off, *body_len;
 };
 
-static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                       int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
-                       const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                       int64_t *out_len, int64_t *hide_str_offset_out, const EncOffsets *ox);
+// The clip arguments every encode entry point takes (see the header), with one rate pair per clip.
+struct EncClips {
+    const int16_t *pcm;
+    int mem;
+    const int64_t *pcm_off, *n_samples;
+    int32_t n_clips;
+    const int32_t *sample_rate, *bitrate_kbps;
+};
 
-// every entry point runs here: an early return may leave work of the call on the helper streams, drained before the caller reuses buffers
-static int encode_call(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples, int32_t n_clips,
-                       const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits, const int64_t *payload_off,
-                       uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap, int64_t *out_len, int64_t *hide_str_offset_out,
-                       const EncOffsets *ox = nullptr)
-{
-    const int rc = encode_impl(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out,
-                               mp3_off, mp3_cap, out_len, hide_str_offset_out, ox);
-    if (rc != M3S_OK && h) {
-        cudaStreamSynchronize(h->stream);
-        if (h->copy_in) { cudaStreamSynchronize(h->copy_in); cudaStreamSynchronize(h->copy_out); cudaStreamSynchronize(h->aux); }
-    }
-    return rc;
-}
+#define M3S_ENC_MARK(tag) do { if (m3s_trace) { const double t__ = m3s_now_ms(); fprintf(stderr, "[m3s enc] %-22s +%.2f ms\n", tag, t__ - tr_t); tr_t = t__; } } while (0)
 
-extern "C" int m3s_encode(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                          int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
-                          const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                          int64_t *out_len, int64_t *hide_str_offset_out)
+// The checks every entry point starts with; `outputs`: the entry point's own required pointers are set.
+static int check_call(m3s_ctx *h, const EncClips &a, bool outputs)
 {
     if (!h) return M3S_ERR_ARG;
     h->enc_taps_ok = false;
-    if (sr_index_of(sample_rate) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: sample rate %d is not an MPEG-1 rate", sample_rate);
-    if (br_index_of(bitrate_kbps) < 0)
-        return m3s_fail(h, M3S_ERR_ARG, "encode: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", bitrate_kbps);
-    // the batch's one rate pair, broadcast to every clip
-    const std::vector<int32_t> srs((size_t)std::max(n_clips, 0), sample_rate), brs((size_t)std::max(n_clips, 0), bitrate_kbps);
-    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, srs.data(), brs.data(), payload_bits, payload_off, mp3_out, mp3_off,
-                       mp3_cap, out_len, hide_str_offset_out);
-}
-
-extern "C" int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                                int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
-                                const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                                int64_t *out_len, int64_t *hide_str_offset_out)
-{
-    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, payload_bits, payload_off, mp3_out, mp3_off,
-                       mp3_cap, out_len, hide_str_offset_out);
-}
-
-extern "C" int m3s_encode_offsets(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                                  int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *body,
-                                  const int64_t *body_off, const int64_t *cand_off, const uint8_t *head, const int64_t *head_off,
-                                  const int64_t *body_len, int64_t *hide_str_offset_out)
-{
-    const EncOffsets ox{body, body_off, cand_off, head, head_off, body_len};
-    return encode_call(h, pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps, nullptr, nullptr, nullptr, nullptr, nullptr,
-                       nullptr, hide_str_offset_out, &ox);
-}
-
-static const bool g_enc_trace = getenv("M3S_TRACE") != nullptr;   // host-clock stage timing of the encode call (diagnostic)
-static double enc_now_ms()
-{
-    timespec ts;
-    clock_gettime(CLOCK_MONOTONIC, &ts);
-    return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
-}
-#define M3S_ENC_MARK(tag) do { if (g_enc_trace) { const double t__ = enc_now_ms(); fprintf(stderr, "[m3s enc] %-22s +%.2f ms\n", tag, t__ - tr_t); tr_t = t__; } } while (0)
-
-// Offsets mode: the payload length k_enc_probe prunes the variants of caller clip j with (`sure3`).  It is the shortest hiding
-// candidate's: with a longer one the probe would skip end-of-payload variants that a shorter candidate meets.  An empty candidate
-// next to hiding ones needs variant 14 (no bits left) at every granule, which only a payload shorter than 3 bits keeps active.
-// 0 when no candidate hides.
-static int64_t offsets_probe_len(const EncOffsets &ox, int j)
-{
-    int64_t shortest = INT64_MAX;
-    bool empty = false;
-    for (int64_t c = ox.cand_off[j]; c < ox.cand_off[j + 1]; c++) {
-        const int64_t nbits = 8 * (ox.head_off[c + 1] - ox.head_off[c] + ox.body_len[c]);
-        if (nbits == 0) empty = true;
-        else shortest = std::min(shortest, nbits);
-    }
-    if (shortest == INT64_MAX) return 0;
-    return empty ? 1 : shortest;
-}
-
-static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
-                       int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
-                       const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
-                       int64_t *out_len, int64_t *hide_str_offset_out, const EncOffsets *ox)
-{
-    if (!h) return M3S_ERR_ARG;
-    double tr_t = g_enc_trace ? enc_now_ms() : 0.0;
-    h->enc_taps_ok = false;
-    if (!pcm || !n_samples || n_clips <= 0 || !sample_rate || !bitrate_kbps || (!ox && (!mp3_out || !mp3_off)) ||
-        (ox && (!ox->body_off || !ox->cand_off || !ox->head_off || !ox->body_len || !hide_str_offset_out)))
+    if (!a.pcm || !a.n_samples || a.n_clips <= 0 || !a.sample_rate || !a.bitrate_kbps || !outputs)
         return m3s_fail(h, M3S_ERR_ARG, "encode: null argument");
-    if ((uintptr_t)pcm & 3) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm must be 4-byte aligned (one stereo sample per word)");
-    if (ox && ox->cand_off[0] != 0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: cand_off[0] is %lld, not 0", (long long)ox->cand_off[0]);
-    // ---- per-clip checks, in the caller's order, before anything is queued
-    for (int j = 0; j < n_clips; j++) {
-        if (sr_index_of(sample_rate[j]) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: sample rate %d is not an MPEG-1 rate", j, sample_rate[j]);
-        if (br_index_of(bitrate_kbps[j]) < 0)
-            return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", j, bitrate_kbps[j]);
-        if (n_samples[j] < 0 || n_samples[j] % 1152) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d has %lld samples per channel, not a multiple of 1152 (the reference raises IndexError, MP3_Encoder.py:611-614)", j, (long long)n_samples[j]);
-        if (pcm_off && (pcm_off[j] & 1)) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm_off must be even (stereo samples)");
-        if (!ox) continue;
-        const int64_t c0 = ox->cand_off[j], c1 = ox->cand_off[j + 1], b0 = ox->body_off[j], b1 = ox->body_off[j + 1];
-        if (c1 < c0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: cand_off decreases (%lld -> %lld)", j, (long long)c0, (long long)c1);
-        if (b0 < 0 || b1 < b0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: bad body range [%lld, %lld)", j, (long long)b0, (long long)b1);
-        if (b1 > b0 && !ox->body) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: body is NULL", j);
-        for (int64_t c = c0; c < c1; c++) {
-            const int64_t h0 = ox->head_off[c], h1 = ox->head_off[c + 1], bl = ox->body_len[c];
-            if (h0 < 0 || h1 < h0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: bad head range [%lld, %lld)", j, (long long)c, (long long)h0, (long long)h1);
-            if (h1 - h0 > 32) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head of %lld bytes, more than 32", j, (long long)c, (long long)(h1 - h0));
-            if (h1 > h0 && !ox->head) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head is NULL", j, (long long)c);
-            if (bl < 0 || bl > b1 - b0)
-                return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: body_len %lld outside the clip's body of %lld bytes", j, (long long)c, (long long)bl, (long long)(b1 - b0));
-        }
-    }
-    M3S_CUDA(h, cudaSetDevice(h->device));
-    int rc;
-    // ---- the library's clip order: grouped by sample rate (stable), so that in every chunk the frame slots of one sample rate are
-    //      contiguous and the kernels that stage per-rate tables once per CTA (probe, resolve) run once per group.  Clip i of that
-    //      order is the caller's clip order[i]; every output goes back by the caller's index.
-    std::vector<int> order(n_clips), inv(n_clips);
-    for (int i = 0; i < n_clips; i++) order[i] = i;
-    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return sr_index_of(sample_rate[a]) < sr_index_of(sample_rate[b]); });
-    for (int i = 0; i < n_clips; i++) inv[order[i]] = i;
-    int grp[4];   // clips of sample rate index s: [grp[s], grp[s + 1])
+    if ((uintptr_t)a.pcm & 3) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm must be 4-byte aligned (one stereo sample per word)");
+    return M3S_OK;
+}
+
+// The checks of caller clip j, run by every entry point in the caller's order before anything is queued.
+static int check_clip(m3s_ctx *h, const EncClips &a, int j)
+{
+    if (sr_index_of(a.sample_rate[j]) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: sample rate %d is not an MPEG-1 rate", j, a.sample_rate[j]);
+    if (br_index_of(a.bitrate_kbps[j]) < 0)
+        return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", j, a.bitrate_kbps[j]);
+    if (a.n_samples[j] < 0 || a.n_samples[j] % 1152) return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d has %lld samples per channel, not a multiple of 1152 (the reference raises IndexError, MP3_Encoder.py:611-614)", j, (long long)a.n_samples[j]);
+    if (a.pcm_off && (a.pcm_off[j] & 1)) return m3s_fail(h, M3S_ERR_ARG, "encode: pcm_off must be even (stereo samples)");
+    return M3S_OK;
+}
+
+// The host-side layout of a call.  The library's clip order groups the clips by sample rate (stable), so that in every chunk the
+// frame slots of one sample rate are contiguous and the kernels that stage per-rate tables once per CTA (probe, resolve) run once
+// per group.  Clip i of that order is the caller's clip order[i]; every output goes back by the caller's index.
+struct EncLayout {
+    std::vector<int> order, inv;
+    int grp[4];                      // clips of sample rate index s: [grp[s], grp[s + 1])
+    std::vector<M3sEncClip> clips;   // in the library's order; the payload and output fields are the entry point's to fill
+    std::vector<uint32_t> byteoff;   // the padding tables
+    int64_t total_frames = 0, max_frames = 0;
+    // chunking: all clips advance together through windows of `cf` frames so that the intermediates (MDCT spectra 9.2 KB/frame,
+    // quantised values 4.6 KB/frame) stay bounded while every clip keeps its warp busy; chunk_cap = frame slots of the fullest chunk
+    int64_t cf = 0, n_chunks = 0, chunk_cap = 0;
+};
+
+static int enc_layout(m3s_ctx *h, const EncClips &a, EncLayout &L)
+{
+    const int n_clips = a.n_clips;
+    L.order.resize(n_clips);
+    L.inv.resize(n_clips);
+    for (int i = 0; i < n_clips; i++) L.order[i] = i;
+    std::stable_sort(L.order.begin(), L.order.end(), [&](int x, int y) { return sr_index_of(a.sample_rate[x]) < sr_index_of(a.sample_rate[y]); });
+    for (int i = 0; i < n_clips; i++) L.inv[L.order[i]] = i;
     for (int s = 0, i = 0; s < 4; s++) {
-        while (s < 3 && i < n_clips && sr_index_of(sample_rate[order[i]]) < s) i++;
-        grp[s] = s < 3 ? i : n_clips;
+        while (s < 3 && i < n_clips && sr_index_of(a.sample_rate[L.order[i]]) < s) i++;
+        L.grp[s] = s < 3 ? i : n_clips;
     }
     // ---- clip table
-    std::vector<M3sEncClip> clips(n_clips);
-    int64_t total_frames = 0, max_frames = 0, out_total = 0, pay_total = 0;
+    L.clips.resize(n_clips);
     for (int i = 0; i < n_clips; i++) {
-        const int j = order[i];
-        M3sEncClip &c = clips[i];
-        c.pcm_base = pcm_off ? pcm_off[j] : 0;
-        c.n_frames = (int32_t)(n_samples[j] / 1152);
-        c.frame_base = total_frames;
-        c.out_base = ox ? 0 : mp3_off[j];
-        c.payload_base = payload_bits && payload_off ? payload_off[j] : 0;
-        c.payload_len = ox ? offsets_probe_len(*ox, j) : (payload_bits && payload_off ? payload_off[j + 1] - payload_off[j] : 0);
-        c.sr_idx = (int16_t)sr_index_of(sample_rate[j]);
-        c.bitrate_idx = (int16_t)br_index_of(bitrate_kbps[j]);
-        total_frames += c.n_frames;
-        max_frames = std::max<int64_t>(max_frames, c.n_frames);
-        pay_total = std::max(pay_total, c.payload_base + c.payload_len);
+        const int j = L.order[i];
+        M3sEncClip &c = L.clips[i];
+        c.pcm_base = a.pcm_off ? a.pcm_off[j] : 0;
+        c.n_frames = (int32_t)(a.n_samples[j] / 1152);
+        c.frame_base = L.total_frames;
+        c.sr_idx = (int16_t)sr_index_of(a.sample_rate[j]);
+        c.bitrate_idx = (int16_t)br_index_of(a.bitrate_kbps[j]);
+        L.total_frames += c.n_frames;
+        L.max_frames = std::max<int64_t>(L.max_frames, c.n_frames);
     }
-    if (!pcm_off) {   // back to back in the caller's order
+    if (!a.pcm_off) {   // back to back in the caller's order
         int64_t e = 0;
-        for (int j = 0; j < n_clips; j++) { clips[inv[j]].pcm_base = e; e += 2 * n_samples[j]; }
+        for (int j = 0; j < n_clips; j++) { L.clips[L.inv[j]].pcm_base = e; e += 2 * a.n_samples[j]; }
     }
     // ---- padding tables: one per rate pair of the batch, sized to its longest clip, back to back
     int64_t pair_frames[3][16];
     for (auto &r : pair_frames) for (int64_t &v : r) v = -1;
-    for (const M3sEncClip &c : clips) pair_frames[c.sr_idx][c.bitrate_idx] = std::max<int64_t>(pair_frames[c.sr_idx][c.bitrate_idx], c.n_frames);
+    for (const M3sEncClip &c : L.clips) pair_frames[c.sr_idx][c.bitrate_idx] = std::max<int64_t>(pair_frames[c.sr_idx][c.bitrate_idx], c.n_frames);
     static const int kRates[3] = {44100, 48000, 32000};
-    std::vector<uint32_t> byteoff, tab;
+    std::vector<uint32_t> tab;
     int pair_base[3][16] = {}, pair_whole[3][16] = {};
     for (int s = 0; s < 3; s++)
         for (int b = 1; b < 15; b++) {
             if (pair_frames[s][b] < 0) continue;
             padding_prefix(kRates[s], kBitrates[b], pair_frames[s][b], tab, pair_whole[s][b]);
-            if (byteoff.size() + tab.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode: too many frames in one call");
-            pair_base[s][b] = (int)byteoff.size();
-            byteoff.insert(byteoff.end(), tab.begin(), tab.end());
+            if (L.byteoff.size() + tab.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode: too many frames in one call");
+            pair_base[s][b] = (int)L.byteoff.size();
+            L.byteoff.insert(L.byteoff.end(), tab.begin(), tab.end());
         }
-    for (M3sEncClip &c : clips) {
+    for (M3sEncClip &c : L.clips) {
         c.pad_base = pair_base[c.sr_idx][c.bitrate_idx];
         c.whole_slots = pair_whole[c.sr_idx][c.bitrate_idx];
-        c.out_len = (int64_t)(byteoff[(size_t)c.pad_base + c.n_frames] / 4) * 4;
-        out_total = std::max(out_total, c.out_base + c.out_len);
+        c.out_len = (int64_t)(L.byteoff[(size_t)c.pad_base + c.n_frames] / 4) * 4;
     }
-    const int64_t n_cand = ox ? ox->cand_off[n_clips] : 0;
-    for (int j = 0; j < n_clips; j++) {
-        const M3sEncClip &c = clips[inv[j]];
-        if (mp3_cap && mp3_cap[j] < c.out_len) return m3s_fail(h, M3S_ERR_CAPACITY, "encode: clip %d needs %lld output bytes, capacity %lld", j, (long long)c.out_len, (long long)mp3_cap[j]);
-        if (out_len) out_len[j] = c.out_len;
-        if (hide_str_offset_out && !ox) hide_str_offset_out[j] = 0;
-    }
-    for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = 0;
-    if (total_frames == 0 || (ox && n_cand == 0)) return M3S_OK;
-    M3S_ENC_MARK("clip table");
+    if (L.max_frames == 0) return M3S_OK;   // nothing to encode, no chunk
+    // host buffers: smaller chunks, because nothing runs before the first chunk's PCM has crossed PCIe (measured: 10.1 -> 10.5 M frames/s e2e)
+    const int64_t budget_frames = h->enc_chunk_budget > 0 ? h->enc_chunk_budget : (a.mem == M3S_MEM_HOST ? (1 << 17) : (1 << 19));
+    L.cf = std::min(std::max<int64_t>(1, budget_frames / n_clips), L.max_frames);
+    for (const M3sEncClip &c : L.clips) L.chunk_cap += std::min<int64_t>(L.cf, c.n_frames);
+    L.n_chunks = (L.max_frames + L.cf - 1) / L.cf;
+    return M3S_OK;
+}
+
+// What the kernels that follow the probe read in chunk k: frames [c0, c0 + cf) of every clip.
+struct EncChunk {
+    int64_t k, c0, slots;        // slots: the chunk's frame slots
+    const M3sEncClip *clips;     // chunk-local clip records (device)
+    const int32_t *frame_clip;   // clip index of every frame slot of the chunk (device)
+    const int64_t *grp_slot;     // frame slots of sample rate index s: [grp_slot[s], grp_slot[s + 1])
+    const M3sEncSet &set;        // the chunk's intermediates
+};
+
+// Runs every chunk of a call: analysis, probe, then `after_probe` on the main stream.  With host buffers the PCM is staged in and,
+// when mp3_out is given, each chunk's MP3 bytes go back to it from e_out.  The carried states start at zero; `states` receives them.
+static int enc_pipeline(m3s_ctx *h, const EncClips &a, const EncLayout &L, std::vector<M3sEncState> &states, uint8_t *mp3_out,
+                        double tr_t, const std::function<int(const EncChunk &)> &after_probe)
+{
+    int rc;
+    const int n_clips = a.n_clips;
+    const std::vector<M3sEncClip> &clips = L.clips;
+    const int64_t cf = L.cf, n_chunks = L.n_chunks;
     // ---- encoder constant tables (once per handle)
     if (!h->e_tabs.p) {
         std::vector<uint8_t> hostT(sizeof(M3sDevTables));
@@ -1929,101 +1869,26 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     }
     // ---- inputs.  Host buffers are streamed: the PCM of chunk k+1 crosses PCIe on `copy_in` while chunk k is in the
     //      kernels, and the MP3 bytes of chunk k-1 go back on `copy_out` (see the chunk loop below)
-    const bool host = mem == M3S_MEM_HOST;
-    const int16_t *d_pcm = pcm;
-    uint8_t *d_out = mp3_out;
+    const bool host = a.mem == M3S_MEM_HOST;
     if ((rc = m3s_pipeline_init(h))) return rc;
-    if (host && !ox) {
-        if ((rc = m3s_buf_reserve(h, h->e_out, (size_t)out_total + 16))) return rc;
-        d_out = (uint8_t *)h->e_out.p;
+    if ((rc = m3s_buf_reserve(h, h->e_pad, sizeof(uint32_t) * L.byteoff.size()))) return rc;
+    M3S_CUDA(h, cudaMemcpyAsync(h->e_pad.p, L.byteoff.data(), sizeof(uint32_t) * L.byteoff.size(), cudaMemcpyHostToDevice, h->stream));
+    if ((rc = m3s_buf_reserve(h, h->e_state, sizeof(M3sEncState) * states.size()))) return rc;
+    M3S_CUDA(h, cudaMemsetAsync(h->e_state.p, 0, sizeof(M3sEncState) * states.size(), h->stream));
+    const size_t cap = (size_t)L.chunk_cap;
+    for (int q = 0; q < (n_chunks > 1 ? 2 : 1); q++) {   // with several chunks, chunk k uses set k & 1
+        M3sEncSet &es = h->es[q];
+        if ((rc = m3s_buf_reserve(h, es.mdct, cap * 4 * 576 * 4))) return rc;
+        if ((rc = m3s_buf_reserve(h, es.gran, cap * 4 * sizeof(M3sEncStats)))) return rc;
+        if ((rc = m3s_buf_reserve(h, es.scfsi, cap * 8))) return rc;
+        if ((rc = m3s_buf_reserve(h, es.var, cap * 4 * 16 * sizeof(uint4)))) return rc;
+        if ((rc = m3s_buf_reserve(h, es.sum, cap * 4 * sizeof(uint32_t)))) return rc;
     }
-    // offsets mode: the candidates, k_enc_offsets' work items (32 candidates of one clip each, in the library's clip order, so that
-    // the items of one sample rate are [ogrp[s], ogrp[s + 1])), the heads and the bodies, in one buffer
-    std::vector<M3sOffCand> cands;
-    std::vector<M3sOffWork> owork;
-    int ogrp[4] = {0, 0, 0, 0};
-    const M3sOffCand *d_cands = nullptr;
-    const M3sOffWork *d_owork = nullptr;
-    const uint8_t *d_head = nullptr, *d_body = nullptr;
-    if (ox) {
-        cands.resize((size_t)n_cand);
-        int64_t body_total = 0;
-        for (int i = 0; i < n_clips; i++) {
-            const int j = order[i];
-            for (int s = 0; s < 4; s++)
-                if (grp[s] == i) ogrp[s] = (int)owork.size();
-            body_total = std::max(body_total, ox->body_off[j + 1]);
-            for (int64_t c = ox->cand_off[j]; c < ox->cand_off[j + 1]; c++) {
-                M3sOffCand &d = cands[(size_t)c];
-                d.head_base = (int32_t)ox->head_off[c];
-                d.head_len = (int32_t)(ox->head_off[c + 1] - ox->head_off[c]);
-                d.body_base = ox->body_off[j];
-                d.nbits = 8 * (d.head_len + ox->body_len[c]);
-                if ((c - ox->cand_off[j]) % 32 == 0) owork.push_back(M3sOffWork{i, (int32_t)std::min<int64_t>(32, ox->cand_off[j + 1] - c), c});
-            }
-        }
-        for (int s = 0; s < 4; s++)
-            if (grp[s] == n_clips) ogrp[s] = (int)owork.size();
-        const int64_t head_total = ox->head_off[n_cand];
-        if (head_total > INT32_MAX || owork.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: too many candidates in one call");
-        auto al16 = [](size_t b) { return (b + 15) / 16 * 16; };
-        const size_t o_work = al16(sizeof(M3sOffCand) * cands.size()), o_head = o_work + al16(sizeof(M3sOffWork) * owork.size());
-        const size_t o_body = o_head + al16((size_t)head_total);
-        if ((rc = m3s_buf_reserve(h, h->e_cand, o_body + (size_t)body_total + 16))) return rc;
-        char *base = (char *)h->e_cand.p;
-        M3S_CUDA(h, cudaMemcpyAsync(base, cands.data(), sizeof(M3sOffCand) * cands.size(), cudaMemcpyHostToDevice, h->stream));
-        M3S_CUDA(h, cudaMemcpyAsync(base + o_work, owork.data(), sizeof(M3sOffWork) * owork.size(), cudaMemcpyHostToDevice, h->stream));
-        if (head_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_head, ox->head, (size_t)head_total, cudaMemcpyHostToDevice, h->stream));
-        if (body_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_body, ox->body, (size_t)body_total, cudaMemcpyHostToDevice, h->stream));
-        d_cands = (const M3sOffCand *)base;
-        d_owork = (const M3sOffWork *)(base + o_work);
-        d_head = (const uint8_t *)(base + o_head);
-        d_body = (const uint8_t *)(base + o_body);
-    } else {
-        if ((rc = m3s_buf_reserve(h, h->e_payload, (size_t)pay_total + 16))) return rc;
-        if (pay_total > 0) M3S_CUDA(h, cudaMemcpyAsync(h->e_payload.p, payload_bits, (size_t)pay_total, cudaMemcpyHostToDevice, h->stream));
-    }
-    if ((rc = m3s_buf_reserve(h, h->e_pad, sizeof(uint32_t) * byteoff.size()))) return rc;
-    M3S_CUDA(h, cudaMemcpyAsync(h->e_pad.p, byteoff.data(), sizeof(uint32_t) * byteoff.size(), cudaMemcpyHostToDevice, h->stream));
-    const int64_t n_states = ox ? n_cand : n_clips;   // the carried state is per candidate in offsets mode
-    if ((rc = m3s_buf_reserve(h, h->e_state, sizeof(M3sEncState) * n_states))) return rc;
-    M3S_CUDA(h, cudaMemsetAsync(h->e_state.p, 0, sizeof(M3sEncState) * n_states, h->stream));
-    const size_t lastix_bytes = (size_t)n_clips * 4 * 288 * 4;
-    if (!ox && (rc = m3s_buf_reserve(h, h->e_lastix, 2 * lastix_bytes))) return rc;   // two sets: chunk k reads set k & 1 and writes the other
-
-    // ---- chunking: all clips advance together through windows of `cf` frames so that the intermediates
-    //      (MDCT spectra 9.2 KB/frame, quantised values 4.6 KB/frame) stay bounded while every clip keeps its warp busy
-    // host buffers: smaller chunks, because nothing runs before the first chunk's PCM has crossed PCIe (measured: 10.1 -> 10.5 M frames/s e2e)
-    const int64_t budget_frames = h->enc_chunk_budget > 0 ? h->enc_chunk_budget : (mem == M3S_MEM_HOST ? (1 << 17) : (1 << 19));
-    int64_t cf = std::max<int64_t>(1, budget_frames / n_clips);
-    if (cf >= max_frames) cf = max_frames;
-    const bool single_chunk = cf >= max_frames;
-    int64_t chunk_cap = 0;
-    for (int i = 0; i < n_clips; i++) chunk_cap += std::min<int64_t>(cf, clips[i].n_frames);
-    const int64_t n_chunks = (max_frames + cf - 1) / cf;
-    const int nset = n_chunks > 1 ? 2 : 1;   // every per-chunk intermediate exists twice: chunk k uses set k & 1
-    M3sBuf *b_mdct[2] = {&h->e_mdct, &h->e_mdct2}, *b_gran[2] = {&h->e_gran, &h->e_gran2}, *b_ix[2] = {&h->e_ix, &h->e_ix2};
-    M3sBuf *b_info[2] = {&h->e_info, &h->e_info2}, *b_scfsi[2] = {&h->e_scfsi, &h->e_scfsi2};
-    M3sBuf *b_var[2] = {&h->e_var, &h->e_var2}, *b_sum[2] = {&h->e_sum, &h->e_sum2};
-    for (int q = 0; q < nset; q++) {
-        if ((rc = m3s_buf_reserve(h, *b_mdct[q], (size_t)chunk_cap * 4 * 576 * 4))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_gran[q], (size_t)chunk_cap * 4 * sizeof(M3sEncStats)))) return rc;
-        if (!ox && (rc = m3s_buf_reserve(h, *b_ix[q], (size_t)chunk_cap * 4 * 288 * 4))) return rc;
-        if (!ox && (rc = m3s_buf_reserve(h, *b_info[q], (size_t)chunk_cap * 4 * ENC_INFO_FIELDS * 4))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_scfsi[q], (size_t)chunk_cap * 8))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_var[q], (size_t)chunk_cap * 4 * 16 * sizeof(uint4)))) return rc;
-        if ((rc = m3s_buf_reserve(h, *b_sum[q], (size_t)chunk_cap * 4 * sizeof(uint32_t)))) return rc;
-    }
-
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ProbeSmem)));
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_probe, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_resolve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis_fold, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Ana3Smem)));
     M3S_CUDA(h, cudaFuncSetAttribute(k_enc_analysis_fold, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     const int64_t ana_run = Ana3Smem::RUN;   // granules per analysis work item
-    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PackSmem)));
-    if (ox) M3S_CUDA(h, cudaFuncSetAttribute(k_enc_offsets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
     auto frames_in_chunk = [&](int i, int64_t c0) { return std::max<int64_t>(0, std::min<int64_t>(cf, clips[i].n_frames - c0)); };
     // host staging: per chunk every clip owns a region of cf * 1152 + 1056 stereo samples (1056 = the analysis history the
     // first granule of the chunk reaches back to: 480 window taps + one warm-up granule), two region sets for double buffering
@@ -2035,8 +1900,8 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
     bool free_recorded[2] = {false, false};
     struct ChunkEv { cudaEvent_t c0, c1, a0, a1, r1, p1, o1; };   // M3S_TRACE: copy in, analysis, rate loop, pack, copy out of every chunk
     std::vector<ChunkEv> tev;
-    if (g_enc_trace) tev.assign((size_t)n_chunks, ChunkEv{});
-    auto tmark = [&](cudaEvent_t &e, cudaStream_t st) { if (g_enc_trace) { cudaEventCreate(&e); cudaEventRecord(e, st); } };
+    if (m3s_trace) tev.assign((size_t)n_chunks, ChunkEv{});
+    auto tmark = [&](cudaEvent_t &e, cudaStream_t st) { if (m3s_trace) { cudaEventCreate(&e); cudaEventRecord(e, st); } };
     auto stage_chunk = [&](int64_t k) -> cudaError_t {   // H2D of the PCM that chunk k reads, into staging set k & 1
         const int64_t c0 = k * cf;
         const int pb = (int)(k & 1);
@@ -2047,16 +1912,16 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             const int64_t first = c0 * 1152 - 1056, s0 = std::max<int64_t>(first, 0), s1 = (c0 + nfc) * 1152;
             M3sRow r;
             r.dst = (char *)h->e_pcm.p + (size_t)pb * stage_bytes + ((size_t)i * region + (size_t)(s0 - first)) * 4;
-            r.src = (const char *)pcm + clips[i].pcm_base * 2 + s0 * 4;
+            r.src = (const char *)a.pcm + clips[i].pcm_base * 2 + s0 * 4;
             r.bytes = (size_t)(s1 - s0) * 4;
             rows.push_back(r);
         }
         cudaError_t e = cudaSuccess;
         if (free_recorded[pb]) e = cudaStreamWaitEvent(h->copy_in, h->ev_free[pb], 0);
-        if (g_enc_trace) tmark(tev[k].c0, h->copy_in);
+        if (m3s_trace) tmark(tev[k].c0, h->copy_in);
         if (e == cudaSuccess) e = m3s_copy_rows(rows, cudaMemcpyHostToDevice, h->copy_in);
         if (e == cudaSuccess) e = cudaEventRecord(h->ev_in[pb], h->copy_in);
-        if (g_enc_trace) tmark(tev[k].c1, h->copy_in);
+        if (m3s_trace) tmark(tev[k].c1, h->copy_in);
         return e;
     };
     // the first chunk's PCM starts crossing PCIe now, under the host work below (descriptors of every chunk); the descriptors' own
@@ -2075,7 +1940,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         int64_t base = 0;
         for (int i = 0; i < n_clips; i++) {
             for (int s = 0; s < 4; s++)
-                if (grp[s] == i) grp_slot[(size_t)k * 4 + s] = base;
+                if (L.grp[s] == i) grp_slot[(size_t)k * 4 + s] = base;
             const int64_t nfc = frames_in_chunk(i, c0);
             M3sEncClip &cc = cclips[(size_t)k * n_clips + i];
             cc = clips[i];
@@ -2094,7 +1959,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             base += nfc;
         }
         for (int s = 0; s < 4; s++)
-            if (grp[s] == n_clips) grp_slot[(size_t)k * 4 + s] = base;
+            if (L.grp[s] == n_clips) grp_slot[(size_t)k * 4 + s] = base;
         work_off[k + 1] = (int64_t)work.size();
         slot_off[k + 1] = slot_off[k] + base;
     }
@@ -2119,7 +1984,7 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         const int pb = (int)(k & 1);
         const int64_t nw = work_off[k + 1] - work_off[k];
         if (nw == 0) return M3S_OK;
-        const int16_t *k_pcm = d_pcm;
+        const int16_t *k_pcm = a.pcm;
         if (host) {
             k_pcm = (const int16_t *)((const char *)h->e_pcm.p + (size_t)pb * stage_bytes);
             M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_in[pb], 0));
@@ -2129,13 +1994,13 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         // then fills what is left instead of crowding the critical chain out
         if (k >= 2) M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_pack[pb], 0));
         M3sLaunchOn on_aux(h, h->aux);   // timing events of this launch go to the aux stream; restored on every return path
-        if (g_enc_trace) tmark(tev[k].a0, h->aux);
+        if (m3s_trace) tmark(tev[k].a0, h->aux);
         M3S_KBEGIN(h, M3S_K_ENC_ANALYSIS);
         k_enc_analysis_fold<<<(unsigned)nw, 32 * ANA3_WARPS, sizeof(Ana3Smem), h->aux>>>(
             k_pcm, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips, (const M3sEncWork *)h->e_work.p + work_off[k], h->d_tab,
-            (const EncTables *)h->e_tabs.p, 0, (int32_t *)b_mdct[pb]->p, (M3sEncStats *)b_gran[pb]->p, 0u);
+            (const EncTables *)h->e_tabs.p, 0, (int32_t *)h->es[pb].mdct.p, (M3sEncStats *)h->es[pb].gran.p, 0u);
         M3S_LAUNCH_CHECK(h);
-        if (g_enc_trace) tmark(tev[k].a1, h->aux);
+        if (m3s_trace) tmark(tev[k].a1, h->aux);
         M3S_CUDA(h, cudaEventRecord(h->ev_ana[pb], h->aux));
         if (host) {
             M3S_CUDA(h, cudaEventRecord(h->ev_free[pb], h->aux));   // the staging set may be refilled once the analysis has read it
@@ -2157,59 +2022,24 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         const int pb = (int)(k & 1);
         const int64_t chunk_total = slot_off[k + 1] - slot_off[k];
         if (chunk_total == 0) break;
-        const M3sEncClip *d_clips = (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips;
-        const int64_t *gsl = &grp_slot[(size_t)k * 4];
+        const M3sEncSet &es = h->es[pb];
+        const EncChunk chunk{k, c0, chunk_total, (const M3sEncClip *)h->e_clips.p + (size_t)k * n_clips,
+                             (const int32_t *)h->e_misc.p + slot_off[k], &grp_slot[(size_t)k * 4], es};
         M3S_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_ana[pb], 0));
-        const int64_t n_gran = 4 * chunk_total;
         for (int s = 0; s < 3; s++) {
-            const int64_t g0 = 4 * gsl[s], g1 = 4 * gsl[s + 1];
+            const int64_t g0 = 4 * chunk.grp_slot[s], g1 = 4 * chunk.grp_slot[s + 1];
             if (g1 == g0) continue;
             M3S_KBEGIN(h, M3S_K_ENC_RATE);
             k_enc_probe<<<(unsigned)((g1 - g0 + PROBE_WARPS * PROBE_G - 1) / (PROBE_WARPS * PROBE_G)), 32 * PROBE_WARPS, sizeof(ProbeSmem), h->stream>>>(
-                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-                s, g0, g1, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (uint4 *)b_var[pb]->p,
-                (uint32_t *)b_sum[pb]->p, (uint8_t *)b_scfsi[pb]->p);
+                chunk.clips, chunk.frame_clip, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+                s, g0, g1, (const int32_t *)es.mdct.p, (const M3sEncStats *)es.gran.p, (uint4 *)es.var.p,
+                (uint32_t *)es.sum.p, (uint8_t *)es.scfsi.p);
             M3S_LAUNCH_CHECK(h);
         }
-        if (g_enc_trace) tmark(tev[k].r1, h->stream);
-        M3S_CUDA(h, cudaEventRecord(h->ev_rate[pb], h->stream));
+        if (m3s_trace) tmark(tev[k].r1, h->stream);
         if (host && k + 2 < n_chunks) M3S_CUDA(h, stage_chunk(k + 2));
-        if (ox) {   // offsets mode: every candidate's offset chain instead of resolve, emit and pack
-            for (int s = 0; s < 3; s++) {
-                if (gsl[s + 1] == gsl[s] || ogrp[s + 1] == ogrp[s]) continue;
-                M3S_KBEGIN(h, M3S_K_ENC_OFFSETS);
-                k_enc_offsets<<<(unsigned)((ogrp[s + 1] - ogrp[s] + OFFSETS_WARPS - 1) / OFFSETS_WARPS), 32 * OFFSETS_WARPS, sizeof(RateSmem), h->stream>>>(
-                    d_clips, d_owork, ogrp[s], ogrp[s + 1], d_cands, d_head, d_body, (M3sEncState *)h->e_state.p, h->d_tab,
-                    (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
-                    (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (const uint32_t *)b_sum[pb]->p);
-                M3S_LAUNCH_CHECK(h);
-            }
-        } else {
-            for (int s = 0; s < 3; s++) {
-                if (gsl[s + 1] == gsl[s]) continue;   // no clip of this sample rate has a frame in the chunk
-                M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
-                k_enc_resolve<<<(unsigned)((grp[s + 1] - grp[s] + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
-                    d_clips, grp[s], grp[s + 1], (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
-                    (const uint8_t *)h->e_payload.p, s, (int32_t)c0, (int32_t)cf, (const int32_t *)b_mdct[pb]->p,
-                    (const M3sEncStats *)b_gran[pb]->p, (const uint4 *)b_var[pb]->p, (uint32_t *)b_sum[pb]->p, (int32_t *)b_info[pb]->p);
-                M3S_LAUNCH_CHECK(h);
-            }
-            M3S_KBEGIN(h, M3S_K_ENC_AUX);
-            k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
-                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const EncTables *)h->e_tabs.p, (int32_t)c0, (int32_t)cf,
-                n_gran, (const int32_t *)b_mdct[pb]->p, (const M3sEncStats *)b_gran[pb]->p, (const uint32_t *)b_sum[pb]->p,
-                (const int32_t *)b_info[pb]->p, (uint32_t *)b_ix[pb]->p,
-                (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(k & 1) * lastix_bytes),
-                (uint32_t *)((char *)h->e_lastix.p + (size_t)((k + 1) & 1) * lastix_bytes));
-            M3S_LAUNCH_CHECK(h);
-            // packing stays on the rate loop's stream
-            M3S_KBEGIN(h, M3S_K_ENC_PACK);
-            k_enc_pack<<<(unsigned)((chunk_total + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
-                d_clips, (const int32_t *)h->e_misc.p + slot_off[k], h->d_tab, (const uint32_t *)h->e_pad.p, 0, chunk_total,
-                (const uint32_t *)b_ix[pb]->p, (const int32_t *)b_info[pb]->p, (const uint8_t *)b_scfsi[pb]->p, d_out);
-            M3S_LAUNCH_CHECK(h);
-        }
-        if (g_enc_trace) tmark(tev[k].p1, h->stream);
+        if ((rc = after_probe(chunk))) return rc;
+        if (m3s_trace) tmark(tev[k].p1, h->stream);
         M3S_CUDA(h, cudaEventRecord(h->ev_pack[pb], h->stream));
         // the rate loop and the analysis are both issue-bound: the next chunk's analysis waits for this chunk's packing (measured:
         // overlapping them gains nothing and stretches the analysis kernel's own time)
@@ -2217,32 +2047,29 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
             M3S_CUDA(h, cudaStreamWaitEvent(h->aux, h->ev_pack[pb], 0));
             if ((rc = launch_analysis(k + 1))) return rc;
         }
-        if (host && !ox) {   // this chunk's bytes of every clip go home behind the pack kernel
+        if (host && mp3_out) {   // this chunk's bytes of every clip go home behind the pack kernel
             M3S_CUDA(h, cudaStreamWaitEvent(h->copy_out, h->ev_pack[pb], 0));
             rows.clear();
             for (int i = 0; i < n_clips; i++) {
                 const int64_t nfc = frames_in_chunk(i, c0);
                 if (nfc == 0) continue;
-                const uint32_t *bo = byteoff.data() + clips[i].pad_base;
+                const uint32_t *bo = L.byteoff.data() + clips[i].pad_base;
                 const int64_t b0 = bo[c0], b1 = std::min<int64_t>(bo[c0 + nfc], clips[i].out_len);
                 if (b1 <= b0) continue;
                 M3sRow r;
                 r.dst = (char *)mp3_out + clips[i].out_base + b0;
-                r.src = (const char *)d_out + clips[i].out_base + b0;
+                r.src = (const char *)h->e_out.p + clips[i].out_base + b0;
                 r.bytes = (size_t)(b1 - b0);
                 rows.push_back(r);
             }
             M3S_CUDA(h, m3s_copy_rows(rows, cudaMemcpyDeviceToHost, h->copy_out));
-            if (g_enc_trace) tmark(tev[k].o1, h->copy_out);
+            if (m3s_trace) tmark(tev[k].o1, h->copy_out);
         }
     }
     M3S_ENC_MARK("chunks queued");
-    M3S_CUDA(h, cudaStreamSynchronize(h->stream));
-    M3S_CUDA(h, cudaStreamSynchronize(h->aux));
-    M3S_CUDA(h, cudaStreamSynchronize(h->copy_out));
-    if (host) M3S_CUDA(h, cudaStreamSynchronize(h->copy_in));
+    if ((rc = m3s_sync_streams(h))) return rc;
     M3S_ENC_MARK("streams drained");
-    if (g_enc_trace && host) {   // timeline of the call, ms since the first copy was queued
+    if (m3s_trace && host) {   // timeline of the call, ms since the first copy was queued
         auto at = [&](cudaEvent_t e) { float ms = -1.f; if (e) cudaEventElapsedTime(&ms, tev[0].c0, e); return ms; };
         for (int64_t k = 0; k < n_chunks; k++) {
             if (k < 6 || k >= n_chunks - 3)
@@ -2252,44 +2079,256 @@ static int encode_impl(m3s_handle_t h, const int16_t *pcm, int mem, const int64_
         for (int64_t k = 0; k < n_chunks; k++)
             for (cudaEvent_t e : {tev[k].c0, tev[k].c1, tev[k].a0, tev[k].a1, tev[k].r1, tev[k].p1, tev[k].o1}) if (e) cudaEventDestroy(e);
     }
-    if (ox) {   // ---- offsets mode: results by the caller's candidate index
-        std::vector<M3sEncState> states((size_t)n_cand);
-        M3S_CUDA(h, cudaMemcpyAsync(states.data(), h->e_state.p, sizeof(M3sEncState) * n_cand, cudaMemcpyDeviceToHost, h->stream));
-        M3S_CUDA(h, cudaStreamSynchronize(h->stream));
-        for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = states[(size_t)c].hide_off;
-        for (int j = 0; j < n_clips; j++)
-            for (int64_t c = ox->cand_off[j]; c < ox->cand_off[j + 1]; c++)
-                if (states[(size_t)c].overrun)
-                    return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld frame %d: the step search runs past the end of the step "
-                                    "table (quantize would read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)",
-                                    j, (long long)c, states[(size_t)c].overrun - 1);
-        return M3S_OK;
-    }
-    // ---- results, by the caller's clip index
-    std::vector<M3sEncState> states(n_clips);
-    M3S_CUDA(h, cudaMemcpyAsync(states.data(), h->e_state.p, sizeof(M3sEncState) * n_clips, cudaMemcpyDeviceToHost, h->stream));
+    M3S_CUDA(h, cudaMemcpyAsync(states.data(), h->e_state.p, sizeof(M3sEncState) * states.size(), cudaMemcpyDeviceToHost, h->stream));
     M3S_CUDA(h, cudaStreamSynchronize(h->stream));
+    return M3S_OK;
+}
+
+// An error return may leave work of the call on the handle's streams: they are drained before the caller reuses its buffers.
+static int drain_on_error(m3s_ctx *h, int rc)
+{
+    if (rc != M3S_OK && h) { const std::string keep = h->err; m3s_sync_streams(h); h->err = keep; }
+    return rc;
+}
+
+// m3s_encode and m3s_encode_mixed: MP3 bytes, out_len and hide_str_offset of every clip
+static int encode_mp3(m3s_ctx *h, const EncClips &a, const uint8_t *payload_bits, const int64_t *payload_off, uint8_t *mp3_out,
+                      const int64_t *mp3_off, const int64_t *mp3_cap, int64_t *out_len, int64_t *hide_str_offset_out)
+{
+    double tr_t = m3s_trace ? m3s_now_ms() : 0.0;
+    int rc;
+    if ((rc = check_call(h, a, mp3_out && mp3_off))) return rc;
+    for (int j = 0; j < a.n_clips; j++)
+        if ((rc = check_clip(h, a, j))) return rc;
+    M3S_CUDA(h, cudaSetDevice(h->device));
+    EncLayout L;
+    if ((rc = enc_layout(h, a, L))) return rc;
+    const int n_clips = a.n_clips;
+    int64_t out_total = 0, pay_total = 0;
+    for (int j = 0; j < n_clips; j++) {
+        M3sEncClip &c = L.clips[L.inv[j]];
+        c.out_base = mp3_off[j];
+        c.payload_base = payload_bits && payload_off ? payload_off[j] : 0;
+        c.payload_len = payload_bits && payload_off ? payload_off[j + 1] - payload_off[j] : 0;
+        out_total = std::max(out_total, c.out_base + c.out_len);
+        pay_total = std::max(pay_total, c.payload_base + c.payload_len);
+        if (mp3_cap && mp3_cap[j] < c.out_len) return m3s_fail(h, M3S_ERR_CAPACITY, "encode: clip %d needs %lld output bytes, capacity %lld", j, (long long)c.out_len, (long long)mp3_cap[j]);
+        if (out_len) out_len[j] = c.out_len;
+        if (hide_str_offset_out) hide_str_offset_out[j] = 0;
+    }
+    if (L.total_frames == 0) return M3S_OK;
+    M3S_ENC_MARK("clip table");
+    uint8_t *d_out = mp3_out;
+    if (a.mem == M3S_MEM_HOST) {
+        if ((rc = m3s_buf_reserve(h, h->e_out, (size_t)out_total + 16))) return rc;
+        d_out = (uint8_t *)h->e_out.p;
+    }
+    if ((rc = m3s_buf_reserve(h, h->e_payload, (size_t)pay_total + 16))) return rc;
+    if (pay_total > 0) M3S_CUDA(h, cudaMemcpyAsync(h->e_payload.p, payload_bits, (size_t)pay_total, cudaMemcpyHostToDevice, h->stream));
+    const size_t lastix_bytes = (size_t)n_clips * 4 * 288 * 4;
+    if ((rc = m3s_buf_reserve(h, h->e_lastix, 2 * lastix_bytes))) return rc;   // two sets: chunk k reads set k & 1 and writes the other
+    for (int q = 0; q < (L.n_chunks > 1 ? 2 : 1); q++) {
+        if ((rc = m3s_buf_reserve(h, h->es[q].ix, (size_t)L.chunk_cap * 4 * 288 * 4))) return rc;
+        if ((rc = m3s_buf_reserve(h, h->es[q].info, (size_t)L.chunk_cap * 4 * ENC_INFO_FIELDS * 4))) return rc;
+    }
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_resolve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PackSmem)));
+    std::vector<M3sEncState> states(n_clips);
+    rc = enc_pipeline(h, a, L, states, mp3_out, tr_t, [&](const EncChunk &c) -> int {
+        const M3sEncSet &es = c.set;
+        for (int s = 0; s < 3; s++) {
+            if (c.grp_slot[s + 1] == c.grp_slot[s]) continue;   // no clip of this sample rate has a frame in the chunk
+            M3S_KBEGIN(h, M3S_K_ENC_RESOLVE);
+            k_enc_resolve<<<(unsigned)((L.grp[s + 1] - L.grp[s] + RESOLVE_WARPS - 1) / RESOLVE_WARPS), 32 * RESOLVE_WARPS, sizeof(RateSmem), h->stream>>>(
+                c.clips, L.grp[s], L.grp[s + 1], (M3sEncState *)h->e_state.p, h->d_tab, (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p,
+                (const uint8_t *)h->e_payload.p, s, (int32_t)c.c0, (int32_t)L.cf, (const int32_t *)es.mdct.p,
+                (const M3sEncStats *)es.gran.p, (const uint4 *)es.var.p, (uint32_t *)es.sum.p, (int32_t *)es.info.p);
+            M3S_LAUNCH_CHECK(h);
+        }
+        const int64_t n_gran = 4 * c.slots;
+        M3S_KBEGIN(h, M3S_K_ENC_AUX);
+        k_enc_emit<<<(unsigned)((n_gran + EMIT_WARPS * EMIT_G - 1) / (EMIT_WARPS * EMIT_G)), 32 * EMIT_WARPS, sizeof(RateSmem), h->stream>>>(
+            c.clips, c.frame_clip, h->d_tab, (const EncTables *)h->e_tabs.p, (int32_t)c.c0, (int32_t)L.cf,
+            n_gran, (const int32_t *)es.mdct.p, (const M3sEncStats *)es.gran.p, (const uint32_t *)es.sum.p,
+            (const int32_t *)es.info.p, (uint32_t *)es.ix.p,
+            (const uint32_t *)((const char *)h->e_lastix.p + (size_t)(c.k & 1) * lastix_bytes),
+            (uint32_t *)((char *)h->e_lastix.p + (size_t)((c.k + 1) & 1) * lastix_bytes));
+        M3S_LAUNCH_CHECK(h);
+        // packing stays on the rate loop's stream
+        M3S_KBEGIN(h, M3S_K_ENC_PACK);
+        k_enc_pack<<<(unsigned)((c.slots + PACK_WARPS - 1) / PACK_WARPS), 32 * PACK_WARPS, sizeof(PackSmem), h->stream>>>(
+            c.clips, c.frame_clip, h->d_tab, (const uint32_t *)h->e_pad.p, 0, c.slots,
+            (const uint32_t *)es.ix.p, (const int32_t *)es.info.p, (const uint8_t *)es.scfsi.p, d_out);
+        M3S_LAUNCH_CHECK(h);
+        return M3S_OK;
+    });
+    if (rc) return rc;
+    // ---- results, by the caller's clip index
     if (hide_str_offset_out)
-        for (int j = 0; j < n_clips; j++) hide_str_offset_out[j] = states[inv[j]].hide_off;
+        for (int j = 0; j < n_clips; j++) hide_str_offset_out[j] = states[L.inv[j]].hide_off;
     for (int j = 0; j < n_clips; j++)
-        if (states[inv[j]].overrun)
+        if (states[L.inv[j]].overrun)
             return m3s_fail(h, M3S_ERR_ARG, "encode: clip %d frame %d: the step search runs past the end of the step table (quantize would "
-                            "read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)", j, states[inv[j]].overrun - 1);
+                            "read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)", j, states[L.inv[j]].overrun - 1);
     // taps: the device holds the frames in the library's clip order; (device frame, caller frame, frames) runs map them back
     h->enc_tap_runs.clear();
     std::vector<int64_t> caller_fb(n_clips + 1, 0);
-    for (int j = 0; j < n_clips; j++) caller_fb[j + 1] = caller_fb[j] + n_samples[j] / 1152;
+    for (int j = 0; j < n_clips; j++) caller_fb[j + 1] = caller_fb[j] + a.n_samples[j] / 1152;
     for (int i = 0; i < n_clips; i++) {
-        const int64_t src = clips[i].frame_base, dst = caller_fb[order[i]], n = clips[i].n_frames;
+        const int64_t src = L.clips[i].frame_base, dst = caller_fb[L.order[i]], n = L.clips[i].n_frames;
         std::vector<int64_t> &R = h->enc_tap_runs;
         if (n == 0) continue;
         if (!R.empty() && R[R.size() - 3] + R.back() == src && R[R.size() - 2] + R.back() == dst) R.back() += n;
         else R.insert(R.end(), {src, dst, n});
     }
-    h->enc_taps_ok = single_chunk;
-    h->enc_total_frames = total_frames;
-    h->enc_n_clips = n_clips;
+    h->enc_taps_ok = L.n_chunks == 1;
+    h->enc_total_frames = L.total_frames;
     return M3S_OK;
+}
+
+extern "C" int m3s_encode(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                          int32_t n_clips, int32_t sample_rate, int32_t bitrate_kbps, const uint8_t *payload_bits,
+                          const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
+                          int64_t *out_len, int64_t *hide_str_offset_out)
+{
+    if (!h) return M3S_ERR_ARG;
+    h->enc_taps_ok = false;
+    if (sr_index_of(sample_rate) < 0) return m3s_fail(h, M3S_ERR_ARG, "encode: sample rate %d is not an MPEG-1 rate", sample_rate);
+    if (br_index_of(bitrate_kbps) < 0)
+        return m3s_fail(h, M3S_ERR_ARG, "encode: bitrate %d is not an MPEG-1 Layer III rate (WAV_Reader.py:112-114)", bitrate_kbps);
+    // the batch's one rate pair, broadcast to every clip
+    const std::vector<int32_t> srs((size_t)std::max(n_clips, 0), sample_rate), brs((size_t)std::max(n_clips, 0), bitrate_kbps);
+    return drain_on_error(h, encode_mp3(h, EncClips{pcm, mem, pcm_off, n_samples, n_clips, srs.data(), brs.data()}, payload_bits,
+                                        payload_off, mp3_out, mp3_off, mp3_cap, out_len, hide_str_offset_out));
+}
+
+extern "C" int m3s_encode_mixed(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                                int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *payload_bits,
+                                const int64_t *payload_off, uint8_t *mp3_out, const int64_t *mp3_off, const int64_t *mp3_cap,
+                                int64_t *out_len, int64_t *hide_str_offset_out)
+{
+    return drain_on_error(h, encode_mp3(h, EncClips{pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps}, payload_bits,
+                                        payload_off, mp3_out, mp3_off, mp3_cap, out_len, hide_str_offset_out));
+}
+
+// The payload length k_enc_probe prunes the variants of caller clip j with (`sure3`).  It is the shortest hiding candidate's: with a
+// longer one the probe would skip end-of-payload variants that a shorter candidate meets.  An empty candidate next to hiding ones
+// needs variant 14 (no bits left) at every granule, which only a payload shorter than 3 bits keeps active.  0 when no candidate hides.
+static int64_t offsets_probe_len(const EncOffsets &ox, int j)
+{
+    int64_t shortest = INT64_MAX;
+    bool empty = false;
+    for (int64_t c = ox.cand_off[j]; c < ox.cand_off[j + 1]; c++) {
+        const int64_t nbits = 8 * (ox.head_off[c + 1] - ox.head_off[c] + ox.body_len[c]);
+        if (nbits == 0) empty = true;
+        else shortest = std::min(shortest, nbits);
+    }
+    if (shortest == INT64_MAX) return 0;
+    return empty ? 1 : shortest;
+}
+
+// m3s_encode_offsets: analysis and probe as for an encode, then k_enc_offsets instead of resolve, emit and pack;
+// hide_str_offset_out is indexed by candidate
+static int encode_offsets(m3s_ctx *h, const EncClips &a, const EncOffsets &ox, int64_t *hide_str_offset_out)
+{
+    double tr_t = m3s_trace ? m3s_now_ms() : 0.0;
+    int rc;
+    if ((rc = check_call(h, a, ox.body_off && ox.cand_off && ox.head_off && ox.body_len && hide_str_offset_out))) return rc;
+    if (ox.cand_off[0] != 0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: cand_off[0] is %lld, not 0", (long long)ox.cand_off[0]);
+    for (int j = 0; j < a.n_clips; j++) {
+        if ((rc = check_clip(h, a, j))) return rc;
+        const int64_t c0 = ox.cand_off[j], c1 = ox.cand_off[j + 1], b0 = ox.body_off[j], b1 = ox.body_off[j + 1];
+        if (c1 < c0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: cand_off decreases (%lld -> %lld)", j, (long long)c0, (long long)c1);
+        if (b0 < 0 || b1 < b0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: bad body range [%lld, %lld)", j, (long long)b0, (long long)b1);
+        if (b1 > b0 && !ox.body) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d: body is NULL", j);
+        for (int64_t c = c0; c < c1; c++) {
+            const int64_t h0 = ox.head_off[c], h1 = ox.head_off[c + 1], bl = ox.body_len[c];
+            if (h0 < 0 || h1 < h0) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: bad head range [%lld, %lld)", j, (long long)c, (long long)h0, (long long)h1);
+            if (h1 - h0 > 32) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head of %lld bytes, more than 32", j, (long long)c, (long long)(h1 - h0));
+            if (h1 > h0 && !ox.head) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: head is NULL", j, (long long)c);
+            if (bl < 0 || bl > b1 - b0)
+                return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld: body_len %lld outside the clip's body of %lld bytes", j, (long long)c, (long long)bl, (long long)(b1 - b0));
+        }
+    }
+    M3S_CUDA(h, cudaSetDevice(h->device));
+    EncLayout L;
+    if ((rc = enc_layout(h, a, L))) return rc;
+    const int n_clips = a.n_clips;
+    for (int j = 0; j < n_clips; j++) L.clips[L.inv[j]].payload_len = offsets_probe_len(ox, j);
+    const int64_t n_cand = ox.cand_off[n_clips];
+    for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = 0;
+    if (L.total_frames == 0 || n_cand == 0) return M3S_OK;
+    M3S_ENC_MARK("clip table");
+    // the candidates, k_enc_offsets' work items (32 candidates of one clip each, in the library's clip order, so that the items of
+    // one sample rate are [ogrp[s], ogrp[s + 1])), the heads and the bodies, in one buffer
+    std::vector<M3sOffCand> cands((size_t)n_cand);
+    std::vector<M3sOffWork> owork;
+    int ogrp[4] = {0, 0, 0, 0};
+    int64_t body_total = 0;
+    for (int i = 0; i < n_clips; i++) {
+        const int j = L.order[i];
+        for (int s = 0; s < 4; s++)
+            if (L.grp[s] == i) ogrp[s] = (int)owork.size();
+        body_total = std::max(body_total, ox.body_off[j + 1]);
+        for (int64_t c = ox.cand_off[j]; c < ox.cand_off[j + 1]; c++) {
+            M3sOffCand &d = cands[(size_t)c];
+            d.head_base = (int32_t)ox.head_off[c];
+            d.head_len = (int32_t)(ox.head_off[c + 1] - ox.head_off[c]);
+            d.body_base = ox.body_off[j];
+            d.nbits = 8 * (d.head_len + ox.body_len[c]);
+            if ((c - ox.cand_off[j]) % 32 == 0) owork.push_back(M3sOffWork{i, (int32_t)std::min<int64_t>(32, ox.cand_off[j + 1] - c), c});
+        }
+    }
+    for (int s = 0; s < 4; s++)
+        if (L.grp[s] == n_clips) ogrp[s] = (int)owork.size();
+    const int64_t head_total = ox.head_off[n_cand];
+    if (head_total > INT32_MAX || owork.size() > (size_t)INT32_MAX) return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: too many candidates in one call");
+    auto al16 = [](size_t b) { return (b + 15) / 16 * 16; };
+    const size_t o_work = al16(sizeof(M3sOffCand) * cands.size()), o_head = o_work + al16(sizeof(M3sOffWork) * owork.size());
+    const size_t o_body = o_head + al16((size_t)head_total);
+    if ((rc = m3s_buf_reserve(h, h->e_cand, o_body + (size_t)body_total + 16))) return rc;
+    char *base = (char *)h->e_cand.p;
+    M3S_CUDA(h, cudaMemcpyAsync(base, cands.data(), sizeof(M3sOffCand) * cands.size(), cudaMemcpyHostToDevice, h->stream));
+    M3S_CUDA(h, cudaMemcpyAsync(base + o_work, owork.data(), sizeof(M3sOffWork) * owork.size(), cudaMemcpyHostToDevice, h->stream));
+    if (head_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_head, ox.head, (size_t)head_total, cudaMemcpyHostToDevice, h->stream));
+    if (body_total > 0) M3S_CUDA(h, cudaMemcpyAsync(base + o_body, ox.body, (size_t)body_total, cudaMemcpyHostToDevice, h->stream));
+    const M3sOffCand *d_cands = (const M3sOffCand *)base;
+    const M3sOffWork *d_owork = (const M3sOffWork *)(base + o_work);
+    const uint8_t *d_head = (const uint8_t *)(base + o_head), *d_body = (const uint8_t *)(base + o_body);
+    M3S_CUDA(h, cudaFuncSetAttribute(k_enc_offsets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RateSmem)));
+    std::vector<M3sEncState> states((size_t)n_cand);   // the carried state is per candidate
+    rc = enc_pipeline(h, a, L, states, nullptr, tr_t, [&](const EncChunk &c) -> int {
+        for (int s = 0; s < 3; s++) {
+            if (c.grp_slot[s + 1] == c.grp_slot[s] || ogrp[s + 1] == ogrp[s]) continue;
+            M3S_KBEGIN(h, M3S_K_ENC_OFFSETS);
+            k_enc_offsets<<<(unsigned)((ogrp[s + 1] - ogrp[s] + OFFSETS_WARPS - 1) / OFFSETS_WARPS), 32 * OFFSETS_WARPS, sizeof(RateSmem), h->stream>>>(
+                c.clips, d_owork, ogrp[s], ogrp[s + 1], d_cands, d_head, d_body, (M3sEncState *)h->e_state.p, h->d_tab,
+                (const EncTables *)h->e_tabs.p, (const uint32_t *)h->e_pad.p, s, (int32_t)c.c0, (int32_t)L.cf, (const int32_t *)c.set.mdct.p,
+                (const M3sEncStats *)c.set.gran.p, (const uint4 *)c.set.var.p, (const uint32_t *)c.set.sum.p);
+            M3S_LAUNCH_CHECK(h);
+        }
+        return M3S_OK;
+    });
+    if (rc) return rc;
+    // ---- results, by the caller's candidate index
+    for (int64_t c = 0; c < n_cand; c++) hide_str_offset_out[c] = states[(size_t)c].hide_off;
+    for (int j = 0; j < n_clips; j++)
+        for (int64_t c = ox.cand_off[j]; c < ox.cand_off[j + 1]; c++)
+            if (states[(size_t)c].overrun)
+                return m3s_fail(h, M3S_ERR_ARG, "encode_offsets: clip %d candidate %lld frame %d: the step search runs past the end of the step "
+                                "table (quantize would read steptabi[128]; the reference has no defined output for this input, SURVEY A.E13)",
+                                j, (long long)c, states[(size_t)c].overrun - 1);
+    return M3S_OK;
+}
+
+extern "C" int m3s_encode_offsets(m3s_handle_t h, const int16_t *pcm, int mem, const int64_t *pcm_off, const int64_t *n_samples,
+                                  int32_t n_clips, const int32_t *sample_rate, const int32_t *bitrate_kbps, const uint8_t *body,
+                                  const int64_t *body_off, const int64_t *cand_off, const uint8_t *head, const int64_t *head_off,
+                                  const int64_t *body_len, int64_t *hide_str_offset_out)
+{
+    return drain_on_error(h, encode_offsets(h, EncClips{pcm, mem, pcm_off, n_samples, n_clips, sample_rate, bitrate_kbps},
+                                            EncOffsets{body, body_off, cand_off, head, head_off, body_len}, hide_str_offset_out));
 }
 
 extern "C" int m3s_encode_taps(m3s_handle_t h, int32_t *mdct, int32_t *ix, int32_t *info, int32_t *scfsi)
@@ -2301,18 +2340,18 @@ extern "C" int m3s_encode_taps(m3s_handle_t h, int32_t *mdct, int32_t *ix, int32
     const std::vector<int64_t> &R = h->enc_tap_runs;   // (device frame, caller frame, frames): one run when the order is the caller's
     const size_t NM = 4 * 576, NI = 4 * ENC_INFO_FIELDS;   // values per frame
     for (size_t r = 0; r < R.size(); r += 3) {
-        if (mdct) M3S_CUDA(h, cudaMemcpyAsync(mdct + R[r + 1] * NM, (const int32_t *)h->e_mdct.p + R[r] * NM, R[r + 2] * NM * 4, cudaMemcpyDeviceToHost, h->stream));
-        if (info) M3S_CUDA(h, cudaMemcpyAsync(info + R[r + 1] * NI, (const int32_t *)h->e_info.p + R[r] * NI, R[r + 2] * NI * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (mdct) M3S_CUDA(h, cudaMemcpyAsync(mdct + R[r + 1] * NM, (const int32_t *)h->es[0].mdct.p + R[r] * NM, R[r + 2] * NM * 4, cudaMemcpyDeviceToHost, h->stream));
+        if (info) M3S_CUDA(h, cudaMemcpyAsync(info + R[r + 1] * NI, (const int32_t *)h->es[0].info.p + R[r] * NI, R[r + 2] * NI * 4, cudaMemcpyDeviceToHost, h->stream));
     }
     std::vector<int16_t> ix16;
     std::vector<uint8_t> sc8;
     if (ix) {
         ix16.resize((size_t)nf * NM);
-        M3S_CUDA(h, cudaMemcpyAsync(ix16.data(), h->e_ix.p, ix16.size() * 2, cudaMemcpyDeviceToHost, h->stream));
+        M3S_CUDA(h, cudaMemcpyAsync(ix16.data(), h->es[0].ix.p, ix16.size() * 2, cudaMemcpyDeviceToHost, h->stream));
     }
     if (scfsi) {
         sc8.resize((size_t)nf * 8);
-        M3S_CUDA(h, cudaMemcpyAsync(sc8.data(), h->e_scfsi.p, sc8.size(), cudaMemcpyDeviceToHost, h->stream));
+        M3S_CUDA(h, cudaMemcpyAsync(sc8.data(), h->es[0].scfsi.p, sc8.size(), cudaMemcpyDeviceToHost, h->stream));
     }
     M3S_CUDA(h, cudaStreamSynchronize(h->stream));
     for (size_t r = 0; r < R.size(); r += 3) {

@@ -103,6 +103,16 @@ def _i64(a):
     return a, a.ctypes.data_as(_c_i64p)
 
 
+def _pcm_offsets(ns, pcm_off):
+    """Element offset of every clip's PCM, as _i64 gives it: the given offsets, or the clips back to back."""
+    return _i64(np.concatenate([[0], np.cumsum(ns * 2)])[:-1] if pcm_off is None else pcm_off)
+
+
+def _per_clip(x, n):
+    """An int or one entry per clip, as n contiguous int32 values."""
+    return np.ascontiguousarray(np.broadcast_to(np.asarray(x, np.int32), (n,)))
+
+
 def _ptr(x):
     """Raw address of a numpy array / torch tensor / int / None."""
     if x is None:
@@ -161,6 +171,15 @@ class Handle:
     def _check(self, rc, what):
         if rc != 0:
             raise M3SError(f"{what} failed ({rc}): {self._L.m3s_last_error(self._h).decode()}")
+
+    def _check_encode(self, rc, what):
+        """_check, but a step-table overrun raises IndexError: the reference's quantize() indexes its step table past the end
+        for this input (SURVEY A.E13) and gives no output."""
+        if rc == M3S_ERR_ARG:
+            msg = self._L.m3s_last_error(self._h).decode()
+            if STEP_TABLE_OVERRUN in msg:
+                raise IndexError(f"index out of bounds: {msg}")
+        self._check(rc, what)
 
     def set_stream(self, stream_ptr):
         self._check(self._L.m3s_set_stream(self._h, ctypes.c_void_p(stream_ptr) if stream_ptr else None), "m3s_set_stream")
@@ -335,13 +354,10 @@ class Handle:
         L = self._L
         n = len(n_samples)
         ns, ns_p = _i64(n_samples)
-        if pcm_off is None:
-            pcm_off = np.concatenate([[0], np.cumsum(ns * 2)])[:-1]
-        po, po_p = _i64(pcm_off)
+        po, po_p = _pcm_offsets(ns, pcm_off)
         mixed = not (np.isscalar(sample_rate) and np.isscalar(bitrate_kbps))
         if mixed:
-            srs = np.ascontiguousarray(np.broadcast_to(np.asarray(sample_rate, np.int32), (n,)))
-            brs = np.ascontiguousarray(np.broadcast_to(np.asarray(bitrate_kbps, np.int32), (n,)))
+            srs, brs = _per_clip(sample_rate, n), _per_clip(bitrate_kbps, n)
             keys = list(zip(ns.tolist(), srs.tolist(), brs.tolist()))
         else:
             keys = [(int(s), sample_rate, bitrate_kbps) for s in ns]
@@ -379,12 +395,7 @@ class Handle:
         else:
             rc = L.m3s_encode(self._h, _ptr(pcm), mem, po_p, ns_p, n, sample_rate, bitrate_kbps, pl_p, ploff_p, _ptr(mp3_out),
                               mo_p, mc_p, out_len.ctypes.data_as(_c_i64p), hoff.ctypes.data_as(_c_i64p))
-        if rc == M3S_ERR_ARG:
-            msg = L.m3s_last_error(self._h).decode()
-            if STEP_TABLE_OVERRUN in msg:
-                # the reference's quantize() indexes its step table past the end for this input (SURVEY A.E13): no output
-                raise IndexError(f"index out of bounds: {msg}")
-        self._check(rc, "m3s_encode_mixed" if mixed else "m3s_encode")
+        self._check_encode(rc, "m3s_encode_mixed" if mixed else "m3s_encode")
         res = dict(mp3=mp3_out, mp3_off=mo, out_len=out_len, hide_str_offset=hoff)
         if taps:
             nf = int((ns // 1152).sum())
@@ -407,11 +418,8 @@ class Handle:
         if len(bodies) != n or len(candidates) != n:
             raise ValueError("encode_offsets: one body and one candidate list per clip")
         ns, ns_p = _i64(n_samples)
-        if pcm_off is None:
-            pcm_off = np.concatenate([[0], np.cumsum(ns * 2)])[:-1]
-        po, po_p = _i64(pcm_off)
-        srs = np.ascontiguousarray(np.broadcast_to(np.asarray(sample_rate, np.int32), (n,)))
-        brs = np.ascontiguousarray(np.broadcast_to(np.asarray(bitrate_kbps, np.int32), (n,)))
+        po, po_p = _pcm_offsets(ns, pcm_off)
+        srs, brs = _per_clip(sample_rate, n), _per_clip(bitrate_kbps, n)
         body = np.frombuffer(b"".join(bodies) + b"\0", np.uint8)
         bo, bo_p = _i64(np.concatenate([[0], np.cumsum([len(b) for b in bodies])]))
         co, co_p = _i64(np.concatenate([[0], np.cumsum([len(c) for c in candidates])]))
@@ -424,11 +432,7 @@ class Handle:
         rc = L.m3s_encode_offsets(self._h, _ptr(pcm), _mem_of(pcm), po_p, ns_p, n, srs.ctypes.data_as(_c_i32p),
                                   brs.ctypes.data_as(_c_i32p), _ptr(body), bo_p, co_p, _ptr(head), ho_p, bl_p,
                                   out.ctypes.data_as(_c_i64p))
-        if rc == M3S_ERR_ARG:
-            msg = L.m3s_last_error(self._h).decode()
-            if STEP_TABLE_OVERRUN in msg:
-                raise IndexError(f"index out of bounds: {msg}")
-        self._check(rc, "m3s_encode_offsets")
+        self._check_encode(rc, "m3s_encode_offsets")
         return [out[co[i]:co[i + 1]].copy() for i in range(n)]
 
 
